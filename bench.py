@@ -17,6 +17,7 @@ on the data path), so the job size is fixed: "strong" scaling as BASELINE.json's
   --impl reference : the reference's CPU path on this box's host cores on the same fixed sample of blocks.
   --config c4 | c5 | --missing 0.005 : BASELINE.json configs[3], configs[4] and the mask path (parity cases, not the
            headline; their lines are kept under profiles/).
+  --dump-outputs DIR : the betas of the last timed fit (c4 on one GPU: and its PRS scores) as DIR/beta_s.npy, beta_l.npy[, prs.npy].
 """
 import argparse
 import json
@@ -65,7 +66,35 @@ def parse():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--seed", type=int, default=20240003)
     ap.add_argument("--emulate-shard", default="", help="R/N: time rank R's shard of an N-GPU run on one GPU (tuning aid)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float64); "
+                         "in strong scaling over several GPUs, the betas of all ranks gathered in workload order (no PRS)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: the inputs are seeded, so two builds run with the same arguments can be compared output for output.
+    Above DUMP_MAX_BYTES in all, every array keeps the same fraction of its last axis at positions drawn from a fixed seed,
+    written beside it as <name>_index.npy."""
+    arrays = {k: np.ascontiguousarray(v, np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    frac = 1.0
+    if total > DUMP_MAX_BYTES:          # each kept column also costs its 8-byte index; 64 KB left for the .npy headers
+        frac = (DUMP_MAX_BYTES - (64 << 10)) / (total + 8.0 * sum(a.shape[-1] for a in arrays.values()))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        if frac < 1.0:
+            n = a.shape[-1]
+            idx = np.sort(np.random.default_rng(0).choice(n, int(n * frac), replace=False))
+            a = a[..., idx]
+            np.save(os.path.join(out_dir, k + "_index.npy"), idx.astype(np.float64))
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -378,7 +407,7 @@ def main():
         times = []
         kind = "port"
         for i in range(min(args.warmup, 1) + args.steps):       # one warm-up pass is enough on the CPU
-            dt, kind, _, _, _ = run_cpu(w, blocks, threads, sigma_s)
+            dt, kind, ref_bs, ref_bl, _ = run_cpu(w, blocks, threads, sigma_s)
             if i >= min(args.warmup, 1):
                 times.append(dt)
         dt = float(np.mean(times)) if times else float("nan")
@@ -393,7 +422,9 @@ def main():
                 "cpu_baseline": cl,
                 "e2e": {"value": v, "unit": "blocks/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
                 "gpu_launches": 0}
-        print(json.dumps(line))
+        print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"beta_s": ref_bs, "beta_l": ref_bl})
         return
 
     # ---------------- B200 arm
@@ -467,7 +498,7 @@ def main():
         tms.append(t)
         step_ms = t["total_ms"]                    # z upload -> decode -> Gram -> solve -> betas in pinned host memory
         if val:
-            _, kms = score(r)
+            prs_timed, kms = score(r)
             prs_ms.append(kms)
             step_ms += kms
         dev_ms.append(step_ms)
@@ -585,6 +616,20 @@ def main():
         except Exception as e:
             cpu_base = {"value": None, "unit": "blocks/s", "cores": 0, "kind": "port", "sample": f"failed: {e}"}
 
+    # --dump-outputs: with several GPUs in strong scaling the betas are gathered into workload order, so the files do not
+    # depend on how the cost model sharded the blocks; the PRS of a rank is over its own validation panel and is left out
+    outputs = None
+    if args.dump_outputs:
+        if dist is not None and args.scaling == "strong":
+            from dbslmm_b200 import multigpu
+            ww = {"s_off": w["s_off"], "l_off": w["l_off"]}
+            full = [multigpu.gather_betas(ww, owner, rank, world, beta_s_timed[f], beta_l_timed[f], dist) for f in range(len(folds))]
+            outputs = {"beta_s": np.stack([s for s, _ in full]), "beta_l": np.stack([l for _, l in full])}
+        else:
+            outputs = {"beta_s": beta_s_timed, "beta_l": beta_l_timed}
+            if val:
+                outputs["prs"] = prs_timed
+
     dev_total = float(np.sum(dev_ms))
     par_vec = [parity["max_rel_vs_exact_oracle"], 0.0 if parity["gram_bit_exact"] else 1.0, parity["streaming_vs_resident_max_rel"]] if parity else [0.0, 0.0, 0.0]
     stats = torch.tensor([dev_total, wall_e2e, wall_resident, float(my_blocks), float(my_snps), float(n_bad)] + par_vec, dtype=torch.float64, device=dev)
@@ -688,7 +733,9 @@ def main():
         line["parity"] = parity
     if cpu_base:
         line["cpu_baseline"] = cpu_base
-    print(json.dumps(line))
+    print(json.dumps(line), flush=True)
+    if outputs:
+        dump_outputs(args.dump_outputs, outputs)
     if dist is not None:
         dist.destroy_process_group()
 

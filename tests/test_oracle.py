@@ -109,6 +109,13 @@ def test_oracle_ref_mode_matches_reference_golden_ragged(ragged):
                             threads=2, mode=O.MODE_REF)
     assert sing == 0
     assert relmax(bs, d["beta_s"]) <= bar("synth_ragged", "beta_s", "pcg") and relmax(bl, d["beta_l"]) <= bar("synth_ragged", "beta_l", "pcg")
+    # the single-block entry point on block 5: the stored betas of that block are what the reference's estBlock returned
+    # for it (oracle/ref_harness.cpp's ref_est_path calls ref_est_block once per block)
+    s0, s1, l0, l1 = d["s_off"][5], d["s_off"][6], d["l_off"][5], d["l_off"][6]
+    assert l1 > l0
+    o_s, o_l, _, _ = O.est_block(d["bed"], n_ref, n_obs, sig, d["s_pos"][s0:s1], d["s_z"][s0:s1], d["l_pos"][l0:l1], d["l_z"][l0:l1],
+                                 mode=O.MODE_REF)
+    assert relmax(o_s, d["beta_s"][s0:s1]) < 1e-9 and relmax(o_l, d["beta_l"][l0:l1]) < 1e-9
     b, _, _, _ = O.est(d["bed"], n_ref, n_obs, sig, d["lmm_off"], np.arange(d["lmm_z"].size, dtype=np.int32), d["lmm_z"],
                        threads=2, mode=O.MODE_REF)
     assert relmax(b, d["lmm_beta"]) < 1e-9
