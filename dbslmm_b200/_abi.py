@@ -22,7 +22,7 @@ EXPORTS = [
     "dbslmm_b200_abi_version", "dbslmm_b200_device_count", "dbslmm_b200_create", "dbslmm_b200_destroy",
     "dbslmm_b200_last_error", "dbslmm_b200_load_bed", "dbslmm_b200_snp_stats", "dbslmm_b200_plan_shards",
     "dbslmm_b200_fit", "dbslmm_b200_fit_multi", "dbslmm_b200_host_alloc", "dbslmm_b200_host_free", "dbslmm_b200_score", "dbslmm_b200_score_prefetch", "dbslmm_b200_get_row_codes", "dbslmm_b200_get_block_sigma",
-    "dbslmm_b200_get_block_gram", "dbslmm_b200_get_block_iters",
+    "dbslmm_b200_get_block_factor", "dbslmm_b200_get_block_gram", "dbslmm_b200_get_block_iters",
 ]
 
 
@@ -82,6 +82,7 @@ def load():
         lib.dbslmm_b200_score_prefetch.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32]
         lib.dbslmm_b200_get_row_codes.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32]
         lib.dbslmm_b200_get_block_sigma.argtypes = [C.c_void_p, C.c_int32, C.c_void_p]
+        lib.dbslmm_b200_get_block_factor.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]
         lib.dbslmm_b200_get_block_gram.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
         lib.dbslmm_b200_get_block_iters.argtypes = [C.c_void_p, C.c_int32]
         _lib = lib
@@ -265,6 +266,14 @@ class Engine:
         out = np.zeros((m, m), np.float64)
         self._check(self.lib.dbslmm_b200_get_block_sigma(self.h, int(block), out.ctypes.data), "get_block_sigma")
         return out
+
+    def block_factor(self, block, m):
+        """(L, y) of `block` from the last fold of the last Cholesky fit: L = m x m lower-triangular factor of
+        K = Sigma + c diag(1_small, 0_large) (small SNPs first), y = L^-1 z."""
+        L = np.zeros((m, m), np.float64)
+        y = np.zeros(m, np.float64)
+        self._check(self.lib.dbslmm_b200_get_block_factor(self.h, int(block), L.ctypes.data, y.ctypes.data), "get_block_factor")
+        return L, y
 
     def block_gram(self, block, m):
         q = np.zeros((m, m), np.int32)

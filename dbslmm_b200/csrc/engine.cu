@@ -202,6 +202,7 @@ struct dbslmm_b200_handle {
     Plan plan;
 
     int32_t last_flags = 0, last_solver = 0, last_nfolds = 0;
+    bool last_quad = false;                   // the last fit computed quadform_out: nothing was factored
     PFN_cuTensorMapEncodeTiled_v12000 encode = nullptr;
 };
 
@@ -1760,6 +1761,7 @@ int fit_impl(dbslmm_b200_handle* h, const dbslmm_b200_fit_args* a, bool streamin
     }
     h->last_flags = a->flags | (full ? DBSLMM_B200_FLAG_FULL_SIGMA : 0);
     h->last_solver = a->solver;
+    h->last_quad = quad;
     h->last_nfolds = a->n_folds;
     if (a->timing) {
         dbslmm_b200_timing* t = a->timing;
@@ -2091,14 +2093,15 @@ int dbslmm_b200_get_row_codes(dbslmm_b200_handle* h, int32_t block, int32_t j, i
     return DBSLMM_B200_OK;
 }
 
+// The first mp + extra_rows rows (stride ld) of block `block`'s matrix in device buffer `dev` -> tmp.
 static int fetch_block(dbslmm_b200_handle* h, int32_t block, const void* dev, size_t esz, std::vector<uint8_t>& tmp,
-                       const BlockDesc** bd_out) {
+                       const BlockDesc** bd_out, int extra_rows = 0) {
     if (!h->plan.valid) return fail(h, DBSLMM_B200_ERR_STATE, "no fit yet");
     if (block < 0 || block >= h->plan.n_blocks) return fail(h, DBSLMM_B200_ERR_ARG, "block out of range");
     const BlockDesc& bd = h->plan.blocks[block];
     *bd_out = &bd;
     if (bd.m == 0) return DBSLMM_B200_OK;
-    tmp.resize((size_t)bd.mp * bd.ld * esz);
+    tmp.resize((size_t)(bd.mp + extra_rows) * bd.ld * esz);
     CU_TRY(h, cudaSetDevice(h->device));
     CU_TRY(h, cudaMemcpy(tmp.data(), (const uint8_t*)dev + (size_t)bd.moff * esz, tmp.size(), cudaMemcpyDeviceToHost));
     return DBSLMM_B200_OK;
@@ -2108,16 +2111,34 @@ int dbslmm_b200_get_block_sigma(dbslmm_b200_handle* h, int32_t block, double* si
     if (!h || !sigma_out) return DBSLMM_B200_ERR_ARG;
     std::vector<uint8_t> tmp;
     const BlockDesc* bd = nullptr;
-    static const bool fetch_l = std::getenv("DBSLMM_B200_DBG_FETCH_L") != nullptr;      // debugging aid: the factor instead of Sigma
-    int rc = fetch_block(h, block, fetch_l ? h->lbuf.p : h->sigma.p, sizeof(double), tmp, &bd);
+    int rc = fetch_block(h, block, h->sigma.p, sizeof(double), tmp, &bd);
     if (rc != DBSLMM_B200_OK) return rc;
     const double* s = (const double*)tmp.data();
-    const bool full = fetch_l || (h->last_flags & DBSLMM_B200_FLAG_FULL_SIGMA) != 0;
+    const bool full = (h->last_flags & DBSLMM_B200_FLAG_FULL_SIGMA) != 0;
     for (int i = 0; i < bd->m; ++i)
         for (int j = 0; j < bd->m; ++j) {
             const double v = (j <= i || full) ? s[(size_t)i * bd->ld + j] : s[(size_t)j * bd->ld + i];
             sigma_out[(size_t)i * bd->m + j] = v;
         }
+    return DBSLMM_B200_OK;
+}
+
+int dbslmm_b200_get_block_factor(dbslmm_b200_handle* h, int32_t block, double* l_out, double* y_out) {
+    if (!h) return DBSLMM_B200_ERR_ARG;
+    if (h->plan.valid && (h->last_solver != DBSLMM_B200_SOLVER_CHOLESKY || h->last_quad))
+        return fail(h, DBSLMM_B200_ERR_STATE, "last fit did not factor (PCG solver or quadform)");
+    std::vector<uint8_t> tmp;
+    const BlockDesc* bd = nullptr;
+    // rows 0..mp-1 hold L (lower triangle; W_kk^T in the upper triangles of the diagonal tiles), row mp holds y = L^-1 z
+    int rc = fetch_block(h, block, h->lbuf.p, sizeof(double), tmp, &bd, 1);
+    if (rc != DBSLMM_B200_OK) return rc;
+    const double* s = (const double*)tmp.data();
+    const int m = bd->m;
+    if (l_out)
+        for (int i = 0; i < m; ++i)
+            for (int j = 0; j < m; ++j) l_out[(size_t)i * m + j] = (j <= i) ? s[(size_t)i * bd->ld + j] : 0.0;
+    if (y_out)
+        for (int j = 0; j < m; ++j) y_out[j] = s[(size_t)bd->mp * bd->ld + j];
     return DBSLMM_B200_OK;
 }
 

@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define DBSLMM_B200_ABI_VERSION 5
+#define DBSLMM_B200_ABI_VERSION 6
 
 #if defined(__GNUC__)
 #define DBSLMM_B200_API __attribute__((visibility("default")))
@@ -196,6 +196,12 @@ DBSLMM_B200_API int  dbslmm_b200_get_row_codes(dbslmm_b200_handle* h, int32_t bl
 /* Sigma of block b as dense row-major m x m (m = m_s + m_l, small SNPs first).  Lower triangle is
  * always valid; the upper one only with FLAG_FULL_SIGMA / PCG solver (else mirrored on the host). */
 DBSLMM_B200_API int  dbslmm_b200_get_block_sigma(dbslmm_b200_handle* h, int32_t block, double* sigma_out);
+/* The Cholesky factor of block b's bordered system K = Sigma + c diag(1_small, 0_large) from the LAST fold of the last
+ * Cholesky fit: l_out = m x m row-major, the lower triangle of L with its diagonal, zeros above (the W_kk^T the solver
+ * keeps in the upper triangles of the diagonal tiles is not returned); y_out = the m entries of y = L^-1 z (matrix row mp).
+ * Either may be NULL.  DBSLMM_B200_ERR_STATE after a PCG or quadform fit.  tools/l_diff.py uses it to show where the
+ * factors of two fits differ (block, panel, rows). */
+DBSLMM_B200_API int  dbslmm_b200_get_block_factor(dbslmm_b200_handle* h, int32_t block, double* l_out, double* y_out);
 /* raw integer Gram planes (needs FLAG_KEEP_INT_GRAM): Q = G G^T, A_ij = sum g_i M_j, N = M M^T;
  * A and N may be NULL; for blocks without missing calls A_ij = S_i and N = n_ref. */
 DBSLMM_B200_API int  dbslmm_b200_get_block_gram(dbslmm_b200_handle* h, int32_t block, int32_t* q_out, int32_t* a_out, int32_t* n_out);

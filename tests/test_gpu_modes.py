@@ -10,6 +10,8 @@ import pytest
 from dbslmm_b200 import _abi, synth
 from oracle import oracle as O
 
+import solver_ref as R
+
 pytestmark = pytest.mark.gpu
 
 MODES = {
@@ -43,6 +45,10 @@ MODES = {
     "gram_single_cta_l2_hints": {"DBSLMM_B200_GRAM": "single", "DBSLMM_B200_GRAM_HINT": "3"},
     # the panel kernel without the next item's first chunk issued during the epilogue
     "no_next_item_prefetch": {"DBSLMM_B200_NEXT_PF": "0", "DBSLMM_B200_TPC": "8,0"},
+    # the cluster back substitution (chosen per batch from its largest block) on blocks of 5-16 panels, and on every
+    # block, 1-SNP and empty ones included
+    "cluster_backsolve_on_bulk_sizes": {"DBSLMM_B200_CLASSES": "4,20"},
+    "one_size_class": {"DBSLMM_B200_CLASSES": "40"},
 }
 KEYS = sorted({k for m in MODES.values() for k in m})
 
@@ -85,7 +91,9 @@ def test_solver_modes_agree_with_the_oracle(problem, mode):
 
 def test_genome_wide_residuals_and_streaming_equality(engine):
     """BASELINE.json configs[2] at full size (1,703 blocks, 1.1 M SNPs, n_ref 2,000): K x = z residual from the library's
-    own Sigma on sampled blocks (largest, smallest, spread), all block statuses clean, streaming fit == resident fit."""
+    own Sigma and every stage check of tests/solver_ref.py on sampled blocks (largest, smallest, spread), all block
+    statuses clean, streaming fit == resident fit."""
+    from test_gpu_solver import Maxima
     torch = pytest.importorskip("torch")
     import bench
     import argparse
@@ -102,6 +110,7 @@ def test_genome_wide_residuals_and_streaming_equality(engine):
     sizes = w["sizes"]
     order = np.argsort(sizes)
     sample = sorted(set(order[:3].tolist() + order[-4:].tolist() + order[:: max(1, order.size // 16)].tolist()))
+    mx = Maxima()
     for b in sample:
         ms = int(w["s_off"][b + 1] - w["s_off"][b]); ml = int(w["l_off"][b + 1] - w["l_off"][b])
         m = ms + ml
@@ -114,6 +123,15 @@ def test_genome_wide_residuals_and_streaming_equality(engine):
         z = np.concatenate([sz[w["s_off"][b]:w["s_off"][b + 1]], lz[w["l_off"][b]:w["l_off"][b + 1]]])
         res = np.abs(K @ x - z).max() / max(np.abs(z).max(), 1e-300)
         assert res < 1e-10, (b, m, res)
+        # every stage of the block against the extended-precision reference (tests/solver_ref.py)
+        pos = np.concatenate([w["s_pos"][w["s_off"][b]:w["s_off"][b + 1]], w["l_pos"][w["l_off"][b]:w["l_off"][b + 1]]])
+        sstar = R.exact_sigma(w["bed"], w["n_ref"], pos, 0.8)
+        c = R.ridge(sig, n_obs)
+        xstar, kappa = R.refined_solve(R.k_matrix(sstar, ms, c), z)
+        L, y = engine.block_factor(b, m)
+        mx.add(R.check_block(f"{b} (m={m}, genome-wide)", ms=ms, c=c, z=z, sigma_lib=S, sigma_star=sstar, L=L, y=y, x=x,
+                             xstar=xstar, kappa=kappa))
+    mx.record("solver/genome_wide")
     rs = engine.fit(*csr, sigma_s=[sig], n_obs=n_obs, bed=w["bed"], n_ref=w["n_ref"])
     assert relmax(rs["beta_s"], r["beta_s"]) <= 1e-11 and relmax(rs["beta_l"], r["beta_l"]) <= 1e-11
     # run-to-run determinism at full load (every reduction order is fixed): a second resident fit is bit-identical.  This
