@@ -21,7 +21,7 @@ FLAG_PANEL_SUBSET = 8
 EXPORTS = [
     "dbslmm_b200_abi_version", "dbslmm_b200_device_count", "dbslmm_b200_create", "dbslmm_b200_destroy",
     "dbslmm_b200_last_error", "dbslmm_b200_load_bed", "dbslmm_b200_snp_stats", "dbslmm_b200_plan_shards",
-    "dbslmm_b200_fit", "dbslmm_b200_fit_multi", "dbslmm_b200_host_alloc", "dbslmm_b200_host_free", "dbslmm_b200_score", "dbslmm_b200_score_prefetch", "dbslmm_b200_get_row_codes", "dbslmm_b200_get_block_sigma",
+    "dbslmm_b200_fit", "dbslmm_b200_fit_multi", "dbslmm_b200_host_alloc", "dbslmm_b200_host_free", "dbslmm_b200_score", "dbslmm_b200_score_prefetch", "dbslmm_b200_score_stream", "dbslmm_b200_get_row_codes", "dbslmm_b200_get_block_sigma",
     "dbslmm_b200_get_block_factor", "dbslmm_b200_get_block_gram", "dbslmm_b200_get_block_iters",
 ]
 
@@ -79,6 +79,9 @@ def load():
         lib.dbslmm_b200_host_free.restype = None
         lib.dbslmm_b200_score.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64,
                                           C.c_void_p, C.c_int32, C.c_void_p, C.POINTER(C.c_float)]
+        lib.dbslmm_b200_score_stream.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64,
+                                                 C.c_void_p, C.c_int32, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                 C.POINTER(C.c_int32), C.POINTER(C.c_float)]
         lib.dbslmm_b200_score_prefetch.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32]
         lib.dbslmm_b200_get_row_codes.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32]
         lib.dbslmm_b200_get_block_sigma.argtypes = [C.c_void_p, C.c_int32, C.c_void_p]
@@ -254,6 +257,35 @@ class Engine:
         self._check(self.lib.dbslmm_b200_score(self.h, bptr, n_snp_val, n_val, pos.ctypes.data, _ptr(fl),
                                                pos.size, beta.ctypes.data, beta.shape[0], out.ctypes.data, C.byref(ms)), "score")
         return out, ms.value
+
+    def score_stream(self, bed_val, n_val, pos, beta, flip=None, chunk_bytes=0):
+        """PRS over a target panel of any size, streamed through the GPU chunk by chunk (dbslmm_b200_score_stream).
+        bed_val: uint8 payload after the magic bytes ([n_snp, ceil(n_val/4)] or flat), e.g. a numpy.memmap of the .bed
+        opened with offset=3: only the rows named by pos are read.  Returns (scores[n_folds, n_val], cnt[n_val], cnt2[n_val])
+        with PLINK's CNT / CNT2; the summed kernel time of the call is left in self.last_kernel_ms and the number of scored
+        rows without a called genotype in self.last_empty_rows."""
+        n_val = int(n_val)
+        pitch = (n_val + 3) // 4
+        if not (isinstance(bed_val, np.ndarray) and bed_val.dtype == np.uint8 and bed_val.flags.c_contiguous):
+            bed_val = np.ascontiguousarray(bed_val, np.uint8)          # a contiguous memmap is used in place, never copied
+        pos = np.ascontiguousarray(pos, np.int32)
+        beta = np.ascontiguousarray(np.atleast_2d(beta), np.float64)
+        if beta.shape[1] != pos.size or (flip is not None and np.size(flip) != pos.size):
+            raise ValueError("score_stream: beta must be [n_folds, pos.size] and flip [pos.size]")
+        fl = None if flip is None else np.ascontiguousarray(flip, np.uint8)
+        out = np.zeros((beta.shape[0], n_val), np.float64)
+        empty = C.c_int32(0)
+        cnt = np.zeros(n_val, np.int32)
+        cnt2 = np.zeros(n_val, np.int32)
+        ms = C.c_float(0)
+        self._check(self.lib.dbslmm_b200_score_stream(self.h, bed_val.ctypes.data, bed_val.size // pitch, n_val, pos.ctypes.data,
+                                                      _ptr(fl), pos.size, beta.ctypes.data, beta.shape[0], int(chunk_bytes),
+                                                      out.ctypes.data, cnt.ctypes.data, cnt2.ctypes.data, C.byref(empty),
+                                                      C.byref(ms)),
+                    "score_stream")
+        self.last_kernel_ms = ms.value
+        self.last_empty_rows = empty.value
+        return out, cnt, cnt2
 
     # ---- inspection hooks (parity tests)
     def row_codes(self, block, j, n, plane=0):

@@ -1,6 +1,6 @@
 """In-tree build of the sm_100a library and the `dbslmm` CLI (explicit nvcc / g++ calls).
 
-    python -m dbslmm_b200.build            # libdbslmm_b200.so + build/dbslmm
+    python -m dbslmm_b200.build            # libdbslmm_b200.so + build/dbslmm, build/valid, build/score
 Outputs stay inside the repo (git-ignored) so they travel with a gpurun snapshot.
 """
 import concurrent.futures as cf
@@ -16,6 +16,7 @@ BUILD = os.path.join(ROOT, "build")
 LIB = os.path.join(PKG, "libdbslmm_b200.so")
 CLI = os.path.join(BUILD, "dbslmm")
 VALID_CLI = os.path.join(BUILD, "valid")
+SCORE_CLI = os.path.join(BUILD, "score")
 
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 GXX = "/usr/bin/g++"
@@ -76,6 +77,11 @@ def build_cli(force=False):
     vsrcs = [os.path.join(HOST, "valid_main.cpp"), os.path.join(HOST, "ingest.cpp")]
     if os.path.exists(vsrcs[0]) and (force or _newer(VALID_CLI, vsrcs + deps)):
         _run([GXX, "-O2", "-std=c++17", "-pthread", "-I", os.path.join(ROOT, "include"), "-o", VALID_CLI] + vsrcs +
+             ["-L", PKG, "-ldbslmm_b200", "-Wl,-rpath,$ORIGIN/../dbslmm_b200", "-Wl,-rpath," + PKG])
+    # `score`: plink --score <eff>.txt 1 2 4 sum over a target fileset (DBSLMM_script.sh:87), every fold in one pass
+    ssrc = os.path.join(HOST, "score_main.cpp")
+    if os.path.exists(ssrc) and (force or _newer(SCORE_CLI, [ssrc] + deps)):
+        _run([GXX, "-O2", "-std=c++17", "-pthread", "-I", os.path.join(ROOT, "include"), "-o", SCORE_CLI, ssrc] +
              ["-L", PKG, "-ldbslmm_b200", "-Wl,-rpath,$ORIGIN/../dbslmm_b200", "-Wl,-rpath," + PKG])
     return CLI
 

@@ -195,6 +195,11 @@ struct dbslmm_b200_handle {
     int32_t val_n = 0;
     bool val_announced = false, val_inflight = false;
     cudaEvent_t ev_val = nullptr;
+    // streaming scorer (dbslmm_b200_score_stream): pinned staging ring, device chunk slots, per-call work buffer
+    PinBuf s_pin[3];
+    DevBuf s_dev[2], s_work;
+    cudaEvent_t ev_pin_free[3] = {}, ev_copied[2] = {}, ev_slot_free[2] = {};
+    std::vector<cudaEvent_t> ev_chunk;   // 4 timing events per chunk (copy begin / end, kernels begin / end), grow-only
     size_t dirty_rows = 0;               // code rows the dirty map covers
     int32_t dirty_n_ref = 0;             // ... for this panel width (another width = another default mask pattern)
     const void* dirty_codes = nullptr;   // ... and this code buffer
@@ -953,6 +958,10 @@ int dbslmm_b200_create(int device, dbslmm_b200_handle** out) {
     ok = ok && cudaEventCreate(&h->ev_fork) == cudaSuccess;
     ok = ok && cudaEventCreateWithFlags(&h->ev_bed, cudaEventDisableTiming) == cudaSuccess;
     ok = ok && cudaEventCreateWithFlags(&h->ev_val, cudaEventDisableTiming) == cudaSuccess;
+    for (int i = 0; i < 3 && ok; ++i) ok = cudaEventCreateWithFlags(&h->ev_pin_free[i], cudaEventDisableTiming) == cudaSuccess;
+    for (int i = 0; i < 2 && ok; ++i)
+        ok = cudaEventCreateWithFlags(&h->ev_copied[i], cudaEventDisableTiming) == cudaSuccess &&
+             cudaEventCreateWithFlags(&h->ev_slot_free[i], cudaEventDisableTiming) == cudaSuccess;
     ok = ok && chol_configure() == cudaSuccess;
     if (!ok) { dbslmm_b200_destroy(h); return DBSLMM_B200_ERR_CUDA; }
     *out = h;
@@ -969,6 +978,15 @@ void dbslmm_b200_destroy(dbslmm_b200_handle* h) {
     h->h_blob.release();
     h->h_out.release();
     h->h_stats.release();
+    for (PinBuf& b : h->s_pin) b.release();
+    for (DevBuf& b : h->s_dev) b.release();
+    h->s_work.release();
+    for (cudaEvent_t e : h->ev_pin_free) if (e) cudaEventDestroy(e);
+    for (int i = 0; i < 2; ++i) {
+        if (h->ev_copied[i]) cudaEventDestroy(h->ev_copied[i]);
+        if (h->ev_slot_free[i]) cudaEventDestroy(h->ev_slot_free[i]);
+    }
+    for (cudaEvent_t e : h->ev_chunk) cudaEventDestroy(e);
     if (h->ev_bed) cudaEventDestroy(h->ev_bed);
     if (h->ev_val) cudaEventDestroy(h->ev_val);
     for (int i = 0; i < 8; ++i) if (h->ev[i]) cudaEventDestroy(h->ev[i]);
@@ -2028,7 +2046,7 @@ int dbslmm_b200_score(dbslmm_b200_handle* h, const uint8_t* bed_val, int64_t n_s
     cudaStream_t st = h->stream;
     const int32_t pitch = (n_val + 3) / 4;
     const size_t bytes = (size_t)n_snp_val * pitch;
-    const int n_chunks = std::max(1, std::min<int>(4 * h->n_sm / std::max(1, ((pitch + 3) / 4 + 255) / 256), (int)((n_scored + 63) / 64)));
+    const int n_chunks = prs_slices(h->n_sm, n_val, n_scored);
     const int nf_pass = std::min(n_folds, 3);            // folds per pass of the scoring kernel (score.cu: kMaxFolds)
     // work buffer: pos | flip | beta | partial | scores
     size_t o = 0;
@@ -2074,6 +2092,148 @@ int dbslmm_b200_score(dbslmm_b200_handle* h, const uint8_t* bed_val, int64_t n_s
     CU_TRY(h, cudaStreamSynchronize(st));
     h->val_inflight = false;                 // (the stream waited for its event)
     if (kernel_ms_out) cudaEventElapsedTime(kernel_ms_out, h->ev[0], h->ev[1]);
+    return DBSLMM_B200_OK;
+}
+
+// Streaming scorer.  A chunk is rows_cap scored rows (the last one fewer) gathered in scored order by host workers into a
+// pinned staging slot laid out as  genotype rows (pitch bytes each) | beta slice [n_folds][rows] | flip slice [rows],  so
+// one cudaMemcpyAsync on the copy stream carries all of it.  Three staging slots and two device slots: the gather of chunk
+// k + 2, the copy of chunk k + 1 and the kernels of chunk k (statistics, counts, one scoring pass per 3 folds) overlap.
+static constexpr uint64_t kStreamChunkDefault = 64ull << 20;
+struct ChunkLayout {
+    int64_t j0 = 0;
+    int32_t rows = 0;
+    size_t o_beta = 0, o_flip = 0, bytes = 0;
+};
+static ChunkLayout chunk_layout(int64_t j0, int32_t rows, int64_t pitch, int32_t n_folds) {
+    ChunkLayout c;
+    c.j0 = j0;
+    c.rows = rows;
+    c.o_beta = align_up((size_t)rows * pitch + 4, 256);          // + 4: the statistics kernel reads whole words past the last row
+    c.o_flip = c.o_beta + sizeof(double) * (size_t)n_folds * rows;
+    c.bytes = align_up(c.o_flip + (size_t)rows, 256);
+    return c;
+}
+
+int dbslmm_b200_score_stream(dbslmm_b200_handle* h, const uint8_t* bed_val, int64_t n_snp_val, int32_t n_val,
+                             const int32_t* pos, const uint8_t* flip, int64_t n_scored, const double* beta, int32_t n_folds,
+                             uint64_t chunk_bytes, double* scores_out, int32_t* cnt_out, int32_t* cnt2_out, int32_t* n_empty_out,
+                             float* kernel_ms_out) {
+    if (!h) return DBSLMM_B200_ERR_ARG;
+    if (!bed_val || n_snp_val <= 0 || n_val <= 0 || n_scored < 0 || n_folds < 1 || !scores_out || (n_scored > 0 && (!pos || !beta)))
+        return fail(h, DBSLMM_B200_ERR_ARG, "score_stream: bad arguments");
+    if (n_val > kScoreMaxNVal)
+        return fail(h, DBSLMM_B200_ERR_ARG, "score_stream: n_val = " + std::to_string(n_val) + " is above the limit of " +
+                                            std::to_string(kScoreMaxNVal) + " individuals (int32 row sums)");
+    if (n_scored > INT32_MAX / 2) return fail(h, DBSLMM_B200_ERR_ARG, "score_stream: too many SNPs (CNT = 2 x calls must fit in int32)");
+    for (int64_t j = 0; j < n_scored; ++j)
+        if (pos[j] < 0 || pos[j] >= n_snp_val) return fail(h, DBSLMM_B200_ERR_ARG, "score_stream: pos out of range of the .bed");
+    CU_TRY(h, cudaSetDevice(h->device));
+    const Trace tr;
+    cudaStream_t st = h->stream, cp = h->up_stream;
+    const int64_t pitch = (n_val + 3) / 4;
+    const bool counts = cnt_out || cnt2_out;
+    const uint64_t budget = chunk_bytes ? chunk_bytes : kStreamChunkDefault;
+    // rows per chunk: a function of chunk_bytes and n_val only, so fold f of an F-fold call sums exactly like a 1-fold call
+    const int64_t rows_cap = std::max<int64_t>(1, std::min<int64_t>(std::max<int64_t>(n_scored, 1), (int64_t)(budget / (uint64_t)(pitch + 1))));
+    const int64_t n_chunks = (n_scored + rows_cap - 1) / rows_cap;
+    const ChunkLayout full = chunk_layout(0, (int32_t)rows_cap, pitch, n_folds);
+    const int32_t nf_pass = std::min(n_folds, 3);             // folds per scoring pass (score.cu: kMaxFolds)
+    // work buffer: chunk statistics | partial sums of one pass | scores | cnt | cnt2 | empty-row count
+    size_t o = 0;
+    auto place = [&](size_t b) { size_t r = o; o = align_up(o + b, 256); return r; };
+    const size_t o_stats = place(sizeof(SnpStat) * (size_t)rows_cap),
+                 o_part = place(sizeof(double) * (size_t)prs_slices(h->n_sm, n_val, rows_cap) * nf_pass * n_val),
+                 o_sc = place(sizeof(double) * (size_t)n_folds * n_val),
+                 o_cnt = place(sizeof(int32_t) * (size_t)n_val), o_cnt2 = place(sizeof(int32_t) * (size_t)n_val),
+                 o_empty = place(sizeof(int32_t));
+    const int n_pin = (int)std::min<int64_t>(3, std::max<int64_t>(n_chunks, 1)), n_dev = std::min(2, n_pin);
+    for (int i = 0; i < n_pin; ++i) CU_TRY(h, h->s_pin[i].ensure(full.bytes));
+    for (int i = 0; i < n_dev; ++i) CU_TRY(h, h->s_dev[i].ensure(full.bytes));
+    CU_TRY(h, h->s_work.ensure(o));
+    while (h->ev_chunk.size() < (size_t)(4 * n_chunks)) {
+        cudaEvent_t e;
+        CU_TRY(h, cudaEventCreate(&e));
+        h->ev_chunk.push_back(e);
+    }
+    uint8_t* w = (uint8_t*)h->s_work.p;
+    double* scores = (double*)(w + o_sc);
+    int32_t* cnt = (int32_t*)(w + o_cnt);
+    int32_t* cnt2 = (int32_t*)(w + o_cnt2);
+    int32_t* n_empty = (int32_t*)(w + o_empty);
+    CU_TRY(h, cudaMemsetAsync(scores, 0, sizeof(double) * (size_t)n_folds * n_val, st));
+    CU_TRY(h, cudaMemsetAsync(cnt, 0, o - o_cnt, st));
+
+    // host gather of chunk k into staging slot k % 3, cut into pieces of >= 2 MB for the pool's workers
+    HostPool& pool = host_pool();
+    TaskGroup groups[3];
+    struct Drain { HostPool& p; TaskGroup* g; ~Drain() { for (int i = 0; i < 3; ++i) p.wait(g[i]); } } drain{pool, groups};
+    auto layout_of = [&](int64_t k) { const int64_t j0 = k * rows_cap; return chunk_layout(j0, (int32_t)std::min(rows_cap, n_scored - j0), pitch, n_folds); };
+    auto gather = [&](int64_t k) {
+        const ChunkLayout c = layout_of(k);
+        uint8_t* dst = (uint8_t*)h->s_pin[k % 3].p;
+        const int64_t per = std::max<int64_t>(1, ((int64_t)2 << 20) / pitch);
+        for (int64_t r0 = 0; r0 < c.rows; r0 += per) {
+            const int64_t r1 = std::min<int64_t>(c.rows, r0 + per);
+            pool.submit(groups[k % 3], [=]() {
+                for (int64_t r = r0; r < r1; ++r) std::memcpy(dst + r * pitch, bed_val + (int64_t)pos[c.j0 + r] * pitch, (size_t)pitch);
+            });
+        }
+        for (int f = 0; f < n_folds; ++f)
+            std::memcpy(dst + c.o_beta + sizeof(double) * (size_t)f * c.rows, beta + (size_t)f * n_scored + c.j0, sizeof(double) * (size_t)c.rows);
+        if (flip) std::memcpy(dst + c.o_flip, flip + c.j0, (size_t)c.rows);
+    };
+    for (int64_t k = 0; k < std::min<int64_t>(2, n_chunks); ++k) gather(k);
+    for (int64_t k = 0; k < n_chunks; ++k) {
+        const ChunkLayout c = layout_of(k);
+        const int p = (int)(k % 3), d = (int)(k % 2);
+        cudaEvent_t* ev = h->ev_chunk.data() + 4 * k;
+        pool.wait(groups[p]);
+        uint8_t* dev = (uint8_t*)h->s_dev[d].p;
+        if (k >= 2) CU_TRY(h, cudaStreamWaitEvent(cp, h->ev_slot_free[d], 0));          // the kernels of chunk k - 2 are done with it
+        CU_TRY(h, cudaEventRecord(ev[0], cp));
+        CU_TRY(h, cudaMemcpyAsync(dev, h->s_pin[p].p, c.bytes, cudaMemcpyHostToDevice, cp));
+        CU_TRY(h, cudaEventRecord(ev[1], cp));
+        CU_TRY(h, cudaEventRecord(h->ev_pin_free[p], cp));
+        CU_TRY(h, cudaEventRecord(h->ev_copied[d], cp));
+        CU_TRY(h, cudaStreamWaitEvent(st, h->ev_copied[d], 0));
+        CU_TRY(h, cudaEventRecord(ev[2], st));
+        SnpStat* stats = (SnpStat*)(w + o_stats);
+        const uint8_t* cflip = flip ? dev + c.o_flip : nullptr;
+        const int32_t n_slices = prs_slices(h->n_sm, n_val, c.rows);
+        CU_TRY(h, launch_chunk_stats(dev, c.rows, n_val, stats, n_empty, h->n_sm, st));
+        if (counts) CU_TRY(h, launch_score_counts(dev, n_val, cflip, c.rows, n_slices, cnt, cnt2, st));
+        for (int f0 = 0; f0 < n_folds; f0 += 3)
+            CU_TRY(h, launch_prs_chunk(dev, n_val, stats, cflip, (const double*)(dev + c.o_beta) + (size_t)f0 * c.rows, c.rows, c.rows,
+                                       std::min(3, n_folds - f0), n_slices, (double*)(w + o_part), scores + (size_t)f0 * n_val, st));
+        CU_TRY(h, cudaEventRecord(ev[3], st));
+        CU_TRY(h, cudaEventRecord(h->ev_slot_free[d], st));
+        if (k + 2 < n_chunks) {
+            if (k + 2 >= 3) CU_TRY(h, cudaEventSynchronize(h->ev_pin_free[(k + 2) % 3]));    // the copy of chunk k - 1 has left it
+            gather(k + 2);
+        }
+    }
+    CU_TRY(h, cudaMemcpyAsync(scores_out, scores, sizeof(double) * (size_t)n_folds * n_val, cudaMemcpyDeviceToHost, st));
+    if (cnt_out) CU_TRY(h, cudaMemcpyAsync(cnt_out, cnt, sizeof(int32_t) * (size_t)n_val, cudaMemcpyDeviceToHost, st));
+    if (cnt2_out) CU_TRY(h, cudaMemcpyAsync(cnt2_out, cnt2, sizeof(int32_t) * (size_t)n_val, cudaMemcpyDeviceToHost, st));
+    if (n_empty_out) CU_TRY(h, cudaMemcpyAsync(n_empty_out, n_empty, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CU_TRY(h, cudaStreamSynchronize(st));
+    float kms = 0.0f;
+    for (int64_t k = 0; k < n_chunks; ++k) {
+        const cudaEvent_t* ev = h->ev_chunk.data() + 4 * k;
+        float t = 0.0f;
+        CU_TRY(h, cudaEventElapsedTime(&t, ev[2], ev[3]));
+        kms += t;
+        if (tr.on) {
+            // per-chunk timeline relative to the first copy: does the chunk's kernel time hide behind the next copy?
+            float c0 = 0, c1 = 0, k0 = 0, k1 = 0;
+            cudaEventElapsedTime(&c0, h->ev_chunk[0], ev[0]); cudaEventElapsedTime(&c1, h->ev_chunk[0], ev[1]);
+            cudaEventElapsedTime(&k0, h->ev_chunk[0], ev[2]); cudaEventElapsedTime(&k1, h->ev_chunk[0], ev[3]);
+            std::fprintf(stderr, "[dbslmm_b200 trace] score_stream chunk %lld rows %d bytes %zu copy %.4f %.4f kernels %.4f %.4f ms\n",
+                         (long long)k, layout_of(k).rows, layout_of(k).bytes, c0, c1, k0, k1);
+        }
+    }
+    if (kernel_ms_out) *kernel_ms_out = kms;
     return DBSLMM_B200_OK;
 }
 

@@ -100,6 +100,21 @@ cudaError_t launch_quadform(const BlockDesc* blocks, int32_t n_blocks, const dou
 cudaError_t launch_prs(const uint8_t* bed, int32_t n_val, const SnpStat* stats, const int32_t* pos, const uint8_t* flip,
                        const double* beta, int64_t beta_stride, int32_t n_scored, int32_t nf, int32_t n_chunks,
                        double* partial, double* scores, cudaStream_t st);
+// the streaming path: a compact chunk (row k = scored SNP j0 + k, pitch ceil(n_val / 4)) with its own row statistics, flip
+// and beta slices (beta[f * beta_stride + k]); adds into scores[nf][n_val]
+cudaError_t launch_prs_chunk(const uint8_t* chunk, int32_t n_val, const SnpStat* stats, const uint8_t* flip, const double* beta,
+                             int64_t beta_stride, int32_t n_rows, int32_t nf, int32_t n_slices, double* partial, double* scores,
+                             cudaStream_t st);
+// row slices of one scoring launch over n_rows rows (the grid's y extent; partial holds n_slices * nf * n_val doubles)
+int32_t prs_slices(int n_sm, int32_t n_val, int64_t n_rows);
+// per-row statistics of a compact chunk, any n_val <= kScoreMaxNVal (no shared-memory staging); *n_empty (or NULL) += rows
+// without a called genotype
+constexpr int32_t kScoreMaxNVal = 536870911;     // INT32_MAX / 4: the int32 sum of squares of a row
+cudaError_t launch_chunk_stats(const uint8_t* chunk, int32_t n_rows, int32_t n_val, SnpStat* stats, int32_t* n_empty, int n_sm,
+                               cudaStream_t st);
+// cnt[i] += 2 x called genotypes, cnt2[i] += copies of the scored allele, over the chunk's rows
+cudaError_t launch_score_counts(const uint8_t* chunk, int32_t n_val, const uint8_t* flip, int32_t n_rows, int32_t n_slices,
+                                int32_t* cnt, int32_t* cnt2, cudaStream_t st);
 
 // pcg.cu
 struct PcgArgs {

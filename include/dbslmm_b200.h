@@ -188,6 +188,29 @@ DBSLMM_B200_API int  dbslmm_b200_score(dbslmm_b200_handle* h, const uint8_t* bed
                        const int32_t* pos, const uint8_t* flip, int64_t n_scored,
                        const double* beta, int32_t n_folds, double* scores_out, float* kernel_ms_out);
 
+/* Polygenic scores over a target panel of any size, streamed through the GPU: the `plink --bfile <target> --score <eff>.txt
+ * 1 2 4 sum` of DBSLMM_script.sh:87 for every fold in one pass.  Same semantics as dbslmm_b200_score (mean imputation from
+ * the row's called genotypes, flip[j] != 0 scores A2), plus PLINK's .profile counts:
+ *   cnt_out[i]  = 2 x the genotypes of individual i called on the scored rows  (CNT),
+ *   cnt2_out[i] = copies of the scored allele among them                      (CNT2);
+ * either may be NULL.  A row without a called genotype adds nothing to scores, CNT or CNT2; n_empty_rows_out (or NULL)
+ * receives the number of such scored rows.
+ * `bed_val` is the SNP-major payload (after the magic bytes) in ORDINARY host memory -- an mmap of the .bed is fine -- and
+ * only the rows named by pos are read (pos may be unsorted and may repeat).  The call gathers the scored rows chunk by
+ * chunk into pinned staging buffers on the host worker pool and copies each chunk (rows, beta and flip slices) with one
+ * asynchronous copy; gather, copy and kernels of consecutive chunks overlap.  A chunk holds
+ *   R = max(1, floor(chunk_bytes / (ceil(n_val / 4) + 1)))
+ * scored rows (chunk_bytes = 0: 64 MB), i.e. R x (ceil(n_val / 4) + 1 + 8 n_folds) bytes with their beta slices.  Device and
+ * pinned memory are five such chunks plus O(n_val x n_folds), whatever n_snp_val.  R does not depend on n_folds, so fold f of
+ * an F-fold call is bit-identical to the 1-fold call with beta[f].
+ * Deterministic: the same arguments give the same bits; when one chunk holds every scored row the scores are bit-identical
+ * to dbslmm_b200_score.  Limits: n_val <= 536,870,911 (int32 row sums), n_scored <= INT32_MAX / 2 (CNT in int32).
+ * kernel_ms_out (or NULL): the summed device time of the chunks' kernels.  Synchronous. */
+DBSLMM_B200_API int  dbslmm_b200_score_stream(dbslmm_b200_handle* h, const uint8_t* bed_val, int64_t n_snp_val, int32_t n_val,
+                              const int32_t* pos, const uint8_t* flip, int64_t n_scored, const double* beta, int32_t n_folds,
+                              uint64_t chunk_bytes, double* scores_out, int32_t* cnt_out, int32_t* cnt2_out,
+                              int32_t* n_empty_rows_out, float* kernel_ms_out);
+
 /* ---- inspection hooks used by the parity tests (operate on the state of the last fit) ---- */
 /* int8 codes of one decoded row of the last fit: SNP j of block `block` (its small SNPs first, then its large ones),
  * plane 0 = allele counts (missing -> 0), plane 1 = call mask (1 = called; holds the last mask written at that position,
