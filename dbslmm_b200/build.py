@@ -1,6 +1,6 @@
 """In-tree build of the sm_100a library and the `dbslmm` CLI (explicit nvcc / g++ calls).
 
-    python -m dbslmm_b200.build            # libdbslmm_b200.so + build/dbslmm, build/valid, build/score
+    python -m dbslmm_b200.build            # libdbslmm_b200.so + build/dbslmm, build/valid, build/score, build/ldscore
 Outputs stay inside the repo (git-ignored) so they travel with a gpurun snapshot.
 """
 import concurrent.futures as cf
@@ -17,13 +17,14 @@ LIB = os.path.join(PKG, "libdbslmm_b200.so")
 CLI = os.path.join(BUILD, "dbslmm")
 VALID_CLI = os.path.join(BUILD, "valid")
 SCORE_CLI = os.path.join(BUILD, "score")
+LDSCORE_CLI = os.path.join(BUILD, "ldscore")
 
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 GXX = "/usr/bin/g++"
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 CU_FLAGS = ["-O3", "-lineinfo", "-std=c++17", "-ccbin", GXX, "-Xcompiler", "-fPIC,-fvisibility=hidden",
             "-Xptxas", "-v"]
-CU_SOURCES = ["decode.cu", "gram.cu", "chol.cu", "score.cu", "variance.cu", "pcg.cu", "engine.cu"]
+CU_SOURCES = ["decode.cu", "gram.cu", "chol.cu", "score.cu", "variance.cu", "pcg.cu", "ldscore.cu", "engine.cu"]
 HOST_SOURCES = ["dbslmm_main.cpp", "ingest.cpp"]
 
 
@@ -80,9 +81,15 @@ def build_cli(force=False):
              ["-L", PKG, "-ldbslmm_b200", "-Wl,-rpath,$ORIGIN/../dbslmm_b200", "-Wl,-rpath," + PKG])
     # `score`: plink --score <eff>.txt 1 2 4 sum over a target fileset (DBSLMM_script.sh:87), every fold in one pass
     ssrc = os.path.join(HOST, "score_main.cpp")
-    if os.path.exists(ssrc) and (force or _newer(SCORE_CLI, [ssrc] + deps)):
+    if os.path.exists(ssrc) and (force or _newer(SCORE_CLI, [ssrc, os.path.join(HOST, "plink_bed.hpp")] + deps)):
         _run([GXX, "-O2", "-std=c++17", "-pthread", "-I", os.path.join(ROOT, "include"), "-o", SCORE_CLI, ssrc] +
              ["-L", PKG, "-ldbslmm_b200", "-Wl,-rpath,$ORIGIN/../dbslmm_b200", "-Wl,-rpath," + PKG])
+    # `ldscore`: ldsc.py --bfile <panel> --l2 (LD Scores of the reference panel, the input of LDSC's -h / -nsnp)
+    lsrc = os.path.join(HOST, "ldscore_main.cpp")
+    ldeps = [lsrc, os.path.join(HOST, "plink_bed.hpp")] + deps
+    if os.path.exists(lsrc) and (force or _newer(LDSCORE_CLI, ldeps)):
+        _run([GXX, "-O2", "-std=c++17", "-pthread", "-I", os.path.join(ROOT, "include"), "-o", LDSCORE_CLI, lsrc] +
+             ["-L", PKG, "-ldbslmm_b200", "-Wl,-rpath,$ORIGIN/../dbslmm_b200", "-Wl,-rpath," + PKG, "-lz"])
     return CLI
 
 

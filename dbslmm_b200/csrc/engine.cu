@@ -198,6 +198,8 @@ struct dbslmm_b200_handle {
     // streaming scorer (dbslmm_b200_score_stream): pinned staging ring, device chunk slots, per-call work buffer
     PinBuf s_pin[3];
     DevBuf s_dev[2], s_work;
+    // LD scores (dbslmm_b200_ldscore): row statistics, segment code rows + dirty map, decoder scratch, partial slots, reduction
+    DevBuf ld_stats, ld_codes, ld_dirty, ld_work, ld_slots, ld_red;
     cudaEvent_t ev_pin_free[3] = {}, ev_copied[2] = {}, ev_slot_free[2] = {};
     std::vector<cudaEvent_t> ev_chunk;   // 4 timing events per chunk (copy begin / end, kernels begin / end), grow-only
     size_t dirty_rows = 0;               // code rows the dirty map covers
@@ -981,6 +983,7 @@ void dbslmm_b200_destroy(dbslmm_b200_handle* h) {
     for (PinBuf& b : h->s_pin) b.release();
     for (DevBuf& b : h->s_dev) b.release();
     h->s_work.release();
+    for (DevBuf* b : {&h->ld_stats, &h->ld_codes, &h->ld_dirty, &h->ld_work, &h->ld_slots, &h->ld_red}) b->release();
     for (cudaEvent_t e : h->ev_pin_free) if (e) cudaEventDestroy(e);
     for (int i = 0; i < 2; ++i) {
         if (h->ev_copied[i]) cudaEventDestroy(h->ev_copied[i]);
@@ -2115,6 +2118,81 @@ static ChunkLayout chunk_layout(int64_t j0, int32_t rows, int64_t pitch, int32_t
     return c;
 }
 
+}  // extern "C"
+
+// The host gather ring of the streaming calls (dbslmm_b200_score_stream, dbslmm_b200_ldscore).  Chunk k is gathered by the
+// host worker pool into pinned staging slot k % 3 and crosses PCIe in ONE cudaMemcpyAsync on the copy stream into device
+// slot k % 2; its kernels run on the main stream.  The gather of chunk k + 2, the copy of chunk k + 1 and the kernels of
+// chunk k overlap.  gather(k, dst, group) fills staging slot dst (pieces may go to the pool under `group`); launch(k, dev)
+// enqueues the kernels of chunk k, whose bytes are at `dev`, on h->stream.  Events ev_chunk[4 (ev0 + k) + 0..3] record the
+// begin and end of the chunk's copy and kernels.  Returns with the work enqueued; the caller synchronises h->stream.
+template <class BytesOf, class Gather, class Launch>
+static int stream_chunks(dbslmm_b200_handle* h, int64_t n_chunks, size_t max_bytes, int64_t ev0, BytesOf bytes_of, Gather gather,
+                         Launch launch) {
+    cudaStream_t st = h->stream, cp = h->up_stream;
+    const int n_pin = (int)std::min<int64_t>(3, std::max<int64_t>(n_chunks, 1)), n_dev = std::min(2, n_pin);
+    for (int i = 0; i < n_pin; ++i) CU_TRY(h, h->s_pin[i].ensure(max_bytes));
+    for (int i = 0; i < n_dev; ++i) CU_TRY(h, h->s_dev[i].ensure(max_bytes));
+    while (h->ev_chunk.size() < (size_t)(4 * (ev0 + n_chunks))) {
+        cudaEvent_t e;
+        CU_TRY(h, cudaEventCreate(&e));
+        h->ev_chunk.push_back(e);
+    }
+    HostPool& pool = host_pool();
+    TaskGroup groups[3];
+    struct Drain { HostPool& p; TaskGroup* g; ~Drain() { for (int i = 0; i < 3; ++i) p.wait(g[i]); } } drain{pool, groups};
+    for (int64_t k = 0; k < std::min<int64_t>(2, n_chunks); ++k) gather(k, (uint8_t*)h->s_pin[k % 3].p, groups[k % 3]);
+    for (int64_t k = 0; k < n_chunks; ++k) {
+        const int p = (int)(k % 3), d = (int)(k % 2);
+        cudaEvent_t* ev = h->ev_chunk.data() + 4 * (ev0 + k);
+        pool.wait(groups[p]);
+        uint8_t* dev = (uint8_t*)h->s_dev[d].p;
+        if (k >= 2) CU_TRY(h, cudaStreamWaitEvent(cp, h->ev_slot_free[d], 0));          // the kernels of chunk k - 2 are done with it
+        CU_TRY(h, cudaEventRecord(ev[0], cp));
+        CU_TRY(h, cudaMemcpyAsync(dev, h->s_pin[p].p, bytes_of(k), cudaMemcpyHostToDevice, cp));
+        CU_TRY(h, cudaEventRecord(ev[1], cp));
+        CU_TRY(h, cudaEventRecord(h->ev_pin_free[p], cp));
+        CU_TRY(h, cudaEventRecord(h->ev_copied[d], cp));
+        CU_TRY(h, cudaStreamWaitEvent(st, h->ev_copied[d], 0));
+        CU_TRY(h, cudaEventRecord(ev[2], st));
+        const int rc = launch(k, (const uint8_t*)dev);
+        if (rc != DBSLMM_B200_OK) return rc;
+        CU_TRY(h, cudaEventRecord(ev[3], st));
+        CU_TRY(h, cudaEventRecord(h->ev_slot_free[d], st));
+        if (k + 2 < n_chunks) {
+            if (k + 2 >= 3) CU_TRY(h, cudaEventSynchronize(h->ev_pin_free[(k + 2) % 3]));    // the copy of chunk k - 1 has left it
+            gather(k + 2, (uint8_t*)h->s_pin[(k + 2) % 3].p, groups[(k + 2) % 3]);
+        }
+    }
+    return DBSLMM_B200_OK;
+}
+
+// Summed kernel time of the chunks [ev0, ev0 + n) of stream_chunks, once h->stream has been synchronised.  With
+// DBSLMM_B200_TRACE, one line per chunk: its copy and kernel intervals relative to the call's first copy (do the kernels
+// hide behind the next copy?).
+template <class RowsOf, class BytesOf>
+static int chunk_kernel_ms(dbslmm_b200_handle* h, const char* label, int64_t ev0, int64_t n, RowsOf rows_of, BytesOf bytes_of, float* out) {
+    const Trace tr;
+    float kms = 0.0f;
+    for (int64_t k = 0; k < n; ++k) {
+        const cudaEvent_t* ev = h->ev_chunk.data() + 4 * (ev0 + k);
+        float t = 0.0f;
+        CU_TRY(h, cudaEventElapsedTime(&t, ev[2], ev[3]));
+        kms += t;
+        if (tr.on) {
+            float c0 = 0, c1 = 0, k0 = 0, k1 = 0;
+            cudaEventElapsedTime(&c0, h->ev_chunk[0], ev[0]); cudaEventElapsedTime(&c1, h->ev_chunk[0], ev[1]);
+            cudaEventElapsedTime(&k0, h->ev_chunk[0], ev[2]); cudaEventElapsedTime(&k1, h->ev_chunk[0], ev[3]);
+            std::fprintf(stderr, "[dbslmm_b200 trace] %s chunk %lld rows %lld bytes %zu copy %.4f %.4f kernels %.4f %.4f ms\n", label,
+                         (long long)k, (long long)rows_of(k), (size_t)bytes_of(k), c0, c1, k0, k1);
+        }
+    }
+    *out = kms;
+    return DBSLMM_B200_OK;
+}
+
+extern "C" {
+
 int dbslmm_b200_score_stream(dbslmm_b200_handle* h, const uint8_t* bed_val, int64_t n_snp_val, int32_t n_val,
                              const int32_t* pos, const uint8_t* flip, int64_t n_scored, const double* beta, int32_t n_folds,
                              uint64_t chunk_bytes, double* scores_out, int32_t* cnt_out, int32_t* cnt2_out, int32_t* n_empty_out,
@@ -2129,8 +2207,7 @@ int dbslmm_b200_score_stream(dbslmm_b200_handle* h, const uint8_t* bed_val, int6
     for (int64_t j = 0; j < n_scored; ++j)
         if (pos[j] < 0 || pos[j] >= n_snp_val) return fail(h, DBSLMM_B200_ERR_ARG, "score_stream: pos out of range of the .bed");
     CU_TRY(h, cudaSetDevice(h->device));
-    const Trace tr;
-    cudaStream_t st = h->stream, cp = h->up_stream;
+    cudaStream_t st = h->stream;
     const int64_t pitch = (n_val + 3) / 4;
     const bool counts = cnt_out || cnt2_out;
     const uint64_t budget = chunk_bytes ? chunk_bytes : kStreamChunkDefault;
@@ -2147,15 +2224,7 @@ int dbslmm_b200_score_stream(dbslmm_b200_handle* h, const uint8_t* bed_val, int6
                  o_sc = place(sizeof(double) * (size_t)n_folds * n_val),
                  o_cnt = place(sizeof(int32_t) * (size_t)n_val), o_cnt2 = place(sizeof(int32_t) * (size_t)n_val),
                  o_empty = place(sizeof(int32_t));
-    const int n_pin = (int)std::min<int64_t>(3, std::max<int64_t>(n_chunks, 1)), n_dev = std::min(2, n_pin);
-    for (int i = 0; i < n_pin; ++i) CU_TRY(h, h->s_pin[i].ensure(full.bytes));
-    for (int i = 0; i < n_dev; ++i) CU_TRY(h, h->s_dev[i].ensure(full.bytes));
     CU_TRY(h, h->s_work.ensure(o));
-    while (h->ev_chunk.size() < (size_t)(4 * n_chunks)) {
-        cudaEvent_t e;
-        CU_TRY(h, cudaEventCreate(&e));
-        h->ev_chunk.push_back(e);
-    }
     uint8_t* w = (uint8_t*)h->s_work.p;
     double* scores = (double*)(w + o_sc);
     int32_t* cnt = (int32_t*)(w + o_cnt);
@@ -2164,18 +2233,15 @@ int dbslmm_b200_score_stream(dbslmm_b200_handle* h, const uint8_t* bed_val, int6
     CU_TRY(h, cudaMemsetAsync(scores, 0, sizeof(double) * (size_t)n_folds * n_val, st));
     CU_TRY(h, cudaMemsetAsync(cnt, 0, o - o_cnt, st));
 
-    // host gather of chunk k into staging slot k % 3, cut into pieces of >= 2 MB for the pool's workers
+    // host gather of chunk k, cut into pieces of >= 2 MB for the pool's workers
     HostPool& pool = host_pool();
-    TaskGroup groups[3];
-    struct Drain { HostPool& p; TaskGroup* g; ~Drain() { for (int i = 0; i < 3; ++i) p.wait(g[i]); } } drain{pool, groups};
     auto layout_of = [&](int64_t k) { const int64_t j0 = k * rows_cap; return chunk_layout(j0, (int32_t)std::min(rows_cap, n_scored - j0), pitch, n_folds); };
-    auto gather = [&](int64_t k) {
+    auto gather = [&](int64_t k, uint8_t* dst, TaskGroup& g) {
         const ChunkLayout c = layout_of(k);
-        uint8_t* dst = (uint8_t*)h->s_pin[k % 3].p;
         const int64_t per = std::max<int64_t>(1, ((int64_t)2 << 20) / pitch);
         for (int64_t r0 = 0; r0 < c.rows; r0 += per) {
             const int64_t r1 = std::min<int64_t>(c.rows, r0 + per);
-            pool.submit(groups[k % 3], [=]() {
+            pool.submit(g, [=]() {
                 for (int64_t r = r0; r < r1; ++r) std::memcpy(dst + r * pitch, bed_val + (int64_t)pos[c.j0 + r] * pitch, (size_t)pitch);
             });
         }
@@ -2183,21 +2249,8 @@ int dbslmm_b200_score_stream(dbslmm_b200_handle* h, const uint8_t* bed_val, int6
             std::memcpy(dst + c.o_beta + sizeof(double) * (size_t)f * c.rows, beta + (size_t)f * n_scored + c.j0, sizeof(double) * (size_t)c.rows);
         if (flip) std::memcpy(dst + c.o_flip, flip + c.j0, (size_t)c.rows);
     };
-    for (int64_t k = 0; k < std::min<int64_t>(2, n_chunks); ++k) gather(k);
-    for (int64_t k = 0; k < n_chunks; ++k) {
+    auto launch = [&](int64_t k, const uint8_t* dev) -> int {
         const ChunkLayout c = layout_of(k);
-        const int p = (int)(k % 3), d = (int)(k % 2);
-        cudaEvent_t* ev = h->ev_chunk.data() + 4 * k;
-        pool.wait(groups[p]);
-        uint8_t* dev = (uint8_t*)h->s_dev[d].p;
-        if (k >= 2) CU_TRY(h, cudaStreamWaitEvent(cp, h->ev_slot_free[d], 0));          // the kernels of chunk k - 2 are done with it
-        CU_TRY(h, cudaEventRecord(ev[0], cp));
-        CU_TRY(h, cudaMemcpyAsync(dev, h->s_pin[p].p, c.bytes, cudaMemcpyHostToDevice, cp));
-        CU_TRY(h, cudaEventRecord(ev[1], cp));
-        CU_TRY(h, cudaEventRecord(h->ev_pin_free[p], cp));
-        CU_TRY(h, cudaEventRecord(h->ev_copied[d], cp));
-        CU_TRY(h, cudaStreamWaitEvent(st, h->ev_copied[d], 0));
-        CU_TRY(h, cudaEventRecord(ev[2], st));
         SnpStat* stats = (SnpStat*)(w + o_stats);
         const uint8_t* cflip = flip ? dev + c.o_flip : nullptr;
         const int32_t n_slices = prs_slices(h->n_sm, n_val, c.rows);
@@ -2206,34 +2259,310 @@ int dbslmm_b200_score_stream(dbslmm_b200_handle* h, const uint8_t* bed_val, int6
         for (int f0 = 0; f0 < n_folds; f0 += 3)
             CU_TRY(h, launch_prs_chunk(dev, n_val, stats, cflip, (const double*)(dev + c.o_beta) + (size_t)f0 * c.rows, c.rows, c.rows,
                                        std::min(3, n_folds - f0), n_slices, (double*)(w + o_part), scores + (size_t)f0 * n_val, st));
-        CU_TRY(h, cudaEventRecord(ev[3], st));
-        CU_TRY(h, cudaEventRecord(h->ev_slot_free[d], st));
-        if (k + 2 < n_chunks) {
-            if (k + 2 >= 3) CU_TRY(h, cudaEventSynchronize(h->ev_pin_free[(k + 2) % 3]));    // the copy of chunk k - 1 has left it
-            gather(k + 2);
-        }
-    }
+        return DBSLMM_B200_OK;
+    };
+    int rc = stream_chunks(h, n_chunks, full.bytes, 0, [&](int64_t k) { return layout_of(k).bytes; }, gather, launch);
+    if (rc != DBSLMM_B200_OK) return rc;
     CU_TRY(h, cudaMemcpyAsync(scores_out, scores, sizeof(double) * (size_t)n_folds * n_val, cudaMemcpyDeviceToHost, st));
     if (cnt_out) CU_TRY(h, cudaMemcpyAsync(cnt_out, cnt, sizeof(int32_t) * (size_t)n_val, cudaMemcpyDeviceToHost, st));
     if (cnt2_out) CU_TRY(h, cudaMemcpyAsync(cnt2_out, cnt2, sizeof(int32_t) * (size_t)n_val, cudaMemcpyDeviceToHost, st));
     if (n_empty_out) CU_TRY(h, cudaMemcpyAsync(n_empty_out, n_empty, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     CU_TRY(h, cudaStreamSynchronize(st));
     float kms = 0.0f;
-    for (int64_t k = 0; k < n_chunks; ++k) {
-        const cudaEvent_t* ev = h->ev_chunk.data() + 4 * k;
-        float t = 0.0f;
-        CU_TRY(h, cudaEventElapsedTime(&t, ev[2], ev[3]));
-        kms += t;
-        if (tr.on) {
-            // per-chunk timeline relative to the first copy: does the chunk's kernel time hide behind the next copy?
-            float c0 = 0, c1 = 0, k0 = 0, k1 = 0;
-            cudaEventElapsedTime(&c0, h->ev_chunk[0], ev[0]); cudaEventElapsedTime(&c1, h->ev_chunk[0], ev[1]);
-            cudaEventElapsedTime(&k0, h->ev_chunk[0], ev[2]); cudaEventElapsedTime(&k1, h->ev_chunk[0], ev[3]);
-            std::fprintf(stderr, "[dbslmm_b200 trace] score_stream chunk %lld rows %d bytes %zu copy %.4f %.4f kernels %.4f %.4f ms\n",
-                         (long long)k, layout_of(k).rows, layout_of(k).bytes, c0, c1, k0, k1);
+    rc = chunk_kernel_ms(h, "score_stream", 0, n_chunks, [&](int64_t k) { return (int64_t)layout_of(k).rows; },
+                         [&](int64_t k) { return layout_of(k).bytes; }, &kms);
+    if (rc != DBSLMM_B200_OK) return rc;
+    if (kernel_ms_out) *kernel_ms_out = kms;
+    return DBSLMM_B200_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// LD Scores (ldsc --l2), see ldscore.cu.  Pass 1 streams the requested rows through launch_chunk_stats, and the host keeps
+// ldsc's SNPs, builds the windows over the kept SNPs of every chromosome, the band of 128 x 128 tiles and the slot layout.
+// Pass 2 streams segments of consecutive row tiles together with the halo of rows their windows reach (decode -> group
+// flags -> band kernels, one chunk per segment); ld_reduce_kernel then adds each SNP's slots.
+// ---------------------------------------------------------------------------------------------
+namespace {
+struct LdSeg {
+    int64_t T0 = 0, T1 = 0;           // row tiles [T0, T1)
+    int64_t R0 = 0, R1 = 0;           // padded rows on the device: [128 T0, 128 (last tile column reached + 1))
+    int64_t K0 = 0, K1 = 0;           // kept SNPs among them
+    int64_t n_tiles = 0;
+    size_t o_src = 0, o_crow = 0, o_mrow = 0, o_rows = 0, o_tiles = 0, bytes = 0;
+};
+}  // namespace
+
+int dbslmm_b200_ld_windows(const double* coord, int64_t m, double max_dist, int32_t* lo_out, int32_t* hi_out) {
+    if (m < 0 || m > INT32_MAX || (m > 0 && (!lo_out || !hi_out)) || !(max_dist >= 0)) return DBSLMM_B200_ERR_ARG;
+    auto x = [&](int64_t k) { return coord ? coord[k] : (double)k; };
+    int64_t lo = 0, hi = 0;
+    for (int64_t k = 0; k < m; ++k) {
+        while (std::fabs(x(k) - x(lo)) > max_dist) ++lo;                 // ldsc's getBlockLefts
+        hi = std::max(hi, k);
+        while (hi + 1 < m && std::fabs(x(hi + 1) - x(k)) <= max_dist) ++hi;
+        lo_out[k] = (int32_t)lo;
+        hi_out[k] = (int32_t)hi;
+    }
+    return DBSLMM_B200_OK;
+}
+
+int dbslmm_b200_ldscore(dbslmm_b200_handle* h, const uint8_t* bed, int64_t n_snp, int32_t n_ref, const int32_t* rows,
+                        int64_t n_rows, const int32_t* chr_off, int32_t n_chr, int32_t wind_kind, const double* coord,
+                        double max_dist, double maf_min, int64_t segment_rows, uint8_t* kept_out, double* maf_out,
+                        double* l2_out, int32_t* guard_out, float* kernel_ms_out) {
+    if (!h) return DBSLMM_B200_ERR_ARG;
+    auto bad = [&](const std::string& m) { return fail(h, DBSLMM_B200_ERR_ARG, "ldscore: " + m); };
+    if (!bed || n_snp <= 0 || n_ref <= 0 || n_rows < 0 || n_chr < 0 || !chr_off || (n_rows > 0 && !rows))
+        return bad("bad arguments");
+    if (n_ref > decode_max_n_ref())
+        return bad("n_ref = " + std::to_string(n_ref) + " is above the limit of " + std::to_string(decode_max_n_ref()) +
+                   " individuals (the decoder stages whole .bed rows in shared memory)");
+    if (n_rows > INT32_MAX) return bad("n_rows = " + std::to_string(n_rows) + " is above INT32_MAX");
+    if (wind_kind != DBSLMM_B200_LD_WIND_COORD && wind_kind != DBSLMM_B200_LD_WIND_SNPS) return bad("unknown window kind " + std::to_string(wind_kind));
+    if (wind_kind == DBSLMM_B200_LD_WIND_COORD && n_rows > 0 && !coord) return bad("a coordinate window needs coord");
+    if (wind_kind == DBSLMM_B200_LD_WIND_SNPS && coord) return bad("a window in SNPs takes coord = NULL");
+    if (!std::isfinite(max_dist) || max_dist < 0 ||
+        (wind_kind == DBSLMM_B200_LD_WIND_SNPS && (max_dist != std::floor(max_dist) || max_dist > (double)INT32_MAX)))
+        return bad("max_dist must be finite and >= 0 (a whole number for a window in SNPs)");
+    if (!std::isfinite(maf_min) || maf_min < 0 || maf_min >= 0.5) return bad("maf_min must lie in [0, 0.5)");
+    if (segment_rows < 0 || segment_rows % 128 != 0) return bad("segment_rows must be 0 or a positive multiple of 128");
+    if (chr_off[0] != 0 || chr_off[n_chr] != n_rows) return bad("bad chromosome offsets: chr_off[0] must be 0 and chr_off[n_chr] = n_rows");
+    for (int32_t c = 0; c < n_chr; ++c)
+        if (chr_off[c + 1] < chr_off[c]) return bad("bad chromosome offsets: chr_off[" + std::to_string(c + 1) + "] < chr_off[" + std::to_string(c) + "]");
+    for (int64_t i = 0; i < n_rows; ++i)
+        if (rows[i] < 0 || rows[i] >= n_snp) return bad("rows[" + std::to_string(i) + "] = " + std::to_string(rows[i]) + " is out of range of the .bed");
+    if (wind_kind == DBSLMM_B200_LD_WIND_COORD)
+        for (int32_t c = 0; c < n_chr; ++c)
+            for (int64_t i = chr_off[c]; i < chr_off[c + 1]; ++i) {
+                if (!std::isfinite(coord[i])) return bad("coord[" + std::to_string(i) + "] is not finite");
+                if (i > chr_off[c] && coord[i] < coord[i - 1])
+                    return bad("the coordinates of chromosome " + std::to_string(c) + " are not sorted: coord[" + std::to_string(i) + "] < coord[" +
+                               std::to_string(i - 1) + "]");
+            }
+    CU_TRY(h, cudaSetDevice(h->device));
+    cudaStream_t st = h->stream;
+    const int64_t pitch = (n_ref + 3) / 4;
+    const int32_t n_pad = (n_ref + 127) / 128 * 128;
+    HostPool& pool = host_pool();
+    // .bed rows src[0..nr) -> dst (pitch bytes each), in pieces of >= 2 MB for the pool's workers
+    auto gather_rows = [&](uint8_t* dst, const int64_t nr, TaskGroup& g, auto src) {
+        const int64_t per = std::max<int64_t>(1, ((int64_t)2 << 20) / pitch);
+        for (int64_t r0 = 0; r0 < nr; r0 += per) {
+            const int64_t r1 = std::min<int64_t>(nr, r0 + per);
+            pool.submit(g, [=]() { for (int64_t r = r0; r < r1; ++r) std::memcpy(dst + r * pitch, bed + (int64_t)src(r) * pitch, (size_t)pitch); });
+        }
+    };
+
+    // ---- pass 1: per-row statistics of every requested row
+    const int64_t rows1 = std::max<int64_t>(1, std::min<int64_t>(std::max<int64_t>(n_rows, 1), (int64_t)(kStreamChunkDefault / (uint64_t)pitch)));
+    const int64_t n1 = (n_rows + rows1 - 1) / rows1;
+    CU_TRY(h, h->ld_stats.ensure(sizeof(SnpStat) * (size_t)std::max<int64_t>(n_rows, 1)));
+    SnpStat* d_stats = (SnpStat*)h->ld_stats.p;
+    auto rows_of1 = [&](int64_t k) { return std::min<int64_t>(rows1, n_rows - k * rows1); };
+    auto bytes_of1 = [&](int64_t k) { return align_up((size_t)std::max<int64_t>(rows_of1(k), 0) * pitch + 4, 256); };   // + 4: whole-word reads
+    int rc = stream_chunks(h, n1, bytes_of1(0), 0, bytes_of1,
+                           [&](int64_t k, uint8_t* dst, TaskGroup& g) {
+                               const int64_t j0 = k * rows1;
+                               gather_rows(dst, rows_of1(k), g, [=](int64_t r) { return rows[j0 + r]; });
+                           },
+                           [&](int64_t k, const uint8_t* dev) -> int {
+                               CU_TRY(h, launch_chunk_stats(dev, (int32_t)rows_of1(k), n_ref, d_stats + k * rows1, nullptr, h->n_sm, st));
+                               return DBSLMM_B200_OK;
+                           });
+    if (rc != DBSLMM_B200_OK) return rc;
+    std::vector<SnpStat> hs((size_t)n_rows);
+    if (n_rows > 0) CU_TRY(h, cudaMemcpyAsync(hs.data(), d_stats, sizeof(SnpStat) * (size_t)n_rows, cudaMemcpyDeviceToHost, st));
+    CU_TRY(h, cudaStreamSynchronize(st));
+    float ms1 = 0.0f;
+    rc = chunk_kernel_ms(h, "ldscore pass1", 0, n1, rows_of1, bytes_of1, &ms1);
+    if (rc != DBSLMM_B200_OK) return rc;
+
+    // ---- kept SNPs (ldsc's __filter_snps_maf__): min(f, 1 - f) > maf_min and missing + het < n
+    std::vector<uint8_t> keep((size_t)n_rows);
+    for (int64_t i = 0; i < n_rows; ++i) {
+        const SnpStat& s = hs[i];
+        const double f = s.n_nonmiss > 0 ? (double)s.sum / (2.0 * (double)s.n_nonmiss) : 0.0;
+        const double maf = std::min(f, 1.0 - f);
+        const int64_t hom2 = ((int64_t)s.sumsq - s.sum) / 2, het = (int64_t)s.sum - 2 * hom2, miss = (int64_t)n_ref - s.n_nonmiss;
+        keep[i] = (maf > maf_min && miss + het < n_ref) ? 1 : 0;
+        if (maf_out) maf_out[i] = maf;
+        if (kept_out) kept_out[i] = keep[i];
+    }
+    // ---- windows (ldsc's getBlockLefts over the kept SNPs of each chromosome, both ends), tiles and slots.  Chromosome c
+    // takes the padded rows [128 T_c, 128 (T_c + ceil(m_c / 128))); its kept SNP k sits at padded row 128 T_c + k.
+    std::vector<int64_t> kept, kpad, klo, khi;          // per kept SNP: row index, padded row, window (padded rows, inclusive)
+    std::vector<int64_t> tlo, thi, tbase;               // per row tile: tile columns reached, first slot
+    std::vector<int32_t> tnslot;
+    int64_t slots_total = 0;
+    for (int32_t c = 0; c < n_chr; ++c) {
+        const int64_t T_c = (int64_t)tlo.size(), k0 = (int64_t)kept.size();
+        for (int64_t i = chr_off[c]; i < chr_off[c + 1]; ++i) if (keep[i]) kept.push_back(i);
+        const int64_t m = (int64_t)kept.size() - k0;
+        std::vector<double> x;
+        if (wind_kind == DBSLMM_B200_LD_WIND_COORD)
+            for (int64_t k = 0; k < m; ++k) x.push_back(coord[kept[k0 + k]]);
+        std::vector<int32_t> lo((size_t)m), hi((size_t)m);
+        dbslmm_b200_ld_windows(x.empty() ? nullptr : x.data(), m, max_dist, lo.data(), hi.data());
+        for (int64_t k = 0; k < m; ++k) {
+            kpad.push_back(128 * T_c + k);
+            klo.push_back(128 * T_c + lo[k]);
+            khi.push_back(128 * T_c + hi[k]);
+        }
+        if (guard_out) guard_out[c] = (m > 0 && klo.back() == 128 * T_c) ? 1 : 0;
+        for (int64_t t = 0; t < (m + 127) / 128; ++t) {
+            tlo.push_back(klo[k0 + 128 * t] / 128);
+            thi.push_back(khi[k0 + std::min(m, 128 * t + 128) - 1] / 128);
+            tnslot.push_back((int32_t)(thi.back() - tlo.back() + 1));
+            tbase.push_back(slots_total);
+            slots_total += 128 * (int64_t)tnslot.back();
         }
     }
-    if (kernel_ms_out) *kernel_ms_out = kms;
+    const int64_t n_trows = (int64_t)tlo.size(), n_prows = 128 * n_trows, n_kept = (int64_t)kept.size();
+    if (l2_out)
+        for (int64_t i = 0; i < n_rows; ++i) l2_out[i] = std::nan("");
+    if (n_kept == 0 || !l2_out) {                       // (l2_out NULL: the statistics pass only)
+        if (kernel_ms_out) *kernel_ms_out = ms1;
+        return DBSLMM_B200_OK;
+    }
+
+    // ---- segments: consecutive row tiles; nonzero segment_rows fixes their size, else 64 MB of .bed rows while the code rows
+    // of the widest segment (with its halo) take at most half of the free device memory
+    auto plan = [&](int64_t seg_tiles, std::vector<LdSeg>& segs) {
+        segs.clear();
+        int64_t cap = 0;
+        for (int64_t T0 = 0; T0 < n_trows; T0 += seg_tiles) {
+            LdSeg S;
+            S.T0 = T0;
+            S.T1 = std::min(n_trows, T0 + seg_tiles);
+            S.R0 = 128 * S.T0;
+            S.R1 = 128 * (thi[S.T1 - 1] + 1);
+            S.K0 = std::lower_bound(kpad.begin(), kpad.end(), S.R0) - kpad.begin();
+            S.K1 = std::lower_bound(kpad.begin(), kpad.end(), S.R1) - kpad.begin();
+            for (int64_t T = S.T0; T < S.T1; ++T) S.n_tiles += thi[T] - T + 1;
+            const int64_t nr = S.K1 - S.K0, np = S.R1 - S.R0;
+            S.o_src = align_up((size_t)nr * pitch + 16, 256);        // + 16: the decoder's row copies are 16-byte aligned
+            S.o_crow = align_up(S.o_src + sizeof(uint32_t) * nr, 256);
+            S.o_mrow = align_up(S.o_crow + sizeof(int32_t) * nr, 256);
+            S.o_rows = align_up(S.o_mrow + sizeof(int32_t) * nr, 256);
+            S.o_tiles = align_up(S.o_rows + sizeof(LdRow) * np, 256);
+            S.bytes = align_up(S.o_tiles + sizeof(LdTile) * S.n_tiles, 256);
+            cap = std::max(cap, np);
+            segs.push_back(S);
+        }
+        return cap;
+    };
+    std::vector<LdSeg> segs;
+    int64_t seg_tiles = segment_rows > 0 ? segment_rows / 128 : std::max<int64_t>(1, (int64_t)(kStreamChunkDefault / (uint64_t)(128 * pitch)));
+    int64_t cap = plan(seg_tiles, segs);
+    size_t free_b = 0, total_b = 0;
+    CU_TRY(h, cudaMemGetInfo(&free_b, &total_b));
+    auto need = [&](int64_t cp) { return (double)cp * (2.0 * n_pad + 2.0 + 48.0); };
+    if (segment_rows == 0)
+        while (seg_tiles > 1 && need(cap) > 0.5 * (double)free_b) cap = plan(seg_tiles = (seg_tiles + 1) / 2, segs);
+    if (need(cap) + 8.0 * (double)slots_total > 0.9 * (double)free_b)
+        return fail(h, DBSLMM_B200_ERR_NOMEM, "ldscore: a segment of " + std::to_string(cap) + " rows (with the halo its windows reach) and " +
+                                             std::to_string(slots_total) + " partial sums do not fit in device memory");
+    size_t max_bytes = 0;
+    for (const LdSeg& S : segs) max_bytes = std::max(max_bytes, S.bytes);
+
+    // ---- device buffers of pass 2: code rows [genotype rows 0..cap) [mask rows cap..2 cap), the decoder's dirty map (all
+    // ones: every mask row is written the first time its position is used), its per-row outputs, group flags, slots
+    CU_TRY(h, h->ld_codes.ensure((size_t)2 * cap * n_pad));
+    CU_TRY(h, h->ld_dirty.ensure((size_t)2 * cap));
+    CU_TRY(h, cudaMemsetAsync(h->ld_dirty.p, 1, (size_t)2 * cap, st));
+    size_t o = 0;
+    auto place = [&](size_t b) { size_t r = o; o = align_up(o + b, 256); return r; };
+    const size_t o_rowN = place(sizeof(int32_t) * cap), o_rowS = place(sizeof(int32_t) * cap), o_rowR = place(sizeof(double) * cap),
+                 o_rowC = place(sizeof(double2) * cap), o_gfl = place(sizeof(int32_t) * (cap / 128 + 1));
+    CU_TRY(h, h->ld_work.ensure(o));
+    uint8_t* wk = (uint8_t*)h->ld_work.p;
+    int32_t* rowN = (int32_t*)(wk + o_rowN);
+    int32_t* gflags = (int32_t*)(wk + o_gfl);
+    CU_TRY(h, h->ld_slots.ensure(sizeof(double) * (size_t)slots_total));
+    double* slots = (double*)h->ld_slots.p;
+    CU_TRY(h, cudaMemsetAsync(slots, 0, sizeof(double) * (size_t)slots_total, st));
+    CUtensorMap tmap;
+    rc = make_tensor_map(h, &tmap, h->ld_codes.p, 2 * cap, n_pad, 128);
+    if (rc != DBSLMM_B200_OK) return rc;
+
+    auto gather2 = [&](int64_t k, uint8_t* dst, TaskGroup& g) {
+        const LdSeg& S = segs[k];
+        const int64_t nr = S.K1 - S.K0, np = S.R1 - S.R0;
+        const int64_t* kr = kept.data() + S.K0;
+        gather_rows(dst, nr, g, [=](int64_t r) { return rows[kr[r]]; });
+        uint32_t* src = (uint32_t*)(dst + S.o_src);
+        int32_t* crow = (int32_t*)(dst + S.o_crow);
+        int32_t* mrow = (int32_t*)(dst + S.o_mrow);
+        LdRow* lr = (LdRow*)(dst + S.o_rows);
+        LdTile* tl = (LdTile*)(dst + S.o_tiles);
+        for (int64_t p = 0; p < np; ++p) lr[p] = LdRow{0.0, std::nan(""), 0, 1, 0, -1};
+        for (int64_t g2 = 0; g2 < nr; ++g2) {
+            const int64_t kk = S.K0 + g2, p = kpad[kk] - S.R0;
+            const SnpStat& s = hs[kept[kk]];
+            const double d = (double)((int64_t)s.n_nonmiss * s.sumsq - (int64_t)s.sum * s.sum);
+            src[g2] = (uint32_t)g2;
+            crow[g2] = (int32_t)p;
+            mrow[g2] = (int32_t)(p + cap);
+            lr[p] = LdRow{(double)s.sum, 1.0 / std::sqrt((double)s.n_nonmiss * d), s.n_nonmiss, (int32_t)(klo[kk] - S.R0),
+                          (int32_t)(khi[kk] - S.R0), (int32_t)g2};
+        }
+        int64_t n = 0;
+        for (int64_t T = S.T0; T < S.T1; ++T)
+            for (int64_t c = T; c <= thi[T]; ++c)
+                tl[n++] = LdTile{(int32_t)(T - S.T0), (int32_t)(c - S.T0), tnslot[T], tnslot[c], tbase[T] + (c - tlo[T]), tbase[c] + (T - tlo[c])};
+    };
+    auto launch2 = [&](int64_t k, const uint8_t* dev) -> int {
+        const LdSeg& S = segs[k];
+        const int64_t nr = S.K1 - S.K0, ngrp = (S.R1 - S.R0) / 128;
+        CU_TRY(h, launch_decode_rows(dev, n_ref, n_pad, (const uint32_t*)(dev + S.o_src), (const int32_t*)(dev + S.o_crow),
+                                     (const int32_t*)(dev + S.o_mrow), 0, nr, 1.0, (int8_t*)h->ld_codes.p, (uint8_t*)h->ld_dirty.p,
+                                     rowN, (int32_t*)(wk + o_rowS), (double*)(wk + o_rowR), (double2*)(wk + o_rowC), nullptr, h->n_sm, st));
+        CU_TRY(h, cudaMemsetAsync(gflags, 0, sizeof(int32_t) * (size_t)(ngrp + 1), st));
+        const LdRow* lr = (const LdRow*)(dev + S.o_rows);
+        CU_TRY(h, launch_ld_group_flags(lr, (int32_t)ngrp, rowN, n_ref, gflags, gflags + ngrp, st));
+        LdArgs a;
+        a.tiles = (const LdTile*)(dev + S.o_tiles);
+        a.n_tiles = (int32_t)S.n_tiles;
+        a.nk = n_pad / 128;
+        a.n_ref = n_ref;
+        a.mask_off = (int32_t)cap;
+        a.rows = lr;
+        a.gflags = gflags;
+        a.any = gflags + ngrp;
+        a.slots = slots;
+        CU_TRY(h, launch_ld_band(tmap, a, h->n_sm, st));
+        return DBSLMM_B200_OK;
+    };
+    const int64_t n2 = (int64_t)segs.size();
+    auto bytes_of2 = [&](int64_t k) { return segs[k].bytes; };
+    rc = stream_chunks(h, n2, max_bytes, n1, bytes_of2, gather2, launch2);
+    if (rc != DBSLMM_B200_OK) return rc;
+
+    // ---- every SNP's slots in ascending tile-column order, the unbiased-r^2 affine map, back to the caller's rows
+    std::vector<int32_t> wcount((size_t)n_prows, 0);
+    for (int64_t kk = 0; kk < n_kept; ++kk) wcount[kpad[kk]] = (int32_t)(khi[kk] - klo[kk] + 1);
+    o = 0;
+    const size_t o_tb = place(sizeof(int64_t) * n_trows), o_tn = place(sizeof(int32_t) * n_trows), o_wc = place(sizeof(int32_t) * n_prows),
+                 o_l2 = place(sizeof(double) * n_prows);
+    CU_TRY(h, h->ld_red.ensure(o));
+    uint8_t* rd = (uint8_t*)h->ld_red.p;
+    CU_TRY(h, cudaMemcpyAsync(rd + o_tb, tbase.data(), sizeof(int64_t) * n_trows, cudaMemcpyHostToDevice, st));
+    CU_TRY(h, cudaMemcpyAsync(rd + o_tn, tnslot.data(), sizeof(int32_t) * n_trows, cudaMemcpyHostToDevice, st));
+    CU_TRY(h, cudaMemcpyAsync(rd + o_wc, wcount.data(), sizeof(int32_t) * n_prows, cudaMemcpyHostToDevice, st));
+    const double denom = n_ref > 2 ? (double)(n_ref - 2) : (double)n_ref;
+    CU_TRY(h, cudaEventRecord(h->ev[0], st));
+    CU_TRY(h, launch_ld_reduce(slots, (const int64_t*)(rd + o_tb), (const int32_t*)(rd + o_tn), (const int32_t*)(rd + o_wc), n_prows,
+                               1.0 / denom, (double*)(rd + o_l2), st));
+    CU_TRY(h, cudaEventRecord(h->ev[1], st));
+    std::vector<double> l2p((size_t)n_prows);
+    CU_TRY(h, cudaMemcpyAsync(l2p.data(), rd + o_l2, sizeof(double) * n_prows, cudaMemcpyDeviceToHost, st));
+    CU_TRY(h, cudaStreamSynchronize(st));
+    for (int64_t kk = 0; kk < n_kept; ++kk) l2_out[kept[kk]] = l2p[kpad[kk]];
+    float ms2 = 0.0f, msr = 0.0f;
+    rc = chunk_kernel_ms(h, "ldscore pass2", n1, n2, [&](int64_t k) { return segs[k].R1 - segs[k].R0; }, bytes_of2, &ms2);
+    if (rc != DBSLMM_B200_OK) return rc;
+    CU_TRY(h, cudaEventElapsedTime(&msr, h->ev[0], h->ev[1]));
+    if (kernel_ms_out) *kernel_ms_out = ms1 + ms2 + msr;
     return DBSLMM_B200_OK;
 }
 

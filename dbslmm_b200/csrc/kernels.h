@@ -116,6 +116,36 @@ cudaError_t launch_chunk_stats(const uint8_t* chunk, int32_t n_rows, int32_t n_v
 cudaError_t launch_score_counts(const uint8_t* chunk, int32_t n_val, const uint8_t* flip, int32_t n_rows, int32_t n_slices,
                                 int32_t* cnt, int32_t* cnt2, cudaStream_t st);
 
+// ldscore.cu
+struct LdRow {              // one padded row of an LD-score segment (32 bytes); a padding row: w = NaN, N = 0, lo > hi, g = -1
+    double S;               // allele sum over the called genotypes
+    double w;               // 1 / sqrt(N d), d = N sum g^2 - S^2
+    int32_t N;              // called genotypes
+    int32_t lo, hi;         // window: padded rows lo..hi of the segment (inclusive)
+    int32_t g;              // decoder row of this SNP (index into rowN), -1 for padding
+};
+struct LdTile {             // one 128 x 128 tile (t, c) of the band (32 bytes)
+    int32_t ti, tj;         // row tile t (B operand, TMEM columns) and column tile c >= t (A operand, TMEM lanes), segment-local
+    int32_t sr_stride, sc_stride;
+    int64_t sr, sc;         // slot of row i of t: sr + i * sr_stride; of row j of c: sc + j * sc_stride (off the diagonal)
+};
+struct LdArgs {
+    const LdTile* tiles;
+    int32_t n_tiles;
+    int32_t nk;                 // n_pad / 128
+    int32_t n_ref;
+    int32_t mask_off;           // code row of the mask of code row r: r + mask_off
+    const LdRow* rows;          // per padded row of the segment
+    const int32_t* gflags;      // per 128-row group of the segment: has a missing call (device, ld_group_flags_kernel)
+    const int32_t* any;         // some group has
+    double* slots;
+};
+cudaError_t launch_ld_group_flags(const LdRow* rows, int32_t n_groups, const int32_t* rowN, int32_t n_ref, int32_t* gflags,
+                                  int32_t* any, cudaStream_t st);
+cudaError_t launch_ld_band(const CUtensorMap& tmap, const LdArgs& a, int n_sm, cudaStream_t st);
+cudaError_t launch_ld_reduce(const double* slots, const int64_t* tbase, const int32_t* tnslot, const int32_t* wcount,
+                             int64_t n_prows, double a, double* l2, cudaStream_t st);
+
 // pcg.cu
 struct PcgArgs {
     const BlockDesc* blocks;

@@ -1,0 +1,291 @@
+// ldscore_main.cpp -- `ldscore` command line: the `ldsc.py --bfile <panel> --l2` step that makes the LD Scores LDSC needs
+// for the heritability (-h) and SNP count (-nsnp) DBSLMM's driver reads from an LDSC log (DBSLMM_script.sh:63-64).
+//
+//   ldscore --bfile <prefix> --l2 (--ld-wind-cm X | --ld-wind-kb X | --ld-wind-snps N) [--maf X] [--print-snps FILE]
+//           [--yes-really] --out <prefix>
+//
+// Semantics restated from ldsc 1.0.1 (ldscore.py / ldsc.py), computed by dbslmm_b200_ldscore: SNPs with MAF <= --maf (default
+// 0) or without a homozygous call are dropped; r^2 is bias-corrected, r^2 - (1 - r^2) / (n - 2), and summed over a symmetric
+// window of cM (.bim column 3), kb (column 4) or SNPs.  One deliberate difference: windows never cross a chromosome (ldsc
+// would pair SNPs of different chromosomes by raw coordinates).  A chromosome is a run of equal .bim column-1 tokens; it must
+// be contiguous and its window coordinates non-decreasing.  As ldsc does, a chromosome whose last kept SNP's window reaches
+// its first kept SNP is refused without --yes-really: the kept SNPs decide it, so the statistics pass runs first on its own
+// and the LD pass only if no chromosome is refused.
+// Writes <out>.l2.ldscore.gz (CHR SNP BP L2, tab-separated, L2 as %.3f), <out>.l2.M, <out>.l2.M_5_50 and <out>.log -- the
+// file set `ldsc.py --ref-ld <out> --w-ld <out>` reads.  The .bed is mapped, never read whole.
+#include <sys/mman.h>
+#include <zlib.h>
+
+#include <chrono>
+#include <cmath>
+#include <cstdio>
+#include <cstdlib>
+#include <cstring>
+#include <fstream>
+#include <iostream>
+#include <sstream>
+#include <string>
+#include <unordered_map>
+#include <unordered_set>
+#include <vector>
+
+#include "dbslmm_b200.h"
+#include "plink_bed.hpp"
+
+using namespace std;
+
+namespace {
+
+[[noreturn]] void die(const string& msg, int code = 1) {
+    cerr << "ERROR: " << msg << endl;
+    exit(code);
+}
+
+void print_header() {
+    cout << endl;
+    cout << "*************************************************************" << endl;
+    cout << "  LD Scores of a PLINK fileset (ldscore), B200 build" << endl;
+    cout << "  Type ./ldscore -h for detailed help" << endl;
+    cout << "*************************************************************" << endl;
+    cout << endl;
+}
+
+void print_help() {
+    cout << " ldscore --bfile <prefix> --l2 (--ld-wind-cm X | --ld-wind-kb X | --ld-wind-snps N) [--maf X]" << endl;
+    cout << "         [--print-snps FILE] [--yes-really] --out <prefix>" << endl;
+    cout << endl;
+    cout << " --bfile        [prefix]  reference panel: <prefix>.bed (SNP-major), .bim, .fam." << endl;
+    cout << " --l2                     compute LD Scores (required)." << endl;
+    cout << " --ld-wind-cm   [X]       window of X cM (.bim column 3); exactly one window option is required." << endl;
+    cout << " --ld-wind-kb   [X]       window of X kb (.bim column 4)." << endl;
+    cout << " --ld-wind-snps [N]       window of N kept SNPs on each side." << endl;
+    cout << " --maf          [X]       drop SNPs with MAF <= X (default 0)." << endl;
+    cout << " --print-snps   [FILE]    write only the SNPs listed in the first column of FILE (the counts cover all)." << endl;
+    cout << " --yes-really             allow a window that spans a whole chromosome." << endl;
+    cout << " --out          [prefix]  writes <out>.l2.ldscore.gz, <out>.l2.M, <out>.l2.M_5_50 and <out>.log." << endl;
+}
+
+vector<string> split_ws(const string& line) {
+    vector<string> t;
+    istringstream ss(line);
+    string x;
+    while (ss >> x) t.push_back(x);
+    return t;
+}
+
+double parse_num(const string& opt, const string& v) {
+    char* e = nullptr;
+    const double x = strtod(v.c_str(), &e);
+    if (v.empty() || *e != '\0' || !std::isfinite(x) || x < 0) die(opt + " needs a number >= 0, not '" + v + "'");
+    return x;
+}
+
+struct Params {
+    string bfile, out, print_snps;
+    bool l2 = false, yes_really = false;
+    int n_wind = 0;
+    int kind = 0;                 // 0 cM, 1 kb, 2 SNPs
+    double wind = 0.0, maf = 0.0;
+};
+
+Params parse(int argc, char** argv) {
+    Params p;
+    auto value = [&](int& i, const string& a) -> string {
+        if (i + 1 >= argc) die(a + " needs a value");
+        return argv[++i];
+    };
+    for (int i = 1; i < argc; ++i) {
+        const string a = argv[i];
+        if (a == "--bfile") p.bfile = value(i, a);
+        else if (a == "--out") p.out = value(i, a);
+        else if (a == "--l2") p.l2 = true;
+        else if (a == "--yes-really") p.yes_really = true;
+        else if (a == "--print-snps") p.print_snps = value(i, a);
+        else if (a == "--maf") {
+            p.maf = parse_num(a, value(i, a));
+            if (p.maf >= 0.5) die("--maf must be below 0.5");
+        } else if (a == "--ld-wind-cm" || a == "--ld-wind-kb" || a == "--ld-wind-snps") {
+            ++p.n_wind;
+            p.kind = a == "--ld-wind-cm" ? 0 : a == "--ld-wind-kb" ? 1 : 2;
+            p.wind = parse_num(a, value(i, a));
+            if (p.kind == 2 && (p.wind != std::floor(p.wind) || p.wind > 2147483647.0)) die("--ld-wind-snps needs a whole number");
+        } else {
+            die("unsupported option '" + a + "' (ldscore takes --bfile, --l2, --ld-wind-cm/--ld-wind-kb/--ld-wind-snps, --maf, "
+                "--print-snps, --yes-really and --out; ldsc's --annot, --keep, --extract, --per-allele, --pq-exp, --chunk-size "
+                "and the others are refused)");
+        }
+    }
+    if (p.bfile.empty()) die("--bfile is required");
+    if (!p.l2) die("--l2 is required (ldscore computes LD Scores only)");
+    if (p.n_wind != 1) die("exactly one of --ld-wind-cm, --ld-wind-kb and --ld-wind-snps is required");
+    if (p.out.empty()) die("--out is required");
+    return p;
+}
+
+struct Bim { vector<string> chr, snp, bp_tok; vector<double> cm, bp; };
+
+Bim read_bim(const string& path) {
+    ifstream f(path.c_str());
+    if (!f) die(path + " does not exist");
+    Bim b;
+    string line;
+    size_t ln = 0;
+    while (getline(f, line)) {
+        ++ln;
+        const vector<string> t = split_ws(line);
+        if (t.empty()) continue;
+        if (t.size() < 6) die(path + " line " + to_string(ln) + ": a .bim line has 6 columns");
+        char* e1 = nullptr;
+        char* e2 = nullptr;
+        const double cm = strtod(t[2].c_str(), &e1), bp = strtod(t[3].c_str(), &e2);
+        if (*e1 != '\0' || *e2 != '\0' || !std::isfinite(cm) || !std::isfinite(bp))
+            die(path + " line " + to_string(ln) + ": columns 3 and 4 (cM, bp) must be numbers");
+        b.chr.push_back(t[0]); b.snp.push_back(t[1]); b.bp_tok.push_back(t[3]); b.cm.push_back(cm); b.bp.push_back(bp);
+    }
+    return b;
+}
+
+int64_t count_fam(const string& path) {
+    ifstream f(path.c_str());
+    if (!f) die(path + " does not exist");
+    string line;
+    int64_t n = 0;
+    while (getline(f, line)) if (!split_ws(line).empty()) ++n;
+    return n;
+}
+
+}  // namespace
+
+int main(int argc, char* argv[]) {
+    if (argc <= 1) { print_header(); return EXIT_SUCCESS; }
+    if (argc == 2 && (strcmp(argv[1], "-h") == 0 || strcmp(argv[1], "--help") == 0)) { print_help(); return EXIT_SUCCESS; }
+    const auto t0 = chrono::steady_clock::now();
+    const Params P = parse(argc, argv);
+    ostringstream log;
+    auto say = [&](const string& s) { cout << s << endl; log << s << "\n"; };
+    static const char* kWind[3] = {"--ld-wind-cm", "--ld-wind-kb", "--ld-wind-snps"};
+    {
+        ostringstream o;
+        o << "Options: --bfile " << P.bfile << " --l2 " << kWind[P.kind] << " " << P.wind << " --maf " << P.maf;
+        if (!P.print_snps.empty()) o << " --print-snps " << P.print_snps;
+        if (P.yes_really) o << " --yes-really";
+        o << " --out " << P.out;
+        say(o.str());
+    }
+
+    // ---- panel
+    const int64_t n = count_fam(P.bfile + ".fam");
+    const Bim bim = read_bim(P.bfile + ".bim");
+    const int64_t n_snp = (int64_t)bim.chr.size();
+    if (n == 0) die(P.bfile + ".fam lists no individual");
+    if (n > 409344) die(P.bfile + ".fam lists " + to_string(n) + " individuals; ldscore takes at most 409,344");
+    if (n_snp == 0) die(P.bfile + ".bim lists no variant");
+    if (n_snp > 2147483647) die(P.bfile + ".bim: too many variants");
+    const string bed_path = P.bfile + ".bed";
+    BedFile bedf;
+    {
+        const string err = open_bed(bed_path, n, n_snp, bedf);
+        if (!err.empty()) die(err);
+    }
+    say(to_string(n) + " individuals and " + to_string(n_snp) + " variants in " + P.bfile + ".bed/.bim/.fam");
+
+    // ---- chromosomes: contiguous runs, coordinates of the window's kind non-decreasing
+    vector<int32_t> chr_off{0};
+    vector<string> chr_name;
+    unordered_set<string> seen;
+    const vector<double>* cx = P.kind == 0 ? &bim.cm : P.kind == 1 ? &bim.bp : nullptr;
+    for (int64_t i = 0; i < n_snp; ++i) {
+        if (i == 0 || bim.chr[i] != bim.chr[i - 1]) {
+            if (!seen.insert(bim.chr[i]).second)
+                die("chromosome " + bim.chr[i] + " is not contiguous in " + P.bfile + ".bim (it appears again at line " + to_string(i + 1) +
+                    "): sort the fileset by chromosome");
+            if (i > 0) chr_off.push_back((int32_t)i);
+            chr_name.push_back(bim.chr[i]);
+        } else if (cx && (*cx)[i] < (*cx)[i - 1]) {
+            die(P.bfile + ".bim line " + to_string(i + 1) + ": the " + (P.kind == 0 ? "cM" : "bp") + " coordinates of chromosome " +
+                bim.chr[i] + " are not sorted");
+        }
+    }
+    chr_off.push_back((int32_t)n_snp);
+    unordered_set<string> print_ids;
+    if (!P.print_snps.empty()) {
+        ifstream f(P.print_snps.c_str());
+        if (!f) die(P.print_snps + " does not exist");
+        string line;
+        while (getline(f, line)) {
+            const vector<string> t = split_ws(line);
+            if (!t.empty()) print_ids.insert(t[0]);
+        }
+        bool any = false;
+        for (const string& v : bim.snp) any = any || print_ids.count(v);
+        if (!any) die("no SNP of " + P.print_snps + " is in " + P.bfile + ".bim");
+    }
+
+    // ---- GPU
+    void* map = mmap(nullptr, (size_t)bedf.size, PROT_READ, MAP_SHARED, bedf.fd, 0);
+    if (map == MAP_FAILED) die("cannot map " + bed_path);
+    close(bedf.fd);
+    const uint8_t* payload = (const uint8_t*)map + 3;
+    vector<int32_t> rows((size_t)n_snp);
+    for (int64_t i = 0; i < n_snp; ++i) rows[i] = (int32_t)i;
+    vector<double> coord;
+    if (cx) coord = *cx;
+    const double max_dist = P.kind == 1 ? 1000.0 * P.wind : P.wind;
+    const int32_t n_chr = (int32_t)chr_name.size();
+    vector<uint8_t> kept((size_t)n_snp);
+    vector<double> maf((size_t)n_snp), l2((size_t)n_snp);
+    vector<int32_t> guard((size_t)n_chr);
+    float ms = 0.0f;
+    dbslmm_b200_handle* h = nullptr;
+    if (dbslmm_b200_create(0, &h) != DBSLMM_B200_OK) die("cannot initialise the GPU (there is no CPU fallback)", 2);
+    // without --yes-really, the statistics pass alone first (l2 NULL): the kept SNPs decide the guard, and a refused
+    // chromosome must not cost the LD pass (nor fail it for want of device memory)
+    for (int full = P.yes_really ? 1 : 0; full < 2; ++full) {
+        const int rc = dbslmm_b200_ldscore(h, payload, n_snp, (int32_t)n, rows.data(), n_snp, chr_off.data(), n_chr,
+                                           cx ? DBSLMM_B200_LD_WIND_COORD : DBSLMM_B200_LD_WIND_SNPS, cx ? coord.data() : nullptr,
+                                           max_dist, P.maf, 0, kept.data(), maf.data(), full ? l2.data() : nullptr, guard.data(), &ms);
+        if (rc != DBSLMM_B200_OK) die(string("ldscore: ") + dbslmm_b200_last_error(h), 2);
+        for (int32_t c = 0; c < n_chr && !P.yes_really; ++c)
+            if (guard[c])
+                die("the window of the last kept SNP of chromosome " + chr_name[c] + " reaches its first kept SNP: do you really want "
+                    "whole-chromosome LD Scores? (--yes-really)");
+    }
+    dbslmm_b200_destroy(h);
+    munmap(map, (size_t)bedf.size);
+
+    // ---- <out>.l2.ldscore.gz, <out>.l2.M, <out>.l2.M_5_50
+    int64_t m_all = 0, m_5_50 = 0, printed = 0;
+    for (int64_t i = 0; i < n_snp; ++i)
+        if (kept[i]) {
+            ++m_all;
+            if (maf[i] > 0.05) ++m_5_50;
+            if (print_ids.empty() || print_ids.count(bim.snp[i])) ++printed;
+        }
+    if (m_all == 0) die("no SNP is kept (--maf " + to_string(P.maf) + ")");
+    if (printed == 0) die("none of the SNPs of " + P.print_snps + " is kept");
+    const string gz = P.out + ".l2.ldscore.gz";
+    gzFile f = gzopen(gz.c_str(), "wb");
+    if (!f) die("cannot write " + gz);
+    gzputs(f, "CHR\tSNP\tBP\tL2\n");
+    for (int64_t i = 0; i < n_snp; ++i) {
+        if (!kept[i] || (!print_ids.empty() && !print_ids.count(bim.snp[i]))) continue;
+        if (gzprintf(f, "%s\t%s\t%s\t%.3f\n", bim.chr[i].c_str(), bim.snp[i].c_str(), bim.bp_tok[i].c_str(), l2[i]) <= 0) die("cannot write " + gz);
+    }
+    if (gzclose(f) != Z_OK) die("cannot write " + gz);
+    for (const auto& mf : {make_pair(P.out + ".l2.M", m_all), make_pair(P.out + ".l2.M_5_50", m_5_50)}) {
+        FILE* o = fopen(mf.first.c_str(), "w");
+        if (!o || fprintf(o, "%lld\n", (long long)mf.second) < 0 || fclose(o) != 0) die("cannot write " + mf.first);
+    }
+    {
+        ostringstream o;
+        o << m_all << " SNPs kept (" << m_5_50 << " with MAF > 0.05) on " << n_chr << " chromosome(s); " << printed
+          << " written to " << gz;
+        say(o.str());
+        ostringstream t;
+        t << "GPU kernel time " << ms << " ms; wall time " << chrono::duration<double>(chrono::steady_clock::now() - t0).count() << " s";
+        say(t.str());
+    }
+    ofstream lf((P.out + ".log").c_str());
+    lf << log.str();
+    return EXIT_SUCCESS;
+}

@@ -30,6 +30,7 @@
 #include <vector>
 
 #include "dbslmm_b200.h"
+#include "plink_bed.hpp"
 
 using namespace std;
 
@@ -240,20 +241,10 @@ int main(int argc, char* argv[]) {
     if (n > INT32_MAX) die(P.bfile + ".fam: too many individuals");
     const int64_t pitch = (n + 3) / 4;
     const string bed_path = P.bfile + ".bed";
-    const int fd = open(bed_path.c_str(), O_RDONLY);
-    if (fd < 0) die(bed_path + " does not exist");
-    struct stat sb;
-    if (fstat(fd, &sb) != 0) die("cannot stat " + bed_path);
-    unsigned char magic[3] = {0, 0, 0};
-    if (sb.st_size < 3 || pread(fd, magic, 3, 0) != 3 || magic[0] != 0x6c || magic[1] != 0x1b)
-        die(bed_path + " is not a PLINK .bed file (magic bytes 6c 1b expected)");
-    if (magic[2] != 0x01) die(bed_path + " is individual-major; only SNP-major .bed files (third byte 01) are supported");
-    const uint64_t want = 3 + (uint64_t)n_snp * (uint64_t)pitch;
-    if ((uint64_t)sb.st_size != want) {
-        ostringstream o;
-        o << bed_path << " has " << sb.st_size << " bytes; " << n_snp << " variants x " << n << " individuals need " << want
-          << " (3 + n_snp x ceil(n/4))";
-        die(o.str());
+    BedFile bedf;
+    {
+        const string err = open_bed(bed_path, n, n_snp, bedf);
+        if (!err.empty()) die(err);
     }
     say(to_string(n) + " individuals and " + to_string(n_snp) + " variants in " + P.bfile + ".bed/.bim/.fam");
 
@@ -304,9 +295,9 @@ int main(int argc, char* argv[]) {
     }
 
     // ---- GPU
-    void* map = mmap(nullptr, (size_t)sb.st_size, PROT_READ, MAP_SHARED, fd, 0);
+    void* map = mmap(nullptr, (size_t)bedf.size, PROT_READ, MAP_SHARED, bedf.fd, 0);
     if (map == MAP_FAILED) die("cannot map " + bed_path);
-    close(fd);
+    close(bedf.fd);
     const uint8_t* payload = (const uint8_t*)map + 3;
     dbslmm_b200_handle* h = nullptr;
     if (dbslmm_b200_create(0, &h) != DBSLMM_B200_OK) die("cannot initialise the GPU (there is no CPU fallback)", 2);
@@ -348,7 +339,7 @@ int main(int argc, char* argv[]) {
         }
     }
     dbslmm_b200_destroy(h);
-    munmap(map, (size_t)sb.st_size);
+    munmap(map, (size_t)bedf.size);
 
     // ---- <out>.profile / <out>_f<k>.profile: FID IID PHENO CNT CNT2 SCORESUM, one row per .fam line in .fam order
     for (size_t k = 0; k < nf; ++k) {

@@ -211,6 +211,39 @@ DBSLMM_B200_API int  dbslmm_b200_score_stream(dbslmm_b200_handle* h, const uint8
                               uint64_t chunk_bytes, double* scores_out, int32_t* cnt_out, int32_t* cnt2_out,
                               int32_t* n_empty_rows_out, float* kernel_ms_out);
 
+/* LD Scores of a reference panel, as `ldsc.py --bfile <panel> --l2` computes them (ldsc 1.0.1's ldscore.py restated):
+ *   l_j = sum_{k in W(j)} r2adj(j, k),   r2adj = r^2 - (1 - r^2) / (n - 2)   (denominator n_ref when n_ref <= 2),
+ * r = the Pearson correlation of the mean-imputed genotypes of kept SNPs j and k (r_jj = 1), formed from the exact integer
+ * Gram of the decoded rows on the tensor cores.
+ * rows[0..n_rows) are .bed rows, chromosome-major and in coordinate order within a chromosome; chromosome c is
+ * rows[chr_off[c] .. chr_off[c + 1]).  A row is KEPT iff min(f, 1 - f) > maf_min and missing + heterozygous calls < n_ref
+ * (f = allele frequency among the called genotypes, 0 when none is called): every kept SNP has nonzero variance.  W(j) is
+ * the set of kept SNPs k of j's chromosome with |c_k - c_j| <= max_dist, where c is coord[row] (wind_kind = COORD: cM or
+ * base pairs, non-decreasing within a chromosome) or the index among the chromosome's kept SNPs (wind_kind = SNPS, coord
+ * NULL, max_dist a whole number).  Windows never cross a chromosome.
+ * Outputs, each [n_rows] and each may be NULL: kept_out 0/1, maf_out min(f, 1 - f), l2_out the LD Score (NaN where not
+ * kept); guard_out [n_chr]: 1 where the window of the chromosome's last kept SNP reaches its first one (ldsc refuses such a
+ * chromosome unless told otherwise; reported here, not enforced).  With l2_out NULL the call stops after the statistics
+ * pass: kept_out, maf_out and guard_out only, one pass over the rows (a caller can check the guard before the LD pass).
+ * Two passes stream the requested rows from ORDINARY host memory (an mmap of the .bed is fine; only these rows are read)
+ * through pinned staging buffers, as dbslmm_b200_score_stream does: per-row statistics, then segments of consecutive
+ * 128-row tiles with the halo of rows their windows reach.  Device memory: O(segment + halo) x 2 x n_pad bytes plus one
+ * double per (SNP, 128-row tile its window reaches).  segment_rows = 0 sizes the segments from free device memory; a
+ * nonzero multiple of 128 fixes them.  Deterministic: the result does not depend on the segment size, on which other
+ * chromosomes are in the call, or on the run.  Limits: n_ref <= 409,344, n_rows <= INT32_MAX.  kernel_ms_out (or NULL):
+ * the summed device time of the call's kernels.  Synchronous. */
+/* Inspection hook (the tests check the window rule through it): the window rule of dbslmm_b200_ldscore over the m kept
+ * SNPs of one chromosome, the library's own host code (needs no GPU): W(k) = [lo_out[k],
+ * hi_out[k]] = the k' with |c_k' - c_k| <= max_dist, c = coord (non-decreasing) or, with coord NULL, the index k.  The
+ * chromosome's guard is lo_out[m - 1] == 0. */
+DBSLMM_B200_API int  dbslmm_b200_ld_windows(const double* coord, int64_t m, double max_dist, int32_t* lo_out, int32_t* hi_out);
+#define DBSLMM_B200_LD_WIND_COORD 0
+#define DBSLMM_B200_LD_WIND_SNPS  1
+DBSLMM_B200_API int  dbslmm_b200_ldscore(dbslmm_b200_handle* h, const uint8_t* bed, int64_t n_snp, int32_t n_ref,
+                         const int32_t* rows, int64_t n_rows, const int32_t* chr_off, int32_t n_chr,
+                         int32_t wind_kind, const double* coord, double max_dist, double maf_min, int64_t segment_rows,
+                         uint8_t* kept_out, double* maf_out, double* l2_out, int32_t* guard_out, float* kernel_ms_out);
+
 /* ---- inspection hooks used by the parity tests (operate on the state of the last fit) ---- */
 /* int8 codes of one decoded row of the last fit: SNP j of block `block` (its small SNPs first, then its large ones),
  * plane 0 = allele counts (missing -> 0), plane 1 = call mask (1 = called; holds the last mask written at that position,
