@@ -19,11 +19,12 @@ FLAG_PLAN_CACHED = 4
 FLAG_PANEL_SUBSET = 8
 LD_WIND_COORD = 0
 LD_WIND_SNPS = 1
+LD_MAX_ANNOT = 4096
 
 EXPORTS = [
     "dbslmm_b200_abi_version", "dbslmm_b200_device_count", "dbslmm_b200_create", "dbslmm_b200_destroy",
     "dbslmm_b200_last_error", "dbslmm_b200_load_bed", "dbslmm_b200_snp_stats", "dbslmm_b200_plan_shards",
-    "dbslmm_b200_fit", "dbslmm_b200_fit_multi", "dbslmm_b200_host_alloc", "dbslmm_b200_host_free", "dbslmm_b200_score", "dbslmm_b200_score_prefetch", "dbslmm_b200_score_stream", "dbslmm_b200_ldscore", "dbslmm_b200_ld_windows", "dbslmm_b200_get_row_codes", "dbslmm_b200_get_block_sigma",
+    "dbslmm_b200_fit", "dbslmm_b200_fit_multi", "dbslmm_b200_host_alloc", "dbslmm_b200_host_free", "dbslmm_b200_score", "dbslmm_b200_score_prefetch", "dbslmm_b200_score_stream", "dbslmm_b200_ldscore", "dbslmm_b200_ldscore_annot", "dbslmm_b200_ld_windows", "dbslmm_b200_get_row_codes", "dbslmm_b200_get_block_sigma",
     "dbslmm_b200_get_block_factor", "dbslmm_b200_get_block_gram", "dbslmm_b200_get_block_iters",
 ]
 
@@ -87,6 +88,10 @@ def load():
         lib.dbslmm_b200_ldscore.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p,
                                             C.c_int32, C.c_int32, C.c_void_p, C.c_double, C.c_double, C.c_int64, C.c_void_p,
                                             C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_float)]
+        lib.dbslmm_b200_ldscore_annot.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p,
+                                                  C.c_int32, C.c_int32, C.c_void_p, C.c_double, C.c_double, C.c_int64,
+                                                  C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                  C.POINTER(C.c_float)]
         lib.dbslmm_b200_ld_windows.argtypes = [C.c_void_p, C.c_int64, C.c_double, C.c_void_p, C.c_void_p]
         lib.dbslmm_b200_score_prefetch.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32]
         lib.dbslmm_b200_get_row_codes.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32]
@@ -306,14 +311,17 @@ class Engine:
         self.last_empty_rows = empty.value
         return out, cnt, cnt2
 
-    def ldscore(self, bed, n_ref, rows, chr_off, coord=None, *, max_dist, maf_min=0.0, segment_rows=0, stats_only=False):
+    def ldscore(self, bed, n_ref, rows, chr_off, coord=None, *, max_dist, maf_min=0.0, segment_rows=0, stats_only=False,
+                annot=None):
         """LD Scores of .bed rows `rows` (dbslmm_b200_ldscore, `ldsc.py --l2`): chromosome c is rows[chr_off[c]:chr_off[c+1]],
         in coordinate order.  coord (float64[rows.size], cM or bp) gives a window of |c_k - c_j| <= max_dist; coord=None a
         window of max_dist kept SNPs.  bed: uint8 payload after the magic bytes ([n_snp, ceil(n_ref/4)] or flat), e.g. a
         numpy.memmap of the .bed opened with offset=3: only the listed rows are read.  Returns (l2, kept, maf, guard):
         l2 float64[rows.size] (NaN where not kept), kept bool, maf float64, guard bool[n_chr] (the window of a chromosome's
         last kept SNP reaches its first).  stats_only=True stops after the statistics pass (l2 is then None).  The summed
-        kernel time is left in self.last_kernel_ms."""
+        kernel time is left in self.last_kernel_ms.
+        annot (float64 [rows.size, C], `ldsc.py --l2 --annot`): partitioned LD Scores (dbslmm_b200_ldscore_annot), l2 is then
+        [rows.size, C], column c the window sum of r2adj(j, k) a_kc."""
         n_ref = int(n_ref)
         pitch = (n_ref + 3) // 4
         if not (isinstance(bed, np.ndarray) and bed.dtype == np.uint8 and bed.flags.c_contiguous):
@@ -327,18 +335,22 @@ class Engine:
         n_chr = chr_off.size - 1
         if n_chr < 0:
             raise ValueError("ldscore: chr_off needs n_chr + 1 entries")
-        l2 = np.zeros(rows.size, np.float64)
+        if annot is not None:
+            annot = np.ascontiguousarray(annot, np.float64)
+            if annot.ndim != 2 or annot.shape[0] != rows.size:
+                raise ValueError("ldscore: annot must be [rows.size, n_annot]")
+        l2 = np.zeros(rows.size if annot is None else annot.shape, np.float64)
         kept = np.zeros(rows.size, np.uint8)
         maf = np.zeros(rows.size, np.float64)
         guard = np.zeros(max(n_chr, 1), np.int32)
         ms = C.c_float(0)
-        self._check(self.lib.dbslmm_b200_ldscore(self.h, bed.ctypes.data, bed.size // pitch, n_ref, rows.ctypes.data, rows.size,
-                                                 chr_off.ctypes.data, n_chr, LD_WIND_SNPS if coord is None else LD_WIND_COORD,
-                                                 _ptr(coord), float(max_dist), float(maf_min), int(segment_rows),
-                                                 kept.ctypes.data, maf.ctypes.data, None if stats_only else l2.ctypes.data,
-                                                 guard.ctypes.data,
-                                                 C.byref(ms)),
-                    "ldscore")
+        common = (self.h, bed.ctypes.data, bed.size // pitch, n_ref, rows.ctypes.data, rows.size, chr_off.ctypes.data, n_chr,
+                  LD_WIND_SNPS if coord is None else LD_WIND_COORD, _ptr(coord), float(max_dist), float(maf_min), int(segment_rows))
+        outs = (kept.ctypes.data, maf.ctypes.data, None if stats_only else l2.ctypes.data, guard.ctypes.data, C.byref(ms))
+        if annot is None:
+            self._check(self.lib.dbslmm_b200_ldscore(*common, *outs), "ldscore")
+        else:
+            self._check(self.lib.dbslmm_b200_ldscore_annot(*common, annot.ctypes.data, annot.shape[1], *outs), "ldscore_annot")
         self.last_kernel_ms = ms.value
         return None if stats_only else l2, kept.astype(bool), maf, guard[:n_chr].astype(bool)
 

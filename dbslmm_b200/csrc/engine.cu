@@ -2281,6 +2281,10 @@ int dbslmm_b200_score_stream(dbslmm_b200_handle* h, const uint8_t* bed_val, int6
 // ldsc's SNPs, builds the windows over the kept SNPs of every chromosome, the band of 128 x 128 tiles and the slot layout.
 // Pass 2 streams segments of consecutive row tiles together with the halo of rows their windows reach (decode -> group
 // flags -> band kernels, one chunk per segment); ld_reduce_kernel then adds each SNP's slots.
+// With annotations (dbslmm_b200_ldscore_annot) the same host path lists the FULL band instead -- tiles (T, P) for every
+// tile P that T's windows reach, on both sides -- so a row tile depends only on its own segment (which then starts at its
+// left halo, 128 tlo[T0]).  Each segment's chunk also carries its annotation rows; its slots (row, tile, half,
+// annotation) live only while the segment is processed: ld_annot_reduce_kernel adds them right after its band kernels.
 // ---------------------------------------------------------------------------------------------
 namespace {
 struct LdSeg {
@@ -2288,7 +2292,9 @@ struct LdSeg {
     int64_t R0 = 0, R1 = 0;           // padded rows on the device: [128 T0, 128 (last tile column reached + 1))
     int64_t K0 = 0, K1 = 0;           // kept SNPs among them
     int64_t n_tiles = 0;
+    int64_t n_slots = 0;              // annotated: partial sums of the segment
     size_t o_src = 0, o_crow = 0, o_mrow = 0, o_rows = 0, o_tiles = 0, bytes = 0;
+    size_t o_annot = 0, o_sbase = 0, o_nslot = 0;    // annotated: annotation rows [R1 - R0][C], slot base and count per row tile
 };
 }  // namespace
 
@@ -2306,12 +2312,16 @@ int dbslmm_b200_ld_windows(const double* coord, int64_t m, double max_dist, int3
     return DBSLMM_B200_OK;
 }
 
-int dbslmm_b200_ldscore(dbslmm_b200_handle* h, const uint8_t* bed, int64_t n_snp, int32_t n_ref, const int32_t* rows,
+// n_annot = 0: dbslmm_b200_ldscore (annot NULL, l2_out [n_rows]); n_annot >= 1: dbslmm_b200_ldscore_annot.
+static int ldscore_impl(dbslmm_b200_handle* h, const uint8_t* bed, int64_t n_snp, int32_t n_ref, const int32_t* rows,
                         int64_t n_rows, const int32_t* chr_off, int32_t n_chr, int32_t wind_kind, const double* coord,
-                        double max_dist, double maf_min, int64_t segment_rows, uint8_t* kept_out, double* maf_out,
-                        double* l2_out, int32_t* guard_out, float* kernel_ms_out) {
+                        double max_dist, double maf_min, int64_t segment_rows, const double* annot, int32_t n_annot,
+                        uint8_t* kept_out, double* maf_out, double* l2_out, int32_t* guard_out, float* kernel_ms_out) {
     if (!h) return DBSLMM_B200_ERR_ARG;
-    auto bad = [&](const std::string& m) { return fail(h, DBSLMM_B200_ERR_ARG, "ldscore: " + m); };
+    const char* who = n_annot > 0 ? "ldscore_annot: " : "ldscore: ";
+    auto bad = [&](const std::string& m) { return fail(h, DBSLMM_B200_ERR_ARG, who + m); };
+    const bool an = n_annot > 0;
+    const int64_t C = an ? n_annot : 1;             // values per row of l2_out
     if (!bed || n_snp <= 0 || n_ref <= 0 || n_rows < 0 || n_chr < 0 || !chr_off || (n_rows > 0 && !rows))
         return bad("bad arguments");
     if (n_ref > decode_max_n_ref())
@@ -2339,6 +2349,11 @@ int dbslmm_b200_ldscore(dbslmm_b200_handle* h, const uint8_t* bed, int64_t n_snp
                     return bad("the coordinates of chromosome " + std::to_string(c) + " are not sorted: coord[" + std::to_string(i) + "] < coord[" +
                                std::to_string(i - 1) + "]");
             }
+    if (an) {
+        for (int64_t x = 0; x < n_rows * C; ++x)
+            if (!std::isfinite(annot[x]))
+                return bad("annot[" + std::to_string(x / C) + "][" + std::to_string(x % C) + "] is not finite");
+    }
     CU_TRY(h, cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
     const int64_t pitch = (n_ref + 3) / 4;
@@ -2419,14 +2434,19 @@ int dbslmm_b200_ldscore(dbslmm_b200_handle* h, const uint8_t* bed, int64_t n_snp
     }
     const int64_t n_trows = (int64_t)tlo.size(), n_prows = 128 * n_trows, n_kept = (int64_t)kept.size();
     if (l2_out)
-        for (int64_t i = 0; i < n_rows; ++i) l2_out[i] = std::nan("");
+        for (int64_t i = 0; i < n_rows * C; ++i) l2_out[i] = std::nan("");
     if (n_kept == 0 || !l2_out) {                       // (l2_out NULL: the statistics pass only)
         if (kernel_ms_out) *kernel_ms_out = ms1;
         return DBSLMM_B200_OK;
     }
 
-    // ---- segments: consecutive row tiles; nonzero segment_rows fixes their size, else 64 MB of .bed rows while the code rows
-    // of the widest segment (with its halo) take at most half of the free device memory
+    // ---- segments: consecutive row tiles; nonzero segment_rows fixes their size, else 64 MB of .bed rows (and annotation
+    // rows) while the code rows of the widest segment (with its halo), and with annotations its partial sums, take at most
+    // half of the free device memory
+    int64_t max_nslot = 0;
+    for (int64_t T = 0; T < n_trows; ++T) max_nslot = std::max<int64_t>(max_nslot, tnslot[T]);
+    if (an && 2 * max_nslot * C > INT32_MAX)
+        return bad("a window reaches " + std::to_string(max_nslot) + " tiles of 128 SNPs: too wide for " + std::to_string(C) + " annotations");
     auto plan = [&](int64_t seg_tiles, std::vector<LdSeg>& segs) {
         segs.clear();
         int64_t cap = 0;
@@ -2434,34 +2454,51 @@ int dbslmm_b200_ldscore(dbslmm_b200_handle* h, const uint8_t* bed, int64_t n_snp
             LdSeg S;
             S.T0 = T0;
             S.T1 = std::min(n_trows, T0 + seg_tiles);
-            S.R0 = 128 * S.T0;
+            S.R0 = 128 * (an ? tlo[S.T0] : S.T0);
             S.R1 = 128 * (thi[S.T1 - 1] + 1);
             S.K0 = std::lower_bound(kpad.begin(), kpad.end(), S.R0) - kpad.begin();
             S.K1 = std::lower_bound(kpad.begin(), kpad.end(), S.R1) - kpad.begin();
-            for (int64_t T = S.T0; T < S.T1; ++T) S.n_tiles += thi[T] - T + 1;
-            const int64_t nr = S.K1 - S.K0, np = S.R1 - S.R0;
+            for (int64_t T = S.T0; T < S.T1; ++T) {
+                S.n_tiles += thi[T] - (an ? tlo[T] : T) + 1;
+                S.n_slots += an ? 2 * 128 * C * tnslot[T] : 0;
+            }
+            const int64_t nr = S.K1 - S.K0, np = S.R1 - S.R0, nt = S.T1 - S.T0;
             S.o_src = align_up((size_t)nr * pitch + 16, 256);        // + 16: the decoder's row copies are 16-byte aligned
             S.o_crow = align_up(S.o_src + sizeof(uint32_t) * nr, 256);
             S.o_mrow = align_up(S.o_crow + sizeof(int32_t) * nr, 256);
             S.o_rows = align_up(S.o_mrow + sizeof(int32_t) * nr, 256);
             S.o_tiles = align_up(S.o_rows + sizeof(LdRow) * np, 256);
             S.bytes = align_up(S.o_tiles + sizeof(LdTile) * S.n_tiles, 256);
+            if (an) {
+                S.o_annot = S.bytes;
+                S.o_sbase = align_up(S.o_annot + sizeof(double) * (size_t)(np * C), 256);
+                S.o_nslot = align_up(S.o_sbase + sizeof(int64_t) * nt, 256);
+                S.bytes = align_up(S.o_nslot + sizeof(int32_t) * nt, 256);
+            }
             cap = std::max(cap, np);
             segs.push_back(S);
         }
         return cap;
     };
+    auto seg_slots = [&](const std::vector<LdSeg>& segs) {
+        int64_t m = 0;
+        for (const LdSeg& S : segs) m = std::max(m, S.n_slots);
+        return m;
+    };
     std::vector<LdSeg> segs;
-    int64_t seg_tiles = segment_rows > 0 ? segment_rows / 128 : std::max<int64_t>(1, (int64_t)(kStreamChunkDefault / (uint64_t)(128 * pitch)));
+    const uint64_t row_bytes = (uint64_t)(128 * pitch) + (an ? (uint64_t)(128 * 8 * C) : 0);
+    int64_t seg_tiles = segment_rows > 0 ? segment_rows / 128 : std::max<int64_t>(1, (int64_t)(kStreamChunkDefault / row_bytes));
     int64_t cap = plan(seg_tiles, segs);
     size_t free_b = 0, total_b = 0;
     CU_TRY(h, cudaMemGetInfo(&free_b, &total_b));
     auto need = [&](int64_t cp) { return (double)cp * (2.0 * n_pad + 2.0 + 48.0); };
     if (segment_rows == 0)
-        while (seg_tiles > 1 && need(cap) > 0.5 * (double)free_b) cap = plan(seg_tiles = (seg_tiles + 1) / 2, segs);
-    if (need(cap) + 8.0 * (double)slots_total > 0.9 * (double)free_b)
-        return fail(h, DBSLMM_B200_ERR_NOMEM, "ldscore: a segment of " + std::to_string(cap) + " rows (with the halo its windows reach) and " +
-                                             std::to_string(slots_total) + " partial sums do not fit in device memory");
+        while (seg_tiles > 1 && need(cap) + 8.0 * (double)seg_slots(segs) > 0.5 * (double)free_b) cap = plan(seg_tiles = (seg_tiles + 1) / 2, segs);
+    const int64_t n_slots = an ? seg_slots(segs) : slots_total;
+    const double out_bytes = an ? 8.0 * (double)(n_prows * C) : 0.0;
+    if (need(cap) + 8.0 * (double)n_slots + out_bytes > 0.9 * (double)free_b)
+        return fail(h, DBSLMM_B200_ERR_NOMEM, who + std::string("a segment of ") + std::to_string(cap) + " rows (with the halo its windows reach) and " +
+                                             std::to_string(n_slots) + " partial sums do not fit in device memory");
     size_t max_bytes = 0;
     for (const LdSeg& S : segs) max_bytes = std::max(max_bytes, S.bytes);
 
@@ -2478,9 +2515,14 @@ int dbslmm_b200_ldscore(dbslmm_b200_handle* h, const uint8_t* bed, int64_t n_snp
     uint8_t* wk = (uint8_t*)h->ld_work.p;
     int32_t* rowN = (int32_t*)(wk + o_rowN);
     int32_t* gflags = (int32_t*)(wk + o_gfl);
-    CU_TRY(h, h->ld_slots.ensure(sizeof(double) * (size_t)slots_total));
+    CU_TRY(h, h->ld_slots.ensure(sizeof(double) * (size_t)n_slots));
     double* slots = (double*)h->ld_slots.p;
-    CU_TRY(h, cudaMemsetAsync(slots, 0, sizeof(double) * (size_t)slots_total, st));
+    if (!an) CU_TRY(h, cudaMemsetAsync(slots, 0, sizeof(double) * (size_t)slots_total, st));     // (annotated: every slot is written)
+    double* l2a = nullptr;                                  // annotated: [n_prows][C]
+    if (an) {
+        CU_TRY(h, h->ld_red.ensure(sizeof(double) * (size_t)(n_prows * C)));
+        l2a = (double*)h->ld_red.p;
+    }
     CUtensorMap tmap;
     rc = make_tensor_map(h, &tmap, h->ld_codes.p, 2 * cap, n_pad, 128);
     if (rc != DBSLMM_B200_OK) return rc;
@@ -2507,9 +2549,27 @@ int dbslmm_b200_ldscore(dbslmm_b200_handle* h, const uint8_t* bed, int64_t n_snp
                           (int32_t)(khi[kk] - S.R0), (int32_t)g2};
         }
         int64_t n = 0;
-        for (int64_t T = S.T0; T < S.T1; ++T)
-            for (int64_t c = T; c <= thi[T]; ++c)
-                tl[n++] = LdTile{(int32_t)(T - S.T0), (int32_t)(c - S.T0), tnslot[T], tnslot[c], tbase[T] + (c - tlo[T]), tbase[c] + (T - tlo[c])};
+        if (!an) {
+            for (int64_t T = S.T0; T < S.T1; ++T)
+                for (int64_t c = T; c <= thi[T]; ++c)
+                    tl[n++] = LdTile{(int32_t)(T - S.T0), (int32_t)(c - S.T0), tnslot[T], tnslot[c], tbase[T] + (c - tlo[T]), tbase[c] + (T - tlo[c])};
+            return;
+        }
+        // full band: scored tile T on the TMEM lanes (tj), partner tile P (ti); tiles are numbered from the segment's first row
+        double* ann = (double*)(dst + S.o_annot);
+        int64_t* sbase = (int64_t*)(dst + S.o_sbase);
+        int32_t* nslot = (int32_t*)(dst + S.o_nslot);
+        std::fill(ann, ann + np * C, 0.0);
+        for (int64_t kk = S.K0; kk < S.K1; ++kk) std::memcpy(ann + (kpad[kk] - S.R0) * C, annot + kept[kk] * C, sizeof(double) * (size_t)C);
+        const int64_t D0 = S.R0 / 128;
+        int64_t sb = 0;
+        for (int64_t T = S.T0; T < S.T1; ++T) {
+            sbase[T - S.T0] = sb;
+            nslot[T - S.T0] = tnslot[T];
+            for (int64_t P = tlo[T]; P <= thi[T]; ++P)
+                tl[n++] = LdTile{(int32_t)(P - D0), (int32_t)(T - D0), (int32_t)(2 * tnslot[T] * C), 0, sb + (P - tlo[T]) * 2 * C, 0};
+            sb += 2 * 128 * C * tnslot[T];
+        }
     };
     auto launch2 = [&](int64_t k, const uint8_t* dev) -> int {
         const LdSeg& S = segs[k];
@@ -2530,13 +2590,33 @@ int dbslmm_b200_ldscore(dbslmm_b200_handle* h, const uint8_t* bed, int64_t n_snp
         a.gflags = gflags;
         a.any = gflags + ngrp;
         a.slots = slots;
-        CU_TRY(h, launch_ld_band(tmap, a, h->n_sm, st));
+        if (!an) {
+            CU_TRY(h, launch_ld_band(tmap, a, h->n_sm, st));
+            return DBSLMM_B200_OK;
+        }
+        a.annot = (const double*)(dev + S.o_annot);
+        a.n_annot = n_annot;
+        a.alpha = 1.0 / (n_ref > 2 ? (double)(n_ref - 2) : (double)n_ref);
+        CU_TRY(h, launch_ld_band_annot(tmap, a, h->n_sm, st));
+        CU_TRY(h, launch_ld_annot_reduce(slots, (const int64_t*)(dev + S.o_sbase), (const int32_t*)(dev + S.o_nslot), lr,
+                                         128 * S.T0 - S.R0, 128 * (S.T1 - S.T0), n_annot, l2a + 128 * S.T0 * C, st));
         return DBSLMM_B200_OK;
     };
     const int64_t n2 = (int64_t)segs.size();
     auto bytes_of2 = [&](int64_t k) { return segs[k].bytes; };
     rc = stream_chunks(h, n2, max_bytes, n1, bytes_of2, gather2, launch2);
     if (rc != DBSLMM_B200_OK) return rc;
+    if (an) {                                           // the sums are in: back to the caller's rows
+        std::vector<double> l2p((size_t)(n_prows * C));
+        CU_TRY(h, cudaMemcpyAsync(l2p.data(), l2a, sizeof(double) * l2p.size(), cudaMemcpyDeviceToHost, st));
+        CU_TRY(h, cudaStreamSynchronize(st));
+        for (int64_t kk = 0; kk < n_kept; ++kk) std::memcpy(l2_out + kept[kk] * C, l2p.data() + kpad[kk] * C, sizeof(double) * (size_t)C);
+        float ms2 = 0.0f;
+        rc = chunk_kernel_ms(h, "ldscore_annot pass2", n1, n2, [&](int64_t k) { return segs[k].R1 - segs[k].R0; }, bytes_of2, &ms2);
+        if (rc != DBSLMM_B200_OK) return rc;
+        if (kernel_ms_out) *kernel_ms_out = ms1 + ms2;
+        return DBSLMM_B200_OK;
+    }
 
     // ---- every SNP's slots in ascending tile-column order, the unbiased-r^2 affine map, back to the caller's rows
     std::vector<int32_t> wcount((size_t)n_prows, 0);
@@ -2564,6 +2644,27 @@ int dbslmm_b200_ldscore(dbslmm_b200_handle* h, const uint8_t* bed, int64_t n_snp
     CU_TRY(h, cudaEventElapsedTime(&msr, h->ev[0], h->ev[1]));
     if (kernel_ms_out) *kernel_ms_out = ms1 + ms2 + msr;
     return DBSLMM_B200_OK;
+}
+
+int dbslmm_b200_ldscore(dbslmm_b200_handle* h, const uint8_t* bed, int64_t n_snp, int32_t n_ref, const int32_t* rows,
+                        int64_t n_rows, const int32_t* chr_off, int32_t n_chr, int32_t wind_kind, const double* coord,
+                        double max_dist, double maf_min, int64_t segment_rows, uint8_t* kept_out, double* maf_out,
+                        double* l2_out, int32_t* guard_out, float* kernel_ms_out) {
+    return ldscore_impl(h, bed, n_snp, n_ref, rows, n_rows, chr_off, n_chr, wind_kind, coord, max_dist, maf_min, segment_rows,
+                        nullptr, 0, kept_out, maf_out, l2_out, guard_out, kernel_ms_out);
+}
+
+int dbslmm_b200_ldscore_annot(dbslmm_b200_handle* h, const uint8_t* bed, int64_t n_snp, int32_t n_ref, const int32_t* rows,
+                              int64_t n_rows, const int32_t* chr_off, int32_t n_chr, int32_t wind_kind, const double* coord,
+                              double max_dist, double maf_min, int64_t segment_rows, const double* annot, int32_t n_annot,
+                              uint8_t* kept_out, double* maf_out, double* l2_out, int32_t* guard_out, float* kernel_ms_out) {
+    if (!h) return DBSLMM_B200_ERR_ARG;
+    if (n_annot < 1 || n_annot > DBSLMM_B200_LD_MAX_ANNOT)
+        return fail(h, DBSLMM_B200_ERR_ARG, "ldscore_annot: n_annot = " + std::to_string(n_annot) + " must lie in [1, " +
+                                            std::to_string(DBSLMM_B200_LD_MAX_ANNOT) + "]");
+    if (!annot) return fail(h, DBSLMM_B200_ERR_ARG, "ldscore_annot: annot is NULL");
+    return ldscore_impl(h, bed, n_snp, n_ref, rows, n_rows, chr_off, n_chr, wind_kind, coord, max_dist, maf_min, segment_rows,
+                        annot, n_annot, kept_out, maf_out, l2_out, guard_out, kernel_ms_out);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -139,10 +139,19 @@ struct LdArgs {
     const int32_t* gflags;      // per 128-row group of the segment: has a missing call (device, ld_group_flags_kernel)
     const int32_t* any;         // some group has
     double* slots;
+    // the annotated band only (ld_band_kernel<kMiss, true>)
+    const double* annot;        // per padded row of the segment: n_annot values (0 for padding rows)
+    int32_t n_annot;
+    double alpha;               // r2adj = (1 + alpha) r^2 - alpha
 };
 cudaError_t launch_ld_group_flags(const LdRow* rows, int32_t n_groups, const int32_t* rowN, int32_t n_ref, int32_t* gflags,
                                   int32_t* any, cudaStream_t st);
 cudaError_t launch_ld_band(const CUtensorMap& tmap, const LdArgs& a, int n_sm, cudaStream_t st);
+// the annotated band: tiles (t, c) of the full band, c the scored row tile (TMEM lanes, tj) and t a tile its windows
+// reach (ti); the slot of annotation k of row j of c, half h of t's rows: sr + j * sr_stride + h * n_annot + k
+cudaError_t launch_ld_band_annot(const CUtensorMap& tmap, const LdArgs& a, int n_sm, cudaStream_t st);
+cudaError_t launch_ld_annot_reduce(const double* slots, const int64_t* sbase, const int32_t* nslot, const LdRow* rows, int64_t row0,
+                                   int64_t n_rows, int32_t n_annot, double* l2, cudaStream_t st);
 cudaError_t launch_ld_reduce(const double* slots, const int64_t* tbase, const int32_t* tnslot, const int32_t* wcount,
                              int64_t n_prows, double a, double* l2, cudaStream_t st);
 

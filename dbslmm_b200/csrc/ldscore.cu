@@ -27,6 +27,9 @@
 //   kMiss = true   four planes: g_j . [g_i | M_i] and M_j . [g_i | M_i] as two MMAs of N = 256, all 512 TMEM columns.
 // Which kernel owns a tile is decided on the device: ld_group_flags_kernel marks the 128-row groups with a missing call
 // from the decoder's counts, and a tile is four-plane if either of its groups is marked.
+// Partitioned LD Scores (ld_band_kernel<kMiss, true>, ld_annot_reduce_kernel): L_c(i) = sum_{k in W(i)} r2adj(i, k) a_kc
+// over the FULL band (tiles (t, c) for every c that t's windows reach, both sides): no column partials and no transpose,
+// each epilogue lane contracts its SNP's r2adj with the partners' annotation rows, register group by register group.
 #include <algorithm>
 #include "common.cuh"
 #include "kernels.h"
@@ -37,13 +40,18 @@ static constexpr int kLdTile = 128;
 static constexpr int kLdTileBytes = kLdTile * 128;     // one operand: 128 rows x 128 B (K chunk = 128 samples)
 static constexpr int kLdThreads = 320;
 
-template <bool kMiss>
+static constexpr int kLdGroup = 16;                     // annotations per register group of the annotated epilogue
+
+// kAnnot: the annotated band (ld_band_kernel<kMiss, true>).  It is FP64-bound, so its TMA ring is shallower, and the
+// space freed holds one group of annotation values per epilogue warp: its 64 partner rows x kLdGroup doubles.
+template <bool kMiss, bool kAnnot = false>
 struct LdCfg {
-    static constexpr int kStages = kMiss ? 3 : 6;
+    static constexpr int kStages = kAnnot ? (kMiss ? 2 : 3) : (kMiss ? 3 : 6);
     static constexpr int kStageBytes = (kMiss ? 4 : 2) * kLdTileBytes;
     static constexpr int kAcc = kMiss ? 1 : 4;           // accumulator buffers
     static constexpr int kAccCols = kMiss ? 512 : 128;   // TMEM columns of one
-    static constexpr int kSmem = kStages * kStageBytes + 1024;
+    static constexpr int kAnnotBytes = kAnnot ? 8 * 64 * kLdGroup * (int)sizeof(double) : 0;
+    static constexpr int kSmem = kStages * kStageBytes + kAnnotBytes + 1024;
 };
 
 __device__ __forceinline__ void ld_tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
@@ -85,10 +93,75 @@ __device__ __forceinline__ double lane_transpose_sum(double (&x)[32], int lane) 
     return x[0];
 }
 
-template <bool kMiss>
+// The annotated epilogue, annotations [c0, c0 + W) of one tile (t, c) of the full band: this lane's row j of c (a scored
+// SNP) against this warp's 64 partner rows i of t.  For every annotation the sum runs over the partners in ascending
+// order, one r2adj = fma(1 + alpha, r^2, -alpha) per pair and acc = fma(r2adj, a_ic, acc): it depends neither on W nor on
+// the number of annotations.  The sums go to slots[slot + c0 .. c0 + W).
+template <bool kMiss, int W>
+__device__ __forceinline__ void ld_annot_group(const LdArgs& a, const LdTile& tl, const LdRow* rs, const LdRow& rj, bool diag,
+                                               int half, int jl, int lane, uint32_t tlane, double* stage, int c0, double* slot) {
+    const int64_t i0 = (int64_t)tl.ti * kLdTile + half * 64;
+    __syncwarp();                                                    // every lane is done with the previous group's values
+    for (int e = lane; e < 64 * W; e += 32) stage[e] = a.annot[(i0 + e / W) * a.n_annot + c0 + e % W];
+    __syncwarp();
+    double acc[W];
+#pragma unroll
+    for (int g = 0; g < W; ++g) acc[g] = 0.0;
+    const double alpha = a.alpha, ap1 = 1.0 + alpha;
+    auto term = [&](int r, double rr) {
+        double r2 = rr * rr;
+        if (diag && half * 64 + r == jl) r2 = 1.0;
+        const int ig = (int)i0 + r;
+        const double v = (ig >= rj.lo && ig <= rj.hi) ? fma(ap1, r2, -alpha) : 0.0;   // a select: padding rows carry NaN
+        const double* av = stage + r * W;                                           // warp-uniform: a broadcast
+#pragma unroll
+        for (int g = 0; g < W; ++g) acc[g] = fma(v, av[g], acc[g]);
+    };
+    if (!kMiss) {
+        const double dn = (double)a.n_ref, Sj = rj.S, wj = rj.w * dn;
+#pragma unroll 1
+        for (int c8 = 0; c8 < 8; ++c8) {
+            uint32_t v[8];
+            asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+                         : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
+                         : "r"(tlane + (uint32_t)(c8 * 8))
+                         : "memory");
+            tmem_ld_wait();
+#pragma unroll
+            for (int k = 0; k < 8; ++k) {
+                const LdRow& ri = rs[c8 * 8 + k];
+                term(c8 * 8 + k, fma(-ri.S, Sj, u32_to_f64(v[k]) * dn) * ri.w * wj);
+            }
+        }
+    } else {
+        const int64_t Nj = rj.N, Sj = (int64_t)rj.S;
+#pragma unroll 1
+        for (int c16 = 0; c16 < 4; ++c16) {
+            const uint32_t col0 = (uint32_t)(c16 * 16);
+            uint32_t v0[16], v1[16], v2[16], v3[16];
+            ld_tmem_ld16(tlane + col0, v0);
+            ld_tmem_ld16(tlane + kLdTile + col0, v1);
+            ld_tmem_ld16(tlane + 2 * kLdTile + col0, v2);
+            ld_tmem_ld16(tlane + 3 * kLdTile + col0, v3);
+            tmem_ld_wait();
+#pragma unroll
+            for (int k = 0; k < 16; ++k) {
+                const LdRow& ri = rs[c16 * 16 + k];
+                const int64_t Ni = ri.N, Si = (int64_t)ri.S;
+                const int64_t num = Ni * Nj * (int64_t)v0[k] - Ni * Sj * (int64_t)v2[k] - Nj * Si * (int64_t)v1[k] +
+                                    Si * Sj * (int64_t)v3[k];
+                term(c16 * 16 + k, (double)num * ri.w * rj.w);
+            }
+        }
+    }
+#pragma unroll
+    for (int g = 0; g < W; ++g) slot[c0 + g] = acc[g];
+}
+
+template <bool kMiss, bool kAnnot = false>
 __global__ void __launch_bounds__(kLdThreads, 1)
 ld_band_kernel(const __grid_constant__ CUtensorMap tmap, const LdArgs a) {
-    using Cfg = LdCfg<kMiss>;
+    using Cfg = LdCfg<kMiss, kAnnot>;
     extern __shared__ uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t full_bar[Cfg::kStages], empty_bar[Cfg::kStages], acc_full[Cfg::kAcc], acc_empty[Cfg::kAcc];
     __shared__ __align__(16) LdRow rows_s[8][64];        // per epilogue warp: the constants of its 64 rows of tile t
@@ -175,6 +248,40 @@ ld_band_kernel(const __grid_constant__ CUtensorMap tmap, const LdArgs a) {
                 }
                 __syncwarp();
             }
+            ++lt;
+        }
+    } else if (kAnnot) {
+        // full band: a tile (t, c) scores the rows of c (TMEM lanes) against the partners of t; one slot per (row, tile,
+        // half, annotation), added in order by ld_annot_reduce_kernel
+        const int e = warp - 2, q = warp & 3, half = e >> 2;
+        LdRow* rs = rows_s[e];
+        double* stage = reinterpret_cast<double*>(smem + (size_t)Cfg::kStages * Cfg::kStageBytes) + e * 64 * kLdGroup;
+        const int jl = q * 32 + lane, C = a.n_annot;
+        uint32_t lt = 0;
+        for (int t = t0; t < n_tiles; t += tstride) {
+            const LdTile tl = ld_tile_rec(a.tiles + t);
+            if (ld_tile_missing(a, tl) != kMiss) continue;
+            const bool diag = (tl.ti == tl.tj);
+            const LdRow rj = a.rows[tl.tj * kLdTile + jl];
+            __syncwarp();
+            rs[lane] = a.rows[tl.ti * kLdTile + half * 64 + lane];
+            rs[32 + lane] = a.rows[tl.ti * kLdTile + half * 64 + 32 + lane];
+            __syncwarp();
+            const uint32_t as = lt % Cfg::kAcc;
+            mbar_wait(&acc_full[as], (lt / Cfg::kAcc) & 1u);
+            tc_fence_after();
+            const uint32_t tlane = tmem_base + as * Cfg::kAccCols + ((uint32_t)(q * 32) << 16) + (uint32_t)(half * 64);
+            double* slot = a.slots + tl.sr + (int64_t)jl * tl.sr_stride + half * C;
+            // groups of kLdGroup, then 8, 4, 2, 1: the accumulator stays in TMEM until the last one is done
+            int c0 = 0;
+            for (; c0 + kLdGroup <= C; c0 += kLdGroup) ld_annot_group<kMiss, kLdGroup>(a, tl, rs, rj, diag, half, jl, lane, tlane, stage, c0, slot);
+            if (C - c0 >= 8) { ld_annot_group<kMiss, 8>(a, tl, rs, rj, diag, half, jl, lane, tlane, stage, c0, slot); c0 += 8; }
+            if (C - c0 >= 4) { ld_annot_group<kMiss, 4>(a, tl, rs, rj, diag, half, jl, lane, tlane, stage, c0, slot); c0 += 4; }
+            if (C - c0 >= 2) { ld_annot_group<kMiss, 2>(a, tl, rs, rj, diag, half, jl, lane, tlane, stage, c0, slot); c0 += 2; }
+            if (C - c0 >= 1) ld_annot_group<kMiss, 1>(a, tl, rs, rj, diag, half, jl, lane, tlane, stage, c0, slot);
+            tc_fence_before();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&acc_empty[as]);
             ++lt;
         }
     } else {
@@ -319,6 +426,24 @@ __global__ void ld_reduce_kernel(const double* __restrict__ slots, const int64_t
     l2[p] = fma(sum, 1.0 + a, -(a * (double)w));
 }
 
+// The annotated sums of one segment: l2[p][c] = sum_u slots[base(p) + u C + c] over the 2 x (tile columns) slots of
+// scored row p in ascending (tile column, half) order, base(p) = sbase[p / 128] + (p % 128) * 2 nslot[p / 128] * C; NaN for
+// padding rows.  rows[row0 + p] is the LdRow of scored row p.
+__global__ void ld_annot_reduce_kernel(const double* __restrict__ slots, const int64_t* __restrict__ sbase,
+                                       const int32_t* __restrict__ nslot, const LdRow* __restrict__ rows, int64_t row0,
+                                       int64_t n_rows, int32_t C, double* __restrict__ l2) {
+    const int64_t x = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (x >= n_rows * C) return;
+    const int64_t p = x / C, T = p / kLdTile;
+    const int c = (int)(x - p * C);
+    if (rows[row0 + p].g < 0) { l2[x] = __longlong_as_double(0x7FF8000000000000ll); return; }
+    const int32_t ns = 2 * nslot[T];
+    const double* s = slots + sbase[T] + (p % kLdTile) * ns * (int64_t)C + c;
+    double sum = 0.0;
+    for (int32_t u = 0; u < ns; ++u) sum += s[(int64_t)u * C];
+    l2[x] = sum;
+}
+
 cudaError_t launch_ld_group_flags(const LdRow* rows, int32_t n_groups, const int32_t* rowN, int32_t n_ref, int32_t* gflags,
                                   int32_t* any, cudaStream_t st) {
     if (n_groups == 0) return cudaSuccess;
@@ -339,6 +464,29 @@ cudaError_t launch_ld_band(const CUtensorMap& tmap, const LdArgs& a, int n_sm, c
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     ld_band_kernel<true><<<grid, kLdThreads, LdCfg<true>::kSmem, st>>>(tmap, a);
+    return cudaGetLastError();
+}
+
+// The annotated band: both kernels over the same full-band tile list, as launch_ld_band.
+cudaError_t launch_ld_band_annot(const CUtensorMap& tmap, const LdArgs& a, int n_sm, cudaStream_t st) {
+    if (a.n_tiles == 0) return cudaSuccess;
+    const int grid = std::min(a.n_tiles, n_sm);
+    cudaError_t e = cudaFuncSetAttribute(ld_band_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, LdCfg<false, true>::kSmem);
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(ld_band_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, LdCfg<true, true>::kSmem);
+    if (e != cudaSuccess) return e;
+    ld_band_kernel<false, true><<<grid, kLdThreads, LdCfg<false, true>::kSmem, st>>>(tmap, a);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    ld_band_kernel<true, true><<<grid, kLdThreads, LdCfg<true, true>::kSmem, st>>>(tmap, a);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_ld_annot_reduce(const double* slots, const int64_t* sbase, const int32_t* nslot, const LdRow* rows, int64_t row0,
+                                   int64_t n_rows, int32_t n_annot, double* l2, cudaStream_t st) {
+    const int64_t n = n_rows * n_annot;
+    if (n == 0) return cudaSuccess;
+    ld_annot_reduce_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(slots, sbase, nslot, rows, row0, n_rows, n_annot, l2);
     return cudaGetLastError();
 }
 

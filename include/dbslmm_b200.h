@@ -244,6 +244,24 @@ DBSLMM_B200_API int  dbslmm_b200_ldscore(dbslmm_b200_handle* h, const uint8_t* b
                          int32_t wind_kind, const double* coord, double max_dist, double maf_min, int64_t segment_rows,
                          uint8_t* kept_out, double* maf_out, double* l2_out, int32_t* guard_out, float* kernel_ms_out);
 
+/* Partitioned LD Scores (`ldsc.py --l2 --annot`): one LD Score per annotation column c,
+ *   L_c(j) = sum_{k in W(j)} r2adj(j, k) a_kc,
+ * with dbslmm_b200_ldscore's kept set, windows, guard, r and r2adj.  As ldsc does, the unbiased map is applied per term:
+ * r2adj = fma(1 + 1/denominator, r^2, -1/denominator) once per pair, then acc_c = fma(r2adj, a_kc, acc_c), the partners k
+ * in ascending order within each 128-SNP tile and the tiles in ascending order.  annot is row-major [n_rows][n_annot],
+ * aligned with rows, every value finite; 1 <= n_annot <= DBSLMM_B200_LD_MAX_ANNOT.  l2_out is [n_rows][n_annot] (NaN rows
+ * where a SNP is not kept); l2_out NULL stops after the statistics pass, as in dbslmm_b200_ldscore.  The other arguments
+ * and outputs are dbslmm_b200_ldscore's.  Column c does not depend on the other columns of the call: computed alone or
+ * among others it has the same bits.  Deterministic as dbslmm_b200_ldscore.  Device memory: O(segment + halo) x (2 x n_pad
+ * + 8 n_annot) bytes, 2 x n_annot doubles per (SNP of the segment, 128-row tile its window reaches), and the result,
+ * n_annot doubles per row.  Synchronous. */
+#define DBSLMM_B200_LD_MAX_ANNOT 4096
+DBSLMM_B200_API int  dbslmm_b200_ldscore_annot(dbslmm_b200_handle* h, const uint8_t* bed, int64_t n_snp, int32_t n_ref,
+                         const int32_t* rows, int64_t n_rows, const int32_t* chr_off, int32_t n_chr,
+                         int32_t wind_kind, const double* coord, double max_dist, double maf_min, int64_t segment_rows,
+                         const double* annot, int32_t n_annot,
+                         uint8_t* kept_out, double* maf_out, double* l2_out, int32_t* guard_out, float* kernel_ms_out);
+
 /* ---- inspection hooks used by the parity tests (operate on the state of the last fit) ---- */
 /* int8 codes of one decoded row of the last fit: SNP j of block `block` (its small SNPs first, then its large ones),
  * plane 0 = allele counts (missing -> 0), plane 1 = call mask (1 = called; holds the last mask written at that position,
