@@ -20,11 +20,15 @@ FLAG_PANEL_SUBSET = 8
 LD_WIND_COORD = 0
 LD_WIND_SNPS = 1
 LD_MAX_ANNOT = 4096
+ERR_SINK = -5
+# dbslmm_b200_ld_sink: (user, a0, a1, off[a1 - a0 + 1], b, r) -> 0 to go on
+LD_SINK = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_int64, C.c_int64, C.POINTER(C.c_int64), C.POINTER(C.c_int32),
+                      C.POINTER(C.c_double))
 
 EXPORTS = [
     "dbslmm_b200_abi_version", "dbslmm_b200_device_count", "dbslmm_b200_create", "dbslmm_b200_destroy",
     "dbslmm_b200_last_error", "dbslmm_b200_load_bed", "dbslmm_b200_snp_stats", "dbslmm_b200_plan_shards",
-    "dbslmm_b200_fit", "dbslmm_b200_fit_multi", "dbslmm_b200_host_alloc", "dbslmm_b200_host_free", "dbslmm_b200_score", "dbslmm_b200_score_prefetch", "dbslmm_b200_score_stream", "dbslmm_b200_ldscore", "dbslmm_b200_ldscore_annot", "dbslmm_b200_ld_windows", "dbslmm_b200_get_row_codes", "dbslmm_b200_get_block_sigma",
+    "dbslmm_b200_fit", "dbslmm_b200_fit_multi", "dbslmm_b200_host_alloc", "dbslmm_b200_host_free", "dbslmm_b200_score", "dbslmm_b200_score_prefetch", "dbslmm_b200_score_stream", "dbslmm_b200_ldscore", "dbslmm_b200_ldscore_annot", "dbslmm_b200_ld_windows", "dbslmm_b200_ld_pairs", "dbslmm_b200_get_row_codes", "dbslmm_b200_get_block_sigma",
     "dbslmm_b200_get_block_factor", "dbslmm_b200_get_block_gram", "dbslmm_b200_get_block_iters",
 ]
 
@@ -92,6 +96,10 @@ def load():
                                                   C.c_int32, C.c_int32, C.c_void_p, C.c_double, C.c_double, C.c_int64,
                                                   C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                                   C.POINTER(C.c_float)]
+        lib.dbslmm_b200_ld_pairs.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p,
+                                             C.c_int32, C.c_void_p, C.c_int32, C.c_double, C.c_double, C.c_int64, LD_SINK,
+                                             C.c_void_p, C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64),
+                                             C.POINTER(C.c_float)]
         lib.dbslmm_b200_ld_windows.argtypes = [C.c_void_p, C.c_int64, C.c_double, C.c_void_p, C.c_void_p]
         lib.dbslmm_b200_score_prefetch.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32]
         lib.dbslmm_b200_get_row_codes.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32]
@@ -353,6 +361,56 @@ class Engine:
             self._check(self.lib.dbslmm_b200_ldscore_annot(*common, annot.ctypes.data, annot.shape[1], *outs), "ldscore_annot")
         self.last_kernel_ms = ms.value
         return None if stats_only else l2, kept.astype(bool), maf, guard[:n_chr].astype(bool)
+
+    def ld_pairs(self, bed, n_ref, rows, chr_off, coord, *, max_snps=10, max_dist=1000000.0, r2_min=0.2, segment_rows=0):
+        """SNP pairs within a window and their r (dbslmm_b200_ld_pairs, `plink --r2`): chromosome c is
+        rows[chr_off[c]:chr_off[c+1]], coord (float64[rows.size]) its base-pair positions.  A pair (a, b), a < b positions in
+        rows, is kept when b - a <= max_snps - 1, coord[b] - coord[a] <= max_dist and r^2 >= r2_min.  Returns (a, b, r):
+        int64, int32 and float64 arrays in ascending (a, b) order.  self.last_usable (bool[rows.size]: rows that can form a
+        pair), self.last_n_miss_pairs (pairs with a SNP with missing calls) and self.last_kernel_ms are left behind."""
+        n_ref = int(n_ref)
+        pitch = (n_ref + 3) // 4
+        if not (isinstance(bed, np.ndarray) and bed.dtype == np.uint8 and bed.flags.c_contiguous):
+            bed = np.ascontiguousarray(bed, np.uint8)
+        rows = np.ascontiguousarray(rows, np.int32)
+        chr_off = np.ascontiguousarray(chr_off, np.int32)
+        coord = np.ascontiguousarray(coord, np.float64)
+        if coord.size != rows.size:
+            raise ValueError("ld_pairs: coord must have one entry per row")
+        if chr_off.size < 1:
+            raise ValueError("ld_pairs: chr_off needs n_chr + 1 entries")
+        parts_a, parts_b, parts_r = [], [], []
+        err = []
+
+        def take(user, a0, a1, off, b, r):
+            try:
+                o = np.ctypeslib.as_array(off, (a1 - a0 + 1,)).copy()
+                n = int(o[-1])
+                parts_a.append(np.repeat(np.arange(a0, a1, dtype=np.int64), np.diff(o)))
+                parts_b.append(np.ctypeslib.as_array(b, (n,)).copy() if n else np.zeros(0, np.int32))
+                parts_r.append(np.ctypeslib.as_array(r, (n,)).copy() if n else np.zeros(0, np.float64))
+                return 0
+            except BaseException as e:        # an exception must not cross the C frames
+                err.append(e)
+                return 1
+
+        sink = LD_SINK(take)
+        usable = np.zeros(rows.size, np.uint8)
+        n_pairs, n_miss, ms = C.c_int64(0), C.c_int64(0), C.c_float(0)
+        rc = self.lib.dbslmm_b200_ld_pairs(self.h, bed.ctypes.data, bed.size // pitch, n_ref, rows.ctypes.data, rows.size,
+                                           chr_off.ctypes.data, chr_off.size - 1, coord.ctypes.data, int(max_snps),
+                                           float(max_dist), float(r2_min), int(segment_rows), sink, None, usable.ctypes.data,
+                                           C.byref(n_pairs), C.byref(n_miss), C.byref(ms))
+        if err:
+            raise err[0]
+        self._check(rc, "ld_pairs")
+        self.last_usable = usable.astype(bool)
+        self.last_n_miss_pairs = n_miss.value
+        self.last_kernel_ms = ms.value
+        cat = lambda p, t: np.concatenate(p) if p else np.zeros(0, t)
+        a, b, r = cat(parts_a, np.int64), cat(parts_b, np.int32), cat(parts_r, np.float64)
+        assert a.size == n_pairs.value
+        return a, b, r
 
     # ---- inspection hooks (parity tests)
     def row_codes(self, block, j, n, plane=0):

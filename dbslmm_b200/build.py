@@ -1,6 +1,6 @@
 """In-tree build of the sm_100a library and the `dbslmm` CLI (explicit nvcc / g++ calls).
 
-    python -m dbslmm_b200.build            # libdbslmm_b200.so + build/dbslmm, build/valid, build/score, build/ldscore
+    python -m dbslmm_b200.build            # libdbslmm_b200.so + build/dbslmm, build/valid, build/score, build/ldscore, build/ld
 Outputs stay inside the repo (git-ignored) so they travel with a gpurun snapshot.
 """
 import concurrent.futures as cf
@@ -18,6 +18,7 @@ CLI = os.path.join(BUILD, "dbslmm")
 VALID_CLI = os.path.join(BUILD, "valid")
 SCORE_CLI = os.path.join(BUILD, "score")
 LDSCORE_CLI = os.path.join(BUILD, "ldscore")
+LD_CLI = os.path.join(BUILD, "ld")
 
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 GXX = "/usr/bin/g++"
@@ -89,6 +90,12 @@ def build_cli(force=False):
     ldeps = [lsrc, os.path.join(HOST, "plink_bed.hpp")] + deps
     if os.path.exists(lsrc) and (force or _newer(LDSCORE_CLI, ldeps)):
         _run([GXX, "-O2", "-std=c++17", "-pthread", "-I", os.path.join(ROOT, "include"), "-o", LDSCORE_CLI, lsrc] +
+             ["-L", PKG, "-ldbslmm_b200", "-Wl,-rpath,$ORIGIN/../dbslmm_b200", "-Wl,-rpath," + PKG, "-lz"])
+    # `ld`: plink --r2 (the table of SNP pairs within a window and their r^2)
+    dsrc = os.path.join(HOST, "ld_main.cpp")
+    ddeps = [dsrc, os.path.join(HOST, "plink_bed.hpp"), os.path.join(CSRC, "hostpool.hpp")] + deps
+    if os.path.exists(dsrc) and (force or _newer(LD_CLI, ddeps)):
+        _run([GXX, "-O2", "-std=c++17", "-pthread", "-I", os.path.join(ROOT, "include"), "-o", LD_CLI, dsrc] +
              ["-L", PKG, "-ldbslmm_b200", "-Wl,-rpath,$ORIGIN/../dbslmm_b200", "-Wl,-rpath," + PKG, "-lz"])
     return CLI
 

@@ -200,6 +200,7 @@ struct dbslmm_b200_handle {
     DevBuf s_dev[2], s_work;
     // LD scores (dbslmm_b200_ldscore): row statistics, segment code rows + dirty map, decoder scratch, partial slots, reduction
     DevBuf ld_stats, ld_codes, ld_dirty, ld_work, ld_slots, ld_red;
+    PinBuf ld_pin[2], ld_roff;           // SNP pairs (dbslmm_b200_ld_pairs): the two pinned pair buffers the sink reads, row offsets
     cudaEvent_t ev_pin_free[3] = {}, ev_copied[2] = {}, ev_slot_free[2] = {};
     std::vector<cudaEvent_t> ev_chunk;   // 4 timing events per chunk (copy begin / end, kernels begin / end), grow-only
     size_t dirty_rows = 0;               // code rows the dirty map covers
@@ -984,6 +985,8 @@ void dbslmm_b200_destroy(dbslmm_b200_handle* h) {
     for (DevBuf& b : h->s_dev) b.release();
     h->s_work.release();
     for (DevBuf* b : {&h->ld_stats, &h->ld_codes, &h->ld_dirty, &h->ld_work, &h->ld_slots, &h->ld_red}) b->release();
+    for (PinBuf& b : h->ld_pin) b.release();
+    h->ld_roff.release();
     for (cudaEvent_t e : h->ev_pin_free) if (e) cudaEventDestroy(e);
     for (int i = 0; i < 2; ++i) {
         if (h->ev_copied[i]) cudaEventDestroy(h->ev_copied[i]);
@@ -2191,6 +2194,46 @@ static int chunk_kernel_ms(dbslmm_b200_handle* h, const char* label, int64_t ev0
     return DBSLMM_B200_OK;
 }
 
+// .bed rows src(0..nr) -> dst (pitch bytes each), in pieces of >= 2 MB for the pool's workers
+template <class Src>
+static void gather_bed_rows(HostPool& pool, const uint8_t* bed, int64_t pitch, uint8_t* dst, int64_t nr, TaskGroup& g, Src src) {
+    const int64_t per = std::max<int64_t>(1, ((int64_t)2 << 20) / pitch);
+    for (int64_t r0 = 0; r0 < nr; r0 += per) {
+        const int64_t r1 = std::min<int64_t>(nr, r0 + per);
+        pool.submit(g, [=]() { for (int64_t r = r0; r < r1; ++r) std::memcpy(dst + r * pitch, bed + (int64_t)src(r) * pitch, (size_t)pitch); });
+    }
+}
+
+// Pass 1 of the LD calls: per-row statistics of .bed rows rows[0..n_rows) -> hs, streamed as chunks [0, *n_chunks) of
+// stream_chunks; *ms = their kernel time.
+static int ld_stats_pass(dbslmm_b200_handle* h, const uint8_t* bed, int32_t n_ref, const int32_t* rows, int64_t n_rows,
+                         const char* label, std::vector<SnpStat>& hs, int64_t* n_chunks, float* ms) {
+    cudaStream_t st = h->stream;
+    const int64_t pitch = (n_ref + 3) / 4;
+    HostPool& pool = host_pool();
+    const int64_t rows1 = std::max<int64_t>(1, std::min<int64_t>(std::max<int64_t>(n_rows, 1), (int64_t)(kStreamChunkDefault / (uint64_t)pitch)));
+    const int64_t n1 = (n_rows + rows1 - 1) / rows1;
+    CU_TRY(h, h->ld_stats.ensure(sizeof(SnpStat) * (size_t)std::max<int64_t>(n_rows, 1)));
+    SnpStat* d_stats = (SnpStat*)h->ld_stats.p;
+    auto rows_of1 = [&](int64_t k) { return std::min<int64_t>(rows1, n_rows - k * rows1); };
+    auto bytes_of1 = [&](int64_t k) { return align_up((size_t)std::max<int64_t>(rows_of1(k), 0) * pitch + 4, 256); };   // + 4: whole-word reads
+    int rc = stream_chunks(h, n1, bytes_of1(0), 0, bytes_of1,
+                           [&](int64_t k, uint8_t* dst, TaskGroup& g) {
+                               const int64_t j0 = k * rows1;
+                               gather_bed_rows(pool, bed, pitch, dst, rows_of1(k), g, [=](int64_t r) { return rows[j0 + r]; });
+                           },
+                           [&](int64_t k, const uint8_t* dev) -> int {
+                               CU_TRY(h, launch_chunk_stats(dev, (int32_t)rows_of1(k), n_ref, d_stats + k * rows1, nullptr, h->n_sm, st));
+                               return DBSLMM_B200_OK;
+                           });
+    if (rc != DBSLMM_B200_OK) return rc;
+    hs.assign((size_t)n_rows, SnpStat{});
+    if (n_rows > 0) CU_TRY(h, cudaMemcpyAsync(hs.data(), d_stats, sizeof(SnpStat) * (size_t)n_rows, cudaMemcpyDeviceToHost, st));
+    CU_TRY(h, cudaStreamSynchronize(st));
+    *n_chunks = n1;
+    return chunk_kernel_ms(h, label, 0, n1, rows_of1, bytes_of1, ms);
+}
+
 extern "C" {
 
 int dbslmm_b200_score_stream(dbslmm_b200_handle* h, const uint8_t* bed_val, int64_t n_snp_val, int32_t n_val,
@@ -2295,6 +2338,7 @@ struct LdSeg {
     int64_t n_slots = 0;              // annotated: partial sums of the segment
     size_t o_src = 0, o_crow = 0, o_mrow = 0, o_rows = 0, o_tiles = 0, bytes = 0;
     size_t o_annot = 0, o_sbase = 0, o_nslot = 0;    // annotated: annotation rows [R1 - R0][C], slot base and count per row tile
+    size_t o_rid = 0;                 // pairs: the caller's row index of each padded row
 };
 }  // namespace
 
@@ -2359,37 +2403,13 @@ static int ldscore_impl(dbslmm_b200_handle* h, const uint8_t* bed, int64_t n_snp
     const int64_t pitch = (n_ref + 3) / 4;
     const int32_t n_pad = (n_ref + 127) / 128 * 128;
     HostPool& pool = host_pool();
-    // .bed rows src[0..nr) -> dst (pitch bytes each), in pieces of >= 2 MB for the pool's workers
-    auto gather_rows = [&](uint8_t* dst, const int64_t nr, TaskGroup& g, auto src) {
-        const int64_t per = std::max<int64_t>(1, ((int64_t)2 << 20) / pitch);
-        for (int64_t r0 = 0; r0 < nr; r0 += per) {
-            const int64_t r1 = std::min<int64_t>(nr, r0 + per);
-            pool.submit(g, [=]() { for (int64_t r = r0; r < r1; ++r) std::memcpy(dst + r * pitch, bed + (int64_t)src(r) * pitch, (size_t)pitch); });
-        }
-    };
+    auto gather_rows = [&](uint8_t* dst, const int64_t nr, TaskGroup& g, auto src) { gather_bed_rows(pool, bed, pitch, dst, nr, g, src); };
 
     // ---- pass 1: per-row statistics of every requested row
-    const int64_t rows1 = std::max<int64_t>(1, std::min<int64_t>(std::max<int64_t>(n_rows, 1), (int64_t)(kStreamChunkDefault / (uint64_t)pitch)));
-    const int64_t n1 = (n_rows + rows1 - 1) / rows1;
-    CU_TRY(h, h->ld_stats.ensure(sizeof(SnpStat) * (size_t)std::max<int64_t>(n_rows, 1)));
-    SnpStat* d_stats = (SnpStat*)h->ld_stats.p;
-    auto rows_of1 = [&](int64_t k) { return std::min<int64_t>(rows1, n_rows - k * rows1); };
-    auto bytes_of1 = [&](int64_t k) { return align_up((size_t)std::max<int64_t>(rows_of1(k), 0) * pitch + 4, 256); };   // + 4: whole-word reads
-    int rc = stream_chunks(h, n1, bytes_of1(0), 0, bytes_of1,
-                           [&](int64_t k, uint8_t* dst, TaskGroup& g) {
-                               const int64_t j0 = k * rows1;
-                               gather_rows(dst, rows_of1(k), g, [=](int64_t r) { return rows[j0 + r]; });
-                           },
-                           [&](int64_t k, const uint8_t* dev) -> int {
-                               CU_TRY(h, launch_chunk_stats(dev, (int32_t)rows_of1(k), n_ref, d_stats + k * rows1, nullptr, h->n_sm, st));
-                               return DBSLMM_B200_OK;
-                           });
-    if (rc != DBSLMM_B200_OK) return rc;
-    std::vector<SnpStat> hs((size_t)n_rows);
-    if (n_rows > 0) CU_TRY(h, cudaMemcpyAsync(hs.data(), d_stats, sizeof(SnpStat) * (size_t)n_rows, cudaMemcpyDeviceToHost, st));
-    CU_TRY(h, cudaStreamSynchronize(st));
+    std::vector<SnpStat> hs;
     float ms1 = 0.0f;
-    rc = chunk_kernel_ms(h, "ldscore pass1", 0, n1, rows_of1, bytes_of1, &ms1);
+    int64_t n1 = 0;
+    int rc = ld_stats_pass(h, bed, n_ref, rows, n_rows, "ldscore pass1", hs, &n1, &ms1);
     if (rc != DBSLMM_B200_OK) return rc;
 
     // ---- kept SNPs (ldsc's __filter_snps_maf__): min(f, 1 - f) > maf_min and missing + het < n
@@ -2665,6 +2685,352 @@ int dbslmm_b200_ldscore_annot(dbslmm_b200_handle* h, const uint8_t* bed, int64_t
     if (!annot) return fail(h, DBSLMM_B200_ERR_ARG, "ldscore_annot: annot is NULL");
     return ldscore_impl(h, bed, n_snp, n_ref, rows, n_rows, chr_off, n_chr, wind_kind, coord, max_dist, maf_min, segment_rows,
                         annot, n_annot, kept_out, maf_out, l2_out, guard_out, kernel_ms_out);
+}
+
+// ---------------------------------------------------------------------------------------------
+// SNP pairs (plink --r2), see ldscore.cu.  Pass 1 is ldscore's statistics pass; every row of a chromosome (usable or not)
+// then takes a padded row from a 128-row boundary, so positions in rows and padded rows differ by a constant within a
+// chromosome.  A row tile T lists the tiles (T, P), T <= P <= the tile of its last row's window end.  Segments of
+// consecutive row tiles with their right halo are streamed as in ldscore; for each, the count pass and the offsets scan
+// run, the host reads the per-row offsets and cuts the segment into ranges of row tiles whose pairs fit the pair buffer,
+// and each range is emitted, copied to pinned buffer (range number % 2) and handed to the sink while the next range runs.
+// ---------------------------------------------------------------------------------------------
+static constexpr int64_t kLdPairBuf = (int64_t)1 << 23;      // pairs of the device buffer (12 bytes each)
+
+int dbslmm_b200_ld_pairs(dbslmm_b200_handle* h, const uint8_t* bed, int64_t n_snp, int32_t n_ref, const int32_t* rows,
+                         int64_t n_rows, const int32_t* chr_off, int32_t n_chr, const double* coord, int32_t max_snps,
+                         double max_dist, double r2_min, int64_t segment_rows, dbslmm_b200_ld_sink sink, void* user,
+                         uint8_t* usable_out, int64_t* n_pairs_out, int64_t* n_miss_pairs_out, float* kernel_ms_out) {
+    if (!h) return DBSLMM_B200_ERR_ARG;
+    auto bad = [&](const std::string& m) { return fail(h, DBSLMM_B200_ERR_ARG, "ld_pairs: " + m); };
+    if (!bed || n_snp <= 0 || n_ref <= 0 || n_rows < 0 || n_chr < 0 || !chr_off || (n_rows > 0 && (!rows || !coord)))
+        return bad("bad arguments");
+    if (!sink) return bad("sink is NULL");
+    if (n_ref > decode_max_n_ref())
+        return bad("n_ref = " + std::to_string(n_ref) + " is above the limit of " + std::to_string(decode_max_n_ref()) +
+                   " individuals (the decoder stages whole .bed rows in shared memory)");
+    if (n_rows > INT32_MAX) return bad("n_rows = " + std::to_string(n_rows) + " is above INT32_MAX");
+    if (max_snps < 1) return bad("max_snps must be >= 1");
+    if (!(max_dist >= 0)) return bad("max_dist must be >= 0");
+    if (std::isnan(r2_min)) return bad("r2_min is NaN");
+    if (segment_rows < 0 || segment_rows % 128 != 0) return bad("segment_rows must be 0 or a positive multiple of 128");
+    if (chr_off[0] != 0 || chr_off[n_chr] != n_rows) return bad("bad chromosome offsets: chr_off[0] must be 0 and chr_off[n_chr] = n_rows");
+    for (int32_t c = 0; c < n_chr; ++c)
+        if (chr_off[c + 1] < chr_off[c]) return bad("bad chromosome offsets: chr_off[" + std::to_string(c + 1) + "] < chr_off[" + std::to_string(c) + "]");
+    for (int64_t i = 0; i < n_rows; ++i)
+        if (rows[i] < 0 || rows[i] >= n_snp) return bad("rows[" + std::to_string(i) + "] = " + std::to_string(rows[i]) + " is out of range of the .bed");
+    for (int32_t c = 0; c < n_chr; ++c)
+        for (int64_t i = chr_off[c]; i < chr_off[c + 1]; ++i) {
+            if (!std::isfinite(coord[i])) return bad("coord[" + std::to_string(i) + "] is not finite");
+            if (i > chr_off[c] && coord[i] < coord[i - 1])
+                return bad("the coordinates of chromosome " + std::to_string(c) + " are not sorted: coord[" + std::to_string(i) + "] < coord[" +
+                           std::to_string(i - 1) + "]");
+        }
+    CU_TRY(h, cudaSetDevice(h->device));
+    cudaStream_t st = h->stream;
+    const int64_t pitch = (n_ref + 3) / 4;
+    const int32_t n_pad = (n_ref + 127) / 128 * 128;
+    HostPool& pool = host_pool();
+
+    // ---- pass 1: statistics; usable rows have a called genotype and nonzero variance
+    std::vector<SnpStat> hs;
+    float ms = 0.0f;
+    int64_t n1 = 0;
+    int rc = ld_stats_pass(h, bed, n_ref, rows, n_rows, "ld_pairs pass1", hs, &n1, &ms);
+    if (rc != DBSLMM_B200_OK) return rc;
+    std::vector<uint8_t> usable((size_t)n_rows);
+    for (int64_t i = 0; i < n_rows; ++i) {
+        const SnpStat& x = hs[i];
+        usable[i] = (x.n_nonmiss > 0 && (int64_t)x.n_nonmiss * x.sumsq - (int64_t)x.sum * x.sum > 0) ? 1 : 0;
+        if (usable_out) usable_out[i] = usable[i];
+    }
+
+    // ---- padded rows, windows (hi: the last partner's position), tiles; ub: the most pairs a row tile can have
+    std::vector<int64_t> prow((size_t)n_rows), hi((size_t)n_rows), trow0, thi, ub;
+    for (int32_t c = 0; c < n_chr; ++c) {
+        const int64_t i0 = chr_off[c], m = chr_off[c + 1] - i0, T_c = (int64_t)thi.size();
+        int64_t j = 0;
+        for (int64_t k = 0; k < m; ++k) {
+            j = std::max(j, k);
+            while (j + 1 < m && j + 1 - k <= (int64_t)max_snps - 1 && coord[i0 + j + 1] - coord[i0 + k] <= max_dist) ++j;
+            prow[i0 + k] = 128 * T_c + k;
+            hi[i0 + k] = i0 + j;
+        }
+        for (int64_t t = 0; t < (m + 127) / 128; ++t) {
+            const int64_t a0 = i0 + 128 * t, a1 = std::min(i0 + m, a0 + 128);
+            trow0.push_back(a0);
+            thi.push_back(prow[hi[a1 - 1]] / 128);
+            int64_t u = 0;
+            for (int64_t a = a0; a < a1; ++a) u += usable[a] ? hi[a] - a : 0;
+            ub.push_back(u);
+        }
+    }
+    const int64_t n_trows = (int64_t)thi.size();
+    trow0.push_back(n_rows);
+    std::vector<int64_t> upad;                          // padded rows of the usable rows (the decoded ones)
+    std::vector<int32_t> urow;
+    for (int64_t i = 0; i < n_rows; ++i) if (usable[i]) { upad.push_back(prow[i]); urow.push_back((int32_t)i); }
+    int64_t ub_max = 1, ub_sum = 0;
+    for (int64_t u : ub) { ub_max = std::max(ub_max, u); ub_sum += u; }
+    const int64_t pcap = std::max(ub_max, std::min(kLdPairBuf, ub_sum));
+    int64_t n_pairs = 0, n_miss = 0;
+    if (upad.empty()) {                                 // no row can form a pair: the sink still sees every row
+        std::vector<int64_t> off((size_t)n_rows + 1, 0);
+        if (n_rows > 0 && sink(user, 0, n_rows, off.data(), nullptr, nullptr) != 0)
+            return fail(h, DBSLMM_B200_ERR_SINK, "ld_pairs: the sink returned nonzero");
+        if (n_pairs_out) *n_pairs_out = 0;
+        if (n_miss_pairs_out) *n_miss_pairs_out = 0;
+        if (kernel_ms_out) *kernel_ms_out = ms;
+        return DBSLMM_B200_OK;
+    }
+
+    // ---- segments (as ldscore's): 64 MB of .bed rows, halved while the code rows with their halo and the count slots take
+    // more than half of the free device memory; a nonzero segment_rows fixes them
+    auto plan = [&](int64_t seg_tiles, std::vector<LdSeg>& segs) {
+        segs.clear();
+        int64_t cap = 0;
+        for (int64_t T0 = 0; T0 < n_trows; T0 += seg_tiles) {
+            LdSeg S;
+            S.T0 = T0;
+            S.T1 = std::min(n_trows, T0 + seg_tiles);
+            S.R0 = 128 * S.T0;
+            S.R1 = 128 * (thi[S.T1 - 1] + 1);
+            S.K0 = std::lower_bound(upad.begin(), upad.end(), S.R0) - upad.begin();
+            S.K1 = std::lower_bound(upad.begin(), upad.end(), S.R1) - upad.begin();
+            for (int64_t T = S.T0; T < S.T1; ++T) {
+                S.n_tiles += thi[T] - T + 1;
+                S.n_slots += 2 * 128 * (thi[T] - T + 1);
+            }
+            const int64_t nr = S.K1 - S.K0, np = S.R1 - S.R0, nt = S.T1 - S.T0;
+            S.o_src = align_up((size_t)nr * pitch + 16, 256);
+            S.o_crow = align_up(S.o_src + sizeof(uint32_t) * nr, 256);
+            S.o_mrow = align_up(S.o_crow + sizeof(int32_t) * nr, 256);
+            S.o_rows = align_up(S.o_mrow + sizeof(int32_t) * nr, 256);
+            S.o_tiles = align_up(S.o_rows + sizeof(LdRow) * np, 256);
+            S.o_rid = align_up(S.o_tiles + sizeof(LdTile) * S.n_tiles, 256);
+            S.o_sbase = align_up(S.o_rid + sizeof(int32_t) * np, 256);
+            S.o_nslot = align_up(S.o_sbase + sizeof(int64_t) * nt, 256);
+            S.bytes = align_up(S.o_nslot + sizeof(int32_t) * nt, 256);
+            cap = std::max(cap, np);
+            segs.push_back(S);
+        }
+        return cap;
+    };
+    auto seg_slots = [&](const std::vector<LdSeg>& segs) {
+        int64_t m = 0;
+        for (const LdSeg& S : segs) m = std::max(m, S.n_slots);
+        return m;
+    };
+    std::vector<LdSeg> segs;
+    int64_t seg_tiles = segment_rows > 0 ? segment_rows / 128 : std::max<int64_t>(1, (int64_t)(kStreamChunkDefault / (uint64_t)(128 * pitch)));
+    int64_t cap = plan(seg_tiles, segs);
+    size_t free_b = 0, total_b = 0;
+    CU_TRY(h, cudaMemGetInfo(&free_b, &total_b));
+    auto need = [&](int64_t cp) { return (double)cp * (2.0 * n_pad + 2.0 + 48.0); };
+    if (segment_rows == 0)
+        while (seg_tiles > 1 && need(cap) + 12.0 * (double)seg_slots(segs) > 0.5 * (double)free_b) cap = plan(seg_tiles = (seg_tiles + 1) / 2, segs);
+    const int64_t n_slots = seg_slots(segs), max_srows = 128 * std::min(seg_tiles, n_trows);
+    if (need(cap) + 12.0 * (double)n_slots + 12.0 * (double)pcap > 0.9 * (double)free_b)
+        return fail(h, DBSLMM_B200_ERR_NOMEM, "ld_pairs: a segment of " + std::to_string(cap) + " rows (with the halo its windows reach), " +
+                                              std::to_string(n_slots) + " count slots and a buffer of " + std::to_string(pcap) +
+                                              " pairs do not fit in device memory");
+    size_t max_bytes = 0;
+    for (const LdSeg& S : segs) max_bytes = std::max(max_bytes, S.bytes);
+
+    // ---- device buffers: code rows and dirty map (as ldscore), decoder outputs, group flags, error flag and missing-call
+    // count; count slots | slot offsets | row offsets; the pair buffer b | r; the two pinned pair buffers
+    CU_TRY(h, h->ld_codes.ensure((size_t)2 * cap * n_pad));
+    CU_TRY(h, h->ld_dirty.ensure((size_t)2 * cap));
+    CU_TRY(h, cudaMemsetAsync(h->ld_dirty.p, 1, (size_t)2 * cap, st));
+    size_t o = 0;
+    auto place = [&](size_t b) { size_t r = o; o = align_up(o + b, 256); return r; };
+    const size_t o_rowN = place(sizeof(int32_t) * cap), o_rowS = place(sizeof(int32_t) * cap), o_rowR = place(sizeof(double) * cap),
+                 o_rowC = place(sizeof(double2) * cap), o_gfl = place(sizeof(int32_t) * (cap / 128 + 1)),
+                 o_err = place(sizeof(int32_t)), o_nmiss = place(sizeof(unsigned long long));
+    CU_TRY(h, h->ld_work.ensure(o));
+    uint8_t* wk = (uint8_t*)h->ld_work.p;
+    int32_t* rowN = (int32_t*)(wk + o_rowN);
+    int32_t* gflags = (int32_t*)(wk + o_gfl);
+    int32_t* d_err = (int32_t*)(wk + o_err);
+    unsigned long long* d_nmiss = (unsigned long long*)(wk + o_nmiss);
+    CU_TRY(h, cudaMemsetAsync(wk + o_err, 0, o - o_err, st));
+    o = 0;
+    const size_t o_cnt = place(sizeof(int32_t) * n_slots), o_off = place(sizeof(int64_t) * n_slots),
+                 o_roff = place(sizeof(int64_t) * (max_srows + 1));
+    CU_TRY(h, h->ld_slots.ensure(o));
+    uint8_t* sl = (uint8_t*)h->ld_slots.p;
+    int32_t* d_cnt = (int32_t*)(sl + o_cnt);
+    int64_t* d_off = (int64_t*)(sl + o_off);
+    int64_t* d_roff = (int64_t*)(sl + o_roff);
+    const size_t o_pr = align_up(sizeof(int32_t) * (size_t)pcap, 256);
+    CU_TRY(h, h->ld_red.ensure(o_pr + sizeof(double) * (size_t)pcap));
+    int32_t* d_pb = (int32_t*)h->ld_red.p;
+    double* d_pr = (double*)((uint8_t*)h->ld_red.p + o_pr);
+    const size_t o_flag = align_up(o_pr + sizeof(double) * (size_t)pcap, 256);     // the error flag as of the range's emit
+    for (PinBuf& b : h->ld_pin) CU_TRY(h, b.ensure(o_flag + sizeof(int32_t)));
+    CUtensorMap tmap;
+    rc = make_tensor_map(h, &tmap, h->ld_codes.p, 2 * cap, n_pad, 128);
+    if (rc != DBSLMM_B200_OK) return rc;
+    struct Events {
+        cudaEvent_t e[8] = {};
+        ~Events() { for (cudaEvent_t x : e) if (x) cudaEventDestroy(x); }
+    } ev;                                               // count pass begin / end; per pinned buffer: emit begin / end, copied
+    for (cudaEvent_t& x : ev.e) CU_TRY(h, cudaEventCreate(&x));
+
+    // ---- the range handed to the sink next: pinned buffer x (-1: no pairs, nothing on the device), rows a0 .. a1
+    struct Range { int x = -1; int64_t a0 = 0, a1 = 0, n = 0; std::vector<int64_t> off; bool on = false; } pend;
+    int64_t n_ranges = 0;
+    auto flush = [&]() -> int {
+        if (!pend.on) return DBSLMM_B200_OK;
+        pend.on = false;
+        const int32_t* pb = nullptr;
+        const double* pr = nullptr;
+        if (pend.x >= 0) {
+            CU_TRY(h, cudaEventSynchronize(ev.e[2 + 3 * pend.x + 2]));
+            float t = 0.0f;
+            CU_TRY(h, cudaEventElapsedTime(&t, ev.e[2 + 3 * pend.x], ev.e[2 + 3 * pend.x + 1]));
+            ms += t;
+            const uint8_t* pin = (const uint8_t*)h->ld_pin[pend.x].p;
+            if (*(const int32_t*)(pin + o_flag))       // checked before the sink sees the range
+                return fail(h, DBSLMM_B200_ERR_CUDA, "ld_pairs: the emit pass wrote other pairs than the count pass counted (rows " +
+                                                     std::to_string(pend.a0) + ".." + std::to_string(pend.a1 - 1) + ")");
+            pb = (const int32_t*)pin;
+            pr = (const double*)(pin + o_pr);
+        }
+        n_pairs += pend.n;
+        if (sink(user, pend.a0, pend.a1, pend.off.data(), pb, pr) != 0)
+            return fail(h, DBSLMM_B200_ERR_SINK, "ld_pairs: the sink returned nonzero for rows " + std::to_string(pend.a0) + ".." +
+                                                 std::to_string(pend.a1 - 1));
+        return DBSLMM_B200_OK;
+    };
+
+    auto gather2 = [&](int64_t k, uint8_t* dst, TaskGroup& g) {
+        const LdSeg& S = segs[k];
+        const int64_t nr = S.K1 - S.K0, np = S.R1 - S.R0;
+        const int32_t* ur = urow.data() + S.K0;
+        gather_bed_rows(pool, bed, pitch, dst, nr, g, [=](int64_t r) { return rows[ur[r]]; });
+        uint32_t* src = (uint32_t*)(dst + S.o_src);
+        int32_t* crow = (int32_t*)(dst + S.o_crow);
+        int32_t* mrow = (int32_t*)(dst + S.o_mrow);
+        LdRow* lr = (LdRow*)(dst + S.o_rows);
+        LdTile* tl = (LdTile*)(dst + S.o_tiles);
+        int32_t* rid = (int32_t*)(dst + S.o_rid);
+        int64_t* sbase = (int64_t*)(dst + S.o_sbase);
+        int32_t* nslot = (int32_t*)(dst + S.o_nslot);
+        for (int64_t p = 0; p < np; ++p) { lr[p] = LdRow{0.0, std::nan(""), 0, 1, -1, -1}; rid[p] = -1; }
+        for (int64_t T = S.T0; T <= thi[S.T1 - 1] && T < n_trows; ++T)
+            for (int64_t i = trow0[T]; i < trow0[T + 1]; ++i) rid[prow[i] - S.R0] = (int32_t)i;
+        for (int64_t g2 = 0; g2 < nr; ++g2) {
+            const int64_t i = urow[S.K0 + g2], p = prow[i] - S.R0;
+            const SnpStat& x = hs[i];
+            const double d = (double)((int64_t)x.n_nonmiss * x.sumsq - (int64_t)x.sum * x.sum);
+            src[g2] = (uint32_t)g2;
+            crow[g2] = (int32_t)p;
+            mrow[g2] = (int32_t)(p + cap);
+            lr[p] = LdRow{(double)x.sum, 1.0 / std::sqrt((double)x.n_nonmiss * d), x.n_nonmiss, 0, (int32_t)(prow[hi[i]] - S.R0), (int32_t)g2};
+        }
+        int64_t n = 0, sb = 0;
+        for (int64_t T = S.T0; T < S.T1; ++T) {
+            const int32_t ns = (int32_t)(thi[T] - T + 1);
+            sbase[T - S.T0] = sb;
+            nslot[T - S.T0] = ns;
+            for (int64_t P = T; P <= thi[T]; ++P)
+                tl[n++] = LdTile{(int32_t)(P - S.T0), (int32_t)(T - S.T0), 2 * ns, 0, sb + 2 * (P - T), 0};
+            sb += 2 * 128 * (int64_t)ns;
+        }
+    };
+    CU_TRY(h, h->ld_roff.ensure(sizeof(int64_t) * (size_t)(max_srows + 1)));
+    const int64_t* hroff = (const int64_t*)h->ld_roff.p;
+    auto launch2 = [&](int64_t k, const uint8_t* dev) -> int {
+        const LdSeg& S = segs[k];
+        const int64_t nr = S.K1 - S.K0, ngrp = (S.R1 - S.R0) / 128, nsr = 128 * (S.T1 - S.T0);
+        CU_TRY(h, cudaEventRecord(ev.e[0], st));
+        CU_TRY(h, launch_decode_rows(dev, n_ref, n_pad, (const uint32_t*)(dev + S.o_src), (const int32_t*)(dev + S.o_crow),
+                                     (const int32_t*)(dev + S.o_mrow), 0, nr, 1.0, (int8_t*)h->ld_codes.p, (uint8_t*)h->ld_dirty.p,
+                                     rowN, (int32_t*)(wk + o_rowS), (double*)(wk + o_rowR), (double2*)(wk + o_rowC), nullptr, h->n_sm, st));
+        CU_TRY(h, cudaMemsetAsync(gflags, 0, sizeof(int32_t) * (size_t)(ngrp + 1), st));
+        const LdRow* lr = (const LdRow*)(dev + S.o_rows);
+        CU_TRY(h, launch_ld_group_flags(lr, (int32_t)ngrp, rowN, n_ref, gflags, gflags + ngrp, st));
+        LdArgs a{};
+        a.tiles = (const LdTile*)(dev + S.o_tiles);
+        a.n_tiles = (int32_t)S.n_tiles;
+        a.nk = n_pad / 128;
+        a.n_ref = n_ref;
+        a.mask_off = (int32_t)cap;
+        a.rows = lr;
+        a.gflags = gflags;
+        a.any = gflags + ngrp;
+        LdPairArgs p{};
+        p.r2_min = r2_min;
+        p.cnt = d_cnt;
+        CU_TRY(h, launch_ld_pairs(tmap, a, p, false, h->n_sm, st));
+        CU_TRY(h, launch_ld_pair_scan(d_cnt, (const int64_t*)(dev + S.o_sbase), (const int32_t*)(dev + S.o_nslot), nsr, d_off, d_roff, st));
+        CU_TRY(h, cudaEventRecord(ev.e[1], st));
+        CU_TRY(h, cudaMemcpyAsync(h->ld_roff.p, d_roff, sizeof(int64_t) * (size_t)(nsr + 1), cudaMemcpyDeviceToHost, st));
+        int r = flush();                                // the previous range's sink runs while this segment is counted
+        if (r != DBSLMM_B200_OK) return r;
+        CU_TRY(h, cudaStreamSynchronize(st));
+        float t = 0.0f;
+        CU_TRY(h, cudaEventElapsedTime(&t, ev.e[0], ev.e[1]));
+        ms += t;
+        // ranges of row tiles [Ta, Tb) whose pairs fit the buffer (one tile always does: pcap >= its bound)
+        std::vector<int64_t> tfirst((size_t)(S.T1 - S.T0) + 1, 0);
+        for (int64_t T = S.T0; T < S.T1; ++T) tfirst[T - S.T0 + 1] = tfirst[T - S.T0] + (thi[T] - T + 1);
+        auto at = [&](int64_t T) { return hroff[(size_t)(128 * (T - S.T0))]; };
+        for (int64_t Ta = S.T0; Ta < S.T1;) {
+            int64_t Tb = Ta + 1;
+            while (Tb < S.T1 && at(Tb + 1) - at(Ta) <= pcap) ++Tb;
+            Range R;
+            R.a0 = trow0[Ta];
+            R.a1 = trow0[Tb];
+            R.n = at(Tb) - at(Ta);
+            R.off.resize((size_t)(R.a1 - R.a0 + 1));
+            for (int64_t i = R.a0; i < R.a1; ++i) R.off[i - R.a0] = hroff[(size_t)(prow[i] - S.R0)] - at(Ta);
+            R.off.back() = R.n;
+            R.on = true;
+            if (R.n > 0) {
+                R.x = (int)(n_ranges++ % 2);
+                cudaEvent_t* e = ev.e + 2 + 3 * R.x;
+                a.tiles = (const LdTile*)(dev + S.o_tiles) + tfirst[Ta - S.T0];
+                a.n_tiles = (int32_t)(tfirst[Tb - S.T0] - tfirst[Ta - S.T0]);
+                p.off = d_off;
+                p.rowoff = d_roff;
+                p.base = at(Ta);
+                p.rid = (const int32_t*)(dev + S.o_rid);
+                p.b = d_pb;
+                p.r = d_pr;
+                p.err = d_err;
+                p.nmiss = d_nmiss;
+                CU_TRY(h, cudaEventRecord(e[0], st));
+                CU_TRY(h, launch_ld_pairs(tmap, a, p, true, h->n_sm, st));
+                CU_TRY(h, cudaEventRecord(e[1], st));
+                uint8_t* pin = (uint8_t*)h->ld_pin[R.x].p;
+                CU_TRY(h, cudaMemcpyAsync(pin, d_pb, sizeof(int32_t) * (size_t)R.n, cudaMemcpyDeviceToHost, st));
+                CU_TRY(h, cudaMemcpyAsync(pin + o_pr, d_pr, sizeof(double) * (size_t)R.n, cudaMemcpyDeviceToHost, st));
+                CU_TRY(h, cudaMemcpyAsync(pin + o_flag, d_err, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+                CU_TRY(h, cudaEventRecord(e[2], st));
+            }
+            r = flush();                                // the previous range's sink runs while this one is emitted
+            if (r != DBSLMM_B200_OK) return r;
+            pend = std::move(R);
+            Ta = Tb;
+        }
+        return DBSLMM_B200_OK;
+    };
+    rc = stream_chunks(h, (int64_t)segs.size(), max_bytes, n1, [&](int64_t k) { return segs[k].bytes; }, gather2, launch2);
+    if (rc == DBSLMM_B200_OK) rc = flush();
+    if (rc != DBSLMM_B200_OK) {
+        cudaStreamSynchronize(st);                      // no copy may still be bound for the pinned buffers
+        return rc;
+    }
+    unsigned long long nm = 0;
+    CU_TRY(h, cudaMemcpyAsync(&nm, d_nmiss, sizeof(nm), cudaMemcpyDeviceToHost, st));
+    CU_TRY(h, cudaStreamSynchronize(st));
+    n_miss = (int64_t)nm;
+    if (n_pairs_out) *n_pairs_out = n_pairs;
+    if (n_miss_pairs_out) *n_miss_pairs_out = n_miss;
+    if (kernel_ms_out) *kernel_ms_out = ms;
+    return DBSLMM_B200_OK;
 }
 
 // ---------------------------------------------------------------------------------------------

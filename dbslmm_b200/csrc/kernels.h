@@ -144,6 +144,19 @@ struct LdArgs {
     int32_t n_annot;
     double alpha;               // r2adj = (1 + alpha) r^2 - alpha
 };
+// The pair passes (ld_pairs_kernel, dbslmm_b200_ld_pairs).  A row that never forms a pair has LdRow hi = -1 and g = -1.
+struct LdPairArgs {
+    double r2_min;
+    int32_t* cnt;               // per (row of T, tile, half): passing partners (written by the count pass)
+    const int64_t* off;         // emit: per slot, its first pair among its row's pairs
+    const int64_t* rowoff;      // emit: per padded row, its first pair in the segment
+    int64_t base;               // emit: first pair of the range being emitted
+    const int32_t* rid;         // emit: the caller's row index of every padded row
+    int32_t* b;                 // emit: b of each pair
+    double* r;                  // emit: r of each pair
+    int32_t* err;               // emit: set when a slot emits other than it counted
+    unsigned long long* nmiss;  // emit: += pairs with a row with missing calls
+};
 cudaError_t launch_ld_group_flags(const LdRow* rows, int32_t n_groups, const int32_t* rowN, int32_t n_ref, int32_t* gflags,
                                   int32_t* any, cudaStream_t st);
 cudaError_t launch_ld_band(const CUtensorMap& tmap, const LdArgs& a, int n_sm, cudaStream_t st);
@@ -152,6 +165,11 @@ cudaError_t launch_ld_band(const CUtensorMap& tmap, const LdArgs& a, int n_sm, c
 cudaError_t launch_ld_band_annot(const CUtensorMap& tmap, const LdArgs& a, int n_sm, cudaStream_t st);
 cudaError_t launch_ld_annot_reduce(const double* slots, const int64_t* sbase, const int32_t* nslot, const LdRow* rows, int64_t row0,
                                    int64_t n_rows, int32_t n_annot, double* l2, cudaStream_t st);
+// pairs: the count (emit = false) or emit pass over the upper-band tiles (T, P >= T) of a.tiles, T on the TMEM lanes (tj)
+cudaError_t launch_ld_pairs(const CUtensorMap& tmap, const LdArgs& a, const LdPairArgs& p, bool emit, int n_sm, cudaStream_t st);
+// the count slots of a segment's n_rows padded rows -> off (per slot, within its row) and rowoff[0..n_rows] (per row, from 0)
+cudaError_t launch_ld_pair_scan(const int32_t* cnt, const int64_t* sbase, const int32_t* nslot, int64_t n_rows, int64_t* off,
+                                int64_t* rowoff, cudaStream_t st);
 cudaError_t launch_ld_reduce(const double* slots, const int64_t* tbase, const int32_t* tnslot, const int32_t* wcount,
                              int64_t n_prows, double a, double* l2, cudaStream_t st);
 

@@ -391,6 +391,218 @@ ld_band_kernel(const __grid_constant__ CUtensorMap tmap, const LdArgs a) {
     if (warp == 1) tmem_dealloc<512>(tmem_base);
 }
 
+// Warps 0 and 1 of ld_pairs_kernel: the TMA producer and the MMA issuer of ld_band_kernel, for the tiles of this CTA that
+// belong to the kMiss kernel.  (ld_band_kernel keeps its own copy of these loops: factored through these functions its
+// register allocation, and so its code, would change.)
+template <bool kMiss, class Cfg>
+__device__ __forceinline__ void ld_band_produce(const CUtensorMap& tmap, const LdArgs& a, uint8_t* smem, uint64_t* full_bar,
+                                                uint64_t* empty_bar, int t0, int tstride, int n_tiles, int nk) {
+    uint32_t it = 0;
+    for (int t = t0; t < n_tiles; t += tstride) {
+        const LdTile tl = ld_tile_rec(a.tiles + t);
+        if (ld_tile_missing(a, tl) != kMiss) continue;
+        const bool diag = (tl.ti == tl.tj);
+        const int32_t rowJ = tl.tj * kLdTile, rowI = tl.ti * kLdTile;
+        const uint32_t bytes = kMiss ? 4u * kLdTileBytes : (uint32_t)((diag ? 1 : 2) * kLdTileBytes);
+        for (int ks = 0; ks < nk; ++ks, ++it) {
+            const int s = it % Cfg::kStages;
+            mbar_wait(&empty_bar[s], ((it / Cfg::kStages) & 1u) ^ 1u);
+            uint8_t* st = smem + (size_t)s * Cfg::kStageBytes;
+            if (elect_one()) {
+                mbar_expect_tx(&full_bar[s], bytes);
+                tma_load_2d(st, &tmap, ks * 128, rowJ, &full_bar[s]);
+                if (kMiss) {
+                    // [g_j | M_j | g_i | M_i]: the I-side rows and masks are adjacent, one B operand of 256 rows
+                    tma_load_2d(st + kLdTileBytes, &tmap, ks * 128, rowJ + a.mask_off, &full_bar[s]);
+                    tma_load_2d(st + 2 * kLdTileBytes, &tmap, ks * 128, rowI, &full_bar[s]);
+                    tma_load_2d(st + 3 * kLdTileBytes, &tmap, ks * 128, rowI + a.mask_off, &full_bar[s]);
+                } else if (!diag) {
+                    tma_load_2d(st + kLdTileBytes, &tmap, ks * 128, rowI, &full_bar[s]);
+                }
+            }
+            __syncwarp();
+        }
+    }
+}
+
+template <bool kMiss, class Cfg>
+__device__ __forceinline__ void ld_band_mma(const LdArgs& a, uint8_t* smem, uint64_t* full_bar, uint64_t* empty_bar, uint64_t* acc_full,
+                                            uint64_t* acc_empty, uint32_t tmem_base, int t0, int tstride, int n_tiles, int nk) {
+    constexpr uint32_t idesc = make_i8_idesc(kLdTile, kMiss ? 2 * kLdTile : kLdTile);
+    uint32_t it = 0, lt = 0;
+    for (int t = t0; t < n_tiles; t += tstride) {
+        const LdTile tl = ld_tile_rec(a.tiles + t);
+        if (ld_tile_missing(a, tl) != kMiss) continue;
+        const bool diag = (tl.ti == tl.tj);
+        const uint32_t as = lt % Cfg::kAcc;
+        mbar_wait(&acc_empty[as], ((lt / Cfg::kAcc) & 1u) ^ 1u);      // the epilogue has drained this accumulator
+        tc_fence_after();
+        const uint32_t tm = tmem_base + as * Cfg::kAccCols;
+        for (int ks = 0; ks < nk; ++ks, ++it) {
+            const int s = it % Cfg::kStages;
+            mbar_wait(&full_bar[s], (it / Cfg::kStages) & 1u);
+            tc_fence_after();
+            const uint32_t st = smem_u32(smem + (size_t)s * Cfg::kStageBytes);
+            if (elect_one()) {
+#pragma unroll
+                for (int kk = 0; kk < 4; ++kk) {
+                    const uint32_t acc = (ks > 0 || kk > 0) ? 1u : 0u;
+                    const uint64_t adv = (uint64_t)(kk * 2);         // +32 bytes inside the 128 B swizzle atom
+                    if (kMiss) {
+                        const uint64_t dI = make_sw128_kmajor_desc(st + 2 * kLdTileBytes);
+                        umma_i8(tm, make_sw128_kmajor_desc(st) + adv, dI + adv, idesc, acc);                       // Q | P1
+                        umma_i8(tm + 2 * kLdTile, make_sw128_kmajor_desc(st + kLdTileBytes) + adv, dI + adv, idesc, acc);   // P2 | N
+                    } else {
+                        const uint64_t dJ = make_sw128_kmajor_desc(st), dI = make_sw128_kmajor_desc(diag ? st : st + kLdTileBytes);
+                        umma_i8(tm, dJ + adv, dI + adv, idesc, acc);
+                    }
+                }
+                umma_commit(&empty_bar[s]);
+                if (ks == nk - 1) umma_commit(&acc_full[as]);
+            }
+            __syncwarp();
+        }
+        ++lt;
+    }
+}
+
+// SNP pairs (ld_pairs_kernel<kMiss, kEmit>, dbslmm_b200_ld_pairs): tiles (T, P), P >= T, of
+// the upper band, T on the TMEM lanes (tj) and P the partner tile (ti).  A pair (a, b) of padded rows passes when b > a,
+// b <= hi_a (a's window; -1 for a row that never forms a pair), b is a row with called genotypes and nonzero variance
+// (g >= 0) and ld_pair_pass(r).  Both passes decide every pair through this one function on the same bits of r.
+__device__ __forceinline__ bool ld_pair_pass(double r, double r2_min) { return __dmul_rn(r, r) >= r2_min; }
+
+// The epilogue of both pair passes: this lane owns row a = jl of T, this warp the 64 partners of one half of P, walked in
+// ascending order.  The count pass writes the number of passing partners to the slot of (a, P, half),
+// cnt[sr + jl sr_stride + half]; the emit pass writes b (the caller's row index) and r of each at
+// rowoff[a] + off[slot] - base, counts again, and raises *err where the counts differ (never writing past its slot).
+template <bool kMiss, bool kEmit>
+__device__ __forceinline__ void ld_pairs_epilogue(const LdArgs& a, const LdPairArgs& p, LdRow* rs, uint64_t* acc_full, uint64_t* acc_empty,
+                                                  uint32_t tmem_base, int warp, int lane, int t0, int tstride, int n_tiles) {
+    using Cfg = LdCfg<kMiss>;
+    const int e = warp - 2, q = warp & 3, half = e >> 2;
+    const int jl = q * 32 + lane;
+    const double dn = (double)a.n_ref, r2_min = p.r2_min;
+    uint32_t lt = 0;
+    for (int t = t0; t < n_tiles; t += tstride) {
+        const LdTile tl = ld_tile_rec(a.tiles + t);
+        if (ld_tile_missing(a, tl) != kMiss) continue;
+        const int ag = tl.tj * kLdTile + jl, i0 = tl.ti * kLdTile + half * 64;
+        const LdRow rj = a.rows[ag];
+        __syncwarp();
+        rs[lane] = a.rows[i0 + lane];
+        rs[32 + lane] = a.rows[i0 + 32 + lane];
+        __syncwarp();
+        const int64_t slot = tl.sr + (int64_t)jl * tl.sr_stride + half;
+        int64_t o = 0;
+        int32_t n = 0, cap = 0, ra = 0;
+        uint32_t nmiss = 0;
+        if (kEmit) {
+            cap = p.cnt[slot];
+            o = p.rowoff[ag] + p.off[slot] - p.base;
+            ra = p.rid[ag];
+        }
+        const bool amiss = rj.N != a.n_ref;
+        const uint32_t as = lt % Cfg::kAcc;
+        mbar_wait(&acc_full[as], (lt / Cfg::kAcc) & 1u);
+        tc_fence_after();
+        const uint32_t tlane = tmem_base + as * Cfg::kAccCols + ((uint32_t)(q * 32) << 16) + (uint32_t)(half * 64);
+        auto visit = [&](int r, double rr) {
+            const LdRow& ri = rs[r];
+            const int ig = i0 + r;
+            if (ri.g >= 0 && ig > ag && ig <= rj.hi && ld_pair_pass(rr, r2_min)) {
+                if (kEmit && n < cap) {
+                    p.b[o] = ra + (ig - ag);          // the rows of a chromosome are consecutive padded rows
+                    p.r[o] = rr;
+                    ++o;
+                    nmiss += (amiss || ri.N != a.n_ref) ? 1u : 0u;
+                }
+                ++n;
+            }
+        };
+        if (!kMiss) {
+            uint32_t v[2][32];
+            tmem_ld32(tlane, v[0]);
+            tmem_ld32(tlane + 32, v[1]);
+            tmem_ld_wait();
+            tc_fence_before();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&acc_empty[as]);
+            const double Sj = rj.S, wj = rj.w * dn;
+#pragma unroll
+            for (int c = 0; c < 2; ++c)
+#pragma unroll
+                for (int k = 0; k < 32; ++k) {
+                    const LdRow& ri = rs[c * 32 + k];
+                    visit(c * 32 + k, fma(-ri.S, Sj, u32_to_f64(v[c][k]) * dn) * ri.w * wj);
+                }
+        } else {
+            const int64_t Nj = rj.N, Sj = (int64_t)rj.S;
+#pragma unroll 1
+            for (int c16 = 0; c16 < 4; ++c16) {
+                const uint32_t col0 = (uint32_t)(c16 * 16);
+                uint32_t v0[16], v1[16], v2[16], v3[16];
+                ld_tmem_ld16(tlane + col0, v0);
+                ld_tmem_ld16(tlane + kLdTile + col0, v1);
+                ld_tmem_ld16(tlane + 2 * kLdTile + col0, v2);
+                ld_tmem_ld16(tlane + 3 * kLdTile + col0, v3);
+                tmem_ld_wait();
+#pragma unroll
+                for (int k = 0; k < 16; ++k) {
+                    const LdRow& ri = rs[c16 * 16 + k];
+                    const int64_t Ni = ri.N, Si = (int64_t)ri.S;
+                    const int64_t num = Ni * Nj * (int64_t)v0[k] - Ni * Sj * (int64_t)v2[k] - Nj * Si * (int64_t)v1[k] +
+                                        Si * Sj * (int64_t)v3[k];
+                    visit(c16 * 16 + k, (double)num * ri.w * rj.w);
+                }
+            }
+            tc_fence_before();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&acc_empty[as]);
+        }
+        if (!kEmit) {
+            p.cnt[slot] = n;
+        } else {
+            if (n != cap) atomicOr(p.err, 1);
+            for (int w = 16; w >= 1; w >>= 1) nmiss += __shfl_xor_sync(0xffffffffu, nmiss, w);
+            if (lane == 0 && nmiss) atomicAdd(p.nmiss, (unsigned long long)nmiss);
+        }
+        ++lt;
+    }
+}
+
+// The pair passes over the upper band (see ld_pairs_epilogue): ld_band_kernel's warp roles, with LdCfg<kMiss>'s ring.
+template <bool kMiss, bool kEmit>
+__global__ void __launch_bounds__(kLdThreads, 1)
+ld_pairs_kernel(const __grid_constant__ CUtensorMap tmap, const LdArgs a, const LdPairArgs p) {
+    using Cfg = LdCfg<kMiss>;
+    extern __shared__ uint8_t smem_raw[];
+    __shared__ __align__(8) uint64_t full_bar[Cfg::kStages], empty_bar[Cfg::kStages], acc_full[Cfg::kAcc], acc_empty[Cfg::kAcc];
+    __shared__ __align__(16) LdRow rows_s[8][64];        // per epilogue warp: the constants of its 64 partner rows
+    __shared__ uint32_t tmem_slot;
+    if (kMiss && *a.any == 0) return;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
+    const int t0 = (int)blockIdx.x, tstride = (int)gridDim.x, n_tiles = a.n_tiles;
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < Cfg::kStages; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
+        for (int b = 0; b < Cfg::kAcc; ++b) { mbar_init(&acc_full[b], 1); mbar_init(&acc_empty[b], 8); }
+        mbar_fence_init();
+        tma_prefetch_desc(&tmap);
+    }
+    if (warp == 1) tmem_alloc<512>(&tmem_slot);
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem_base = tmem_slot;
+    if (warp == 0) ld_band_produce<kMiss, Cfg>(tmap, a, smem, full_bar, empty_bar, t0, tstride, n_tiles, a.nk);
+    else if (warp == 1) ld_band_mma<kMiss, Cfg>(a, smem, full_bar, empty_bar, acc_full, acc_empty, tmem_base, t0, tstride, n_tiles, a.nk);
+    else ld_pairs_epilogue<kMiss, kEmit>(a, p, rows_s[warp - 2], acc_full, acc_empty, tmem_base, warp, lane, t0, tstride, n_tiles);
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 1) tmem_dealloc<512>(tmem_base);
+}
+
 // gflags[grp] = some row of 128-row group grp has a missing call (from the decoder's counts rowN); *any |= gflags.  One warp
 // per group.
 __global__ void ld_group_flags_kernel(const LdRow* __restrict__ rows, int32_t n_groups, const int32_t* __restrict__ rowN,
@@ -494,6 +706,79 @@ cudaError_t launch_ld_reduce(const double* slots, const int64_t* tbase, const in
                              int64_t n_prows, double a, double* l2, cudaStream_t st) {
     if (n_prows == 0) return cudaSuccess;
     ld_reduce_kernel<<<(unsigned)((n_prows + 255) / 256), 256, 0, st>>>(slots, tbase, tnslot, wcount, n_prows, a, l2);
+    return cudaGetLastError();
+}
+
+// The pair offsets of one segment, after its count pass.  Row p of the segment's scored tiles (T = p / 128) has the
+// 2 nslot[T] slots sbase[T] + (p % 128) 2 nslot[T] + u, u in (tile, half) order: off[slot] = the pairs of p's earlier
+// slots, rowcnt[p] = all of p's pairs.
+__global__ void ld_pair_rowscan_kernel(const int32_t* __restrict__ cnt, const int64_t* __restrict__ sbase,
+                                       const int32_t* __restrict__ nslot, int64_t n_rows, int64_t* __restrict__ off,
+                                       int64_t* __restrict__ rowcnt) {
+    const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n_rows) return;
+    const int64_t T = p / kLdTile;
+    const int32_t ns = 2 * nslot[T];
+    const int64_t b = sbase[T] + (p % kLdTile) * ns;
+    int64_t s = 0;
+    for (int32_t u = 0; u < ns; ++u) {
+        off[b + u] = s;
+        s += cnt[b + u];
+    }
+    rowcnt[p] = s;
+}
+
+// rowoff[p] = sum of rowcnt[0..p) for p <= n_rows, in place over rowcnt[0..n_rows] (one CTA: each thread scans a contiguous
+// run of rows, then the runs' totals are scanned in shared memory)
+__global__ void __launch_bounds__(1024) ld_pair_offsets_kernel(int64_t* __restrict__ row, int64_t n_rows) {
+    __shared__ int64_t part[1024];
+    const int64_t per = (n_rows + 1023) / 1024, r0 = min(n_rows, (int64_t)threadIdx.x * per), r1 = min(n_rows, r0 + per);
+    int64_t s = 0;
+    for (int64_t p = r0; p < r1; ++p) s += row[p];
+    part[threadIdx.x] = s;
+    __syncthreads();
+    for (int w = 1; w < 1024; w <<= 1) {
+        const int64_t x = threadIdx.x >= (unsigned)w ? part[threadIdx.x - w] : 0;
+        __syncthreads();
+        part[threadIdx.x] += x;
+        __syncthreads();
+    }
+    int64_t acc = part[threadIdx.x] - s;
+    for (int64_t p = r0; p < r1; ++p) {
+        const int64_t c = row[p];
+        row[p] = acc;
+        acc += c;
+    }
+    if (threadIdx.x == 1023) row[n_rows] = part[1023];
+}
+
+// The pair passes: one-plane and four-plane kernels over the same tile list, as launch_ld_band.
+cudaError_t launch_ld_pairs(const CUtensorMap& tmap, const LdArgs& a, const LdPairArgs& p, bool emit, int n_sm, cudaStream_t st) {
+    if (a.n_tiles == 0) return cudaSuccess;
+    const int grid = std::min(a.n_tiles, n_sm);
+    auto go = [&](auto k0, auto k1) {
+        cudaError_t e = cudaFuncSetAttribute(k0, cudaFuncAttributeMaxDynamicSharedMemorySize, LdCfg<false>::kSmem);
+        if (e != cudaSuccess) return e;
+        e = cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, LdCfg<true>::kSmem);
+        if (e != cudaSuccess) return e;
+        k0<<<grid, kLdThreads, LdCfg<false>::kSmem, st>>>(tmap, a, p);
+        e = cudaGetLastError();
+        if (e != cudaSuccess) return e;
+        k1<<<grid, kLdThreads, LdCfg<true>::kSmem, st>>>(tmap, a, p);
+        return cudaGetLastError();
+    };
+    return emit ? go(ld_pairs_kernel<false, true>, ld_pairs_kernel<true, true>)
+                : go(ld_pairs_kernel<false, false>, ld_pairs_kernel<true, false>);
+}
+
+cudaError_t launch_ld_pair_scan(const int32_t* cnt, const int64_t* sbase, const int32_t* nslot, int64_t n_rows, int64_t* off,
+                                int64_t* rowoff, cudaStream_t st) {
+    if (n_rows > 0) {
+        ld_pair_rowscan_kernel<<<(unsigned)((n_rows + 255) / 256), 256, 0, st>>>(cnt, sbase, nslot, n_rows, off, rowoff);
+        cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return e;
+    }
+    ld_pair_offsets_kernel<<<1, 1024, 0, st>>>(rowoff, n_rows);
     return cudaGetLastError();
 }
 

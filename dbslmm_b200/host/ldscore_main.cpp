@@ -37,6 +37,11 @@
 #include "plink_bed.hpp"
 
 using namespace std;
+using plink::Bim;
+using plink::bim_chromosomes;
+using plink::count_fam;
+using plink::read_bim;
+using plink::split_ws;
 
 namespace {
 
@@ -70,14 +75,6 @@ void print_help() {
     cout << " --thin-annot             the --annot file has no CHR BP SNP CM columns: its header holds the names only." << endl;
     cout << " --yes-really             allow a window that spans a whole chromosome." << endl;
     cout << " --out          [prefix]  writes <out>.l2.ldscore.gz, <out>.l2.M, <out>.l2.M_5_50 and <out>.log." << endl;
-}
-
-vector<string> split_ws(const string& line) {
-    vector<string> t;
-    istringstream ss(line);
-    string x;
-    while (ss >> x) t.push_back(x);
-    return t;
 }
 
 double parse_num(const string& opt, const string& v) {
@@ -130,38 +127,6 @@ Params parse(int argc, char** argv) {
     if (p.out.empty()) die("--out is required");
     if (p.thin_annot && p.annot.empty()) die("--thin-annot needs --annot");
     return p;
-}
-
-struct Bim { vector<string> chr, snp, bp_tok; vector<double> cm, bp; };
-
-Bim read_bim(const string& path) {
-    ifstream f(path.c_str());
-    if (!f) die(path + " does not exist");
-    Bim b;
-    string line;
-    size_t ln = 0;
-    while (getline(f, line)) {
-        ++ln;
-        const vector<string> t = split_ws(line);
-        if (t.empty()) continue;
-        if (t.size() < 6) die(path + " line " + to_string(ln) + ": a .bim line has 6 columns");
-        char* e1 = nullptr;
-        char* e2 = nullptr;
-        const double cm = strtod(t[2].c_str(), &e1), bp = strtod(t[3].c_str(), &e2);
-        if (*e1 != '\0' || *e2 != '\0' || !std::isfinite(cm) || !std::isfinite(bp))
-            die(path + " line " + to_string(ln) + ": columns 3 and 4 (cM, bp) must be numbers");
-        b.chr.push_back(t[0]); b.snp.push_back(t[1]); b.bp_tok.push_back(t[3]); b.cm.push_back(cm); b.bp.push_back(bp);
-    }
-    return b;
-}
-
-int64_t count_fam(const string& path) {
-    ifstream f(path.c_str());
-    if (!f) die(path + " does not exist");
-    string line;
-    int64_t n = 0;
-    while (getline(f, line)) if (!split_ws(line).empty()) ++n;
-    return n;
 }
 
 // ldsc's .annot[.gz]: names and a row-major [n_snp][C] matrix; the SNP column (full format) must match the .bim's
@@ -251,8 +216,10 @@ int main(int argc, char* argv[]) {
     }
 
     // ---- panel
-    const int64_t n = count_fam(P.bfile + ".fam");
-    const Bim bim = read_bim(P.bfile + ".bim");
+    int64_t n = 0;
+    Bim bim;
+    for (const string& err : {count_fam(P.bfile + ".fam", n), read_bim(P.bfile + ".bim", bim)})
+        if (!err.empty()) die(err);
     const int64_t n_snp = (int64_t)bim.chr.size();
     if (n == 0) die(P.bfile + ".fam lists no individual");
     if (n > 409344) die(P.bfile + ".fam lists " + to_string(n) + " individuals; ldscore takes at most 409,344");
@@ -267,23 +234,13 @@ int main(int argc, char* argv[]) {
     say(to_string(n) + " individuals and " + to_string(n_snp) + " variants in " + P.bfile + ".bed/.bim/.fam");
 
     // ---- chromosomes: contiguous runs, coordinates of the window's kind non-decreasing
-    vector<int32_t> chr_off{0};
+    vector<int32_t> chr_off;
     vector<string> chr_name;
-    unordered_set<string> seen;
     const vector<double>* cx = P.kind == 0 ? &bim.cm : P.kind == 1 ? &bim.bp : nullptr;
-    for (int64_t i = 0; i < n_snp; ++i) {
-        if (i == 0 || bim.chr[i] != bim.chr[i - 1]) {
-            if (!seen.insert(bim.chr[i]).second)
-                die("chromosome " + bim.chr[i] + " is not contiguous in " + P.bfile + ".bim (it appears again at line " + to_string(i + 1) +
-                    "): sort the fileset by chromosome");
-            if (i > 0) chr_off.push_back((int32_t)i);
-            chr_name.push_back(bim.chr[i]);
-        } else if (cx && (*cx)[i] < (*cx)[i - 1]) {
-            die(P.bfile + ".bim line " + to_string(i + 1) + ": the " + (P.kind == 0 ? "cM" : "bp") + " coordinates of chromosome " +
-                bim.chr[i] + " are not sorted");
-        }
+    {
+        const string err = bim_chromosomes(bim, P.bfile + ".bim", cx, P.kind == 0 ? "cM" : "bp", chr_off, chr_name);
+        if (!err.empty()) die(err);
     }
-    chr_off.push_back((int32_t)n_snp);
     unordered_set<string> print_ids;
     if (!P.print_snps.empty()) {
         ifstream f(P.print_snps.c_str());

@@ -40,6 +40,7 @@ extern "C" {
 #define DBSLMM_B200_ERR_ARG      (-2)   /* bad argument                                    */
 #define DBSLMM_B200_ERR_STATE    (-3)   /* call order (e.g. fit before load_bed)           */
 #define DBSLMM_B200_ERR_NOMEM    (-4)   /* device or host allocation failed                */
+#define DBSLMM_B200_ERR_SINK     (-5)   /* a caller's sink returned nonzero (dbslmm_b200_ld_pairs) */
 
 /* per-block status bits written to block_status_out */
 #define DBSLMM_B200_BLK_OK          0
@@ -261,6 +262,34 @@ DBSLMM_B200_API int  dbslmm_b200_ldscore_annot(dbslmm_b200_handle* h, const uint
                          int32_t wind_kind, const double* coord, double max_dist, double maf_min, int64_t segment_rows,
                          const double* annot, int32_t n_annot,
                          uint8_t* kept_out, double* maf_out, double* l2_out, int32_t* guard_out, float* kernel_ms_out);
+
+/* Windowed r between SNP pairs of a reference panel, as `plink --r2 --ld-window N --ld-window-kb K --ld-window-r2 R` selects
+ * them.  rows, chr_off and coord work as in dbslmm_b200_ldscore (coord: base pairs, non-decreasing within a chromosome,
+ * required).  A pair (a, b), a < b positions in rows, is written when both lie in one chromosome, b - a <= max_snps - 1
+ * (--ld-window N), coord[b] - coord[a] <= max_dist (--ld-window-kb K as K x 1000, edges included) and r^2 >= r2_min
+ * (--ld-window-r2).  Windows never cross a chromosome.  r is dbslmm_b200_ldscore's: the Pearson r of the mean-imputed
+ * allele counts, num / sqrt(n_a n_b d_a d_b) from the exact integer numerator; without missing calls in either SNP it is
+ * the Pearson r of the allele counts.  A row with no called genotype or with zero variance is not USABLE: it never forms a
+ * pair, but it still counts toward the max_snps distance.
+ * The pairs are delivered in ascending (a, b) order through `sink`, called on the calling thread with CSR slices: rows
+ * a0 .. a1 - 1 (consecutive slices cover every row exactly once), off[0 .. a1 - a0] (off[0] = 0), and for the pairs of row
+ * a = a0 + i, entries off[i] .. off[i + 1] - 1 of b (the partner's position in rows) and r (signed).  The arrays are valid
+ * during the call only.  A nonzero return from the sink stops the call with DBSLMM_B200_ERR_SINK; the sink is not called
+ * again.  Outputs (each may be NULL): usable_out [n_rows] 0/1, n_pairs_out the number of pairs written, n_miss_pairs_out
+ * the number of those with a SNP with missing calls, kernel_ms_out the summed device time of the call's kernels.
+ * Two passes over the rows as dbslmm_b200_ldscore, segment_rows as there; each segment is counted on the device, then
+ * emitted in ranges of row tiles whose pairs fit a fixed device buffer (8 Mi pairs, or the most pairs one 128-row tile can
+ * have, whichever is more) and copied to two pinned buffers in turn, so the sink of one range runs while the device
+ * emits the next.  Device and pinned memory do not grow with the number of pairs.  Deterministic: the bits and the order
+ * of the output depend neither on the segment size, nor on the other chromosomes of the call, nor on the run.
+ * Limits: n_ref <= 409,344, n_rows <= INT32_MAX, max_snps >= 1, max_dist >= 0 (may be +inf), r2_min not NaN.
+ * Synchronous. */
+typedef int (*dbslmm_b200_ld_sink)(void* user, int64_t a0, int64_t a1, const int64_t* off, const int32_t* b, const double* r);
+DBSLMM_B200_API int  dbslmm_b200_ld_pairs(dbslmm_b200_handle* h, const uint8_t* bed, int64_t n_snp, int32_t n_ref,
+                         const int32_t* rows, int64_t n_rows, const int32_t* chr_off, int32_t n_chr, const double* coord,
+                         int32_t max_snps, double max_dist, double r2_min, int64_t segment_rows,
+                         dbslmm_b200_ld_sink sink, void* user, uint8_t* usable_out, int64_t* n_pairs_out,
+                         int64_t* n_miss_pairs_out, float* kernel_ms_out);
 
 /* ---- inspection hooks used by the parity tests (operate on the state of the last fit) ---- */
 /* int8 codes of one decoded row of the last fit: SNP j of block `block` (its small SNPs first, then its large ones),
