@@ -107,6 +107,7 @@ struct Plan {
     int32_t max_mp = 0;
     std::vector<BlockDesc> blocks;
     std::vector<int32_t> order;                       // concatenated batch member lists (big classes first)
+    std::vector<int32_t> code_layout;                 // block sizes in code-row order: which code rows are genotype rows, which mask rows
     std::vector<Batch> batches;
     bool streaming = false;                           // layout in batch order (else block-index order)
     bool chain_bound = false;                         // the big classes' dependency chains outlast the bulk's throughput time (make_batches)
@@ -206,6 +207,7 @@ struct dbslmm_b200_handle {
     size_t dirty_rows = 0;               // code rows the dirty map covers
     int32_t dirty_n_ref = 0;             // ... for this panel width (another width = another default mask pattern)
     const void* dirty_codes = nullptr;   // ... and this code buffer
+    std::vector<int32_t> dirty_layout;   // ... and this code-row layout (Plan::code_layout)
     PinBuf h_blob, h_out;
     Plan plan;
 
@@ -428,8 +430,10 @@ int build_plan(dbslmm_b200_handle* h, const dbslmm_b200_fit_args* a, Plan& P, co
     // layout order: block index (resident panel) or batch order (streaming: a batch's rows are one range)
     std::vector<int32_t> lay(nb);
     if (P.streaming) lay = P.order; else std::iota(lay.begin(), lay.end(), 0);
+    P.code_layout.clear();
     for (int b : lay) {
         BlockDesc& d = P.blocks[b];
+        P.code_layout.push_back(d.m);
         const int ms = d.ms, ml = d.m - d.ms;
         d.goff = (int32_t)goff;
         d.croff = (int32_t)croff;
@@ -1289,15 +1293,18 @@ int fit_impl(dbslmm_b200_handle* h, const dbslmm_b200_fit_args* a, bool streamin
     CU_TRY(h, h->codes.ensure((size_t)std::max<int64_t>(P.n_code_rows, 1) * h->n_pad));
     {
         // dirty[c] = code row c holds a mask that is NOT the default pattern (decode.cu).  Rows the map has never covered,
-        // and all rows when the panel width changes, start dirty: the first fit then writes their mask rows once.
+        // and all rows when the panel width or the code-row layout changes, start dirty: the first fit then writes their
+        // mask rows once.  (Under another layout a mask row may have been a genotype row, which the map does not track:
+        // resident and streaming fits lay the blocks out in different orders.)
         const size_t need = (size_t)std::max<int64_t>(P.n_code_rows, 1);
-        if (h->dirty_n_ref != h->n_ref || need > h->dirty_rows || h->dirty_codes != h->codes.p) {
+        if (h->dirty_n_ref != h->n_ref || need > h->dirty_rows || h->dirty_codes != h->codes.p || h->dirty_layout != P.code_layout) {
             CU_TRY(h, h->dirty.ensure(need));
             const size_t cover = h->dirty.cap;
             CU_TRY(h, cudaMemsetAsync(h->dirty.p, 1, cover, st));
             h->dirty_rows = cover;
             h->dirty_n_ref = h->n_ref;
             h->dirty_codes = h->codes.p;         // a re-allocated code buffer has lost every mask row
+            h->dirty_layout = P.code_layout;
         }
     }
     CU_TRY(h, h->bflags.ensure(sizeof(int32_t) * (size_t)(std::max(nb, 1) + kMaxBatches + 1)));

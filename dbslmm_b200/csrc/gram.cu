@@ -5,7 +5,7 @@
 // (scr/dtpr.cpp:375-380).  For one LD block with SNP rows i, j (small SNPs first, then
 // large ones), raw allele counts g in {0,1,2} (missing -> 0) and call mask M:
 //     Q_ij = sum g_i g_j,  A_ij = sum g_i M_j,  N_ij = sum M_i M_j          (exact, s32)
-//     num_ij = n_i n_j Q_ij - n_i S_j A_ij - n_j S_i A_ji + S_i S_j N_ij      (exact integer < 2^53)
+//     num_ij = n_i n_j Q_ij - n_i S_j A_ij - n_j S_i A_ji + S_i S_j N_ij      (an integer; see gram_missing_kernel)
 //     Sigma_ij = num_ij * r_i * r_j + (1 - tau) [i == j],   r_i = sqrt(tau (n-1) / (n n_i d_i)),
 //     d_i = n_i Q_ii - S_i^2
 // which equals tau * X^T X / n + (1 - tau) I for the mean-imputed, (N-1)-standardised X of
@@ -863,11 +863,16 @@ gram_missing_kernel(const __grid_constant__ CUtensorMap tmapJ, const __grid_cons
                     const double Si = rcv.x, Ni = rcv.y, ri = rcv.z;
                     const double Q = u32_to_f64(v0[r]), P1 = u32_to_f64(v1[r]);      // counts are >= 0
                     const double P2 = u32_to_f64(v2[r]), Nn = u32_to_f64(v3[r]);
-                    // A_ij = sum g_i M_j = P2,  A_ji = sum g_j M_i = P1; every product and partial sum is an exact integer < 2^53
-                    double num = (Ni * Nj) * Q;
-                    num = fma(-(Ni * Sj), P2, num);
-                    num = fma(-(Nj * Si), P1, num);
-                    num = fma(Si * Sj, Nn, num);
+                    // A_ij = sum g_i M_j = P2,  A_ji = sum g_j M_i = P1.  num = n_i u - S_i w with u = n_j Q - S_j P2 and
+                    // w = n_j P1 - S_j N: u and w are exact (every product and sum below 4 n^2 < 2^53), but n_i u and S_i w
+                    // reach 4 n^3 = 2.7e17 at n = 409,344, past 2^53 above n = 2^17.  So n_i u is split into p + pe exactly
+                    // (fma gives the low part), p - S_i w is rounded once and pe added: num to within about 2 ulps of itself,
+                    // and exact whenever every term is below 2^53 (n <= 2^17).
+                    const double u = fma(-Sj, P2, Nj * Q);
+                    const double w = fma(-Sj, Nn, Nj * P1);
+                    const double p = Ni * u;
+                    const double pe = fma(Ni, u, -p);
+                    const double num = fma(-Si, w, p) + pe;
                     vals[r] = num * ri * rj;
                 }
 #pragma unroll

@@ -57,17 +57,41 @@ def ridge(sigma_s, n_obs):
     return 1.0 / (float(sigma_s) * float(n_obs))
 
 
-def exact_sigma(bed, n_ref, pos, tau):
-    """Sigma* of the SNPs `pos` in np.longdouble from the integer Gram planes Q = G G^T, A_ij = sum g_i M_j, N = M M^T:
-    num_ij = n_i n_j Q_ij - n_i S_j A_ij - n_j S_i A_ji + S_i S_j N_ij (an exact int64),
-    Sigma_ij = num_ij r_i r_j + (1 - tau) delta_ij,  r_i = sqrt(tau (n - 1) / (n n_i d_i)),  d_i = n_i Q_ii - S_i^2."""
+_CODE_TO_COUNT = np.array([2, -1, 1, 0], np.int8)           # PLINK 2-bit code -> allele count of A1, -1 = missing
+
+
+def bed_genotypes(bed, n_ref, pos):
+    """int8 [len(pos), n_ref] allele counts (-1 = missing) of the .bed rows `pos` (payload rows, pitch ceil(n_ref / 4))."""
+    rows = np.asarray(bed, np.uint8)[np.asarray(pos, np.int64)]
+    codes = np.stack([(rows >> (2 * k)) & 3 for k in range(4)], axis=-1).reshape(rows.shape[0], 4 * rows.shape[1])[:, :int(n_ref)]
+    return _CODE_TO_COUNT[codes]
+
+
+def gram_planes(G, chunk_bytes=256 << 20):
+    """The integer Gram planes of genotype rows G (int8, -1 = missing) with BLAS: Q = g g^T, A_ij = sum g_i M_j,
+    N = M M^T (g = G with missing -> 0, M = call mask), as int64.  An FP32 GEMM is exact here: every term is 0, 1, 2 or 4
+    and every partial sum at most 4 n < 2^24.  Chunked over samples so no FP32 operand exceeds `chunk_bytes`."""
+    G = np.asarray(G, np.int8)
+    m, n = G.shape
+    Q, A, N = (np.zeros((m, m), np.int64) for _ in range(3))
+    step = max(1, int(chunk_bytes) // (4 * max(m, 1)))
+    for s in range(0, n, step):
+        c = G[:, s:s + step]
+        M = (c >= 0).astype(np.float32)
+        g = np.maximum(c, 0).astype(np.float32)
+        Q += (g @ g.T).astype(np.int64)
+        A += (g @ M.T).astype(np.int64)
+        N += (M @ M.T).astype(np.int64)
+    return Q, A, N
+
+
+def sigma_from_planes(Q, A, N, n_ref, tau):
+    """Sigma* in np.longdouble from the integer Gram planes (see exact_sigma)."""
     _require_extended()
-    from oracle import oracle as O
-    pos = np.ascontiguousarray(pos, np.int32)
-    m = pos.size
+    Q, A, N = (np.asarray(x, np.int64) for x in (Q, A, N))
+    m = Q.shape[0]
     if m == 0:
         return np.zeros((0, 0), np.longdouble)
-    Q, A, N = (x.astype(np.int64) for x in O.gram_int(bed, int(n_ref), pos))
     S = np.diag(A).copy()
     ni = np.diag(N).copy()
     num = np.outer(ni, ni) * Q - (ni[:, None] * S[None, :]) * A - (ni[None, :] * S[:, None]) * A.T + np.outer(S, S) * N
@@ -79,6 +103,15 @@ def exact_sigma(bed, n_ref, pos, tau):
     sig = num.astype(LD) * r[:, None] * r[None, :]
     sig[np.arange(m), np.arange(m)] += LD(1) - t
     return np.tril(sig) + np.tril(sig, -1).T                   # exactly symmetric
+
+
+def exact_sigma(bed, n_ref, pos, tau):
+    """Sigma* of the SNPs `pos` in np.longdouble from the integer Gram planes Q = G G^T, A_ij = sum g_i M_j, N = M M^T:
+    num_ij = n_i n_j Q_ij - n_i S_j A_ij - n_j S_i A_ji + S_i S_j N_ij (an exact int64: every term is below
+    4 n^3 <= 2.8e17 up to n = 409,344), Sigma_ij = num_ij r_i r_j + (1 - tau) delta_ij,
+    r_i = sqrt(tau (n - 1) / (n n_i d_i)),  d_i = n_i Q_ii - S_i^2."""
+    pos = np.ascontiguousarray(pos, np.int32)
+    return sigma_from_planes(*gram_planes(bed_genotypes(bed, n_ref, pos)), n_ref, tau)
 
 
 def k_matrix(sigma, ms, c):

@@ -169,3 +169,78 @@ def test_tile_check_detects_ten_times_its_floor(m):
     assert scaled_tile_rho(b, 0.0) < R.BARS["tiles"] / 4
     assert scaled_tile_rho(b, 10 * FLOORS[m]) >= R.BARS["tiles"]
     assert scaled_tile_rho(b, FLOORS[m] / 10) < R.BARS["tiles"]
+
+
+# ---- the integer Gram planes by BLAS, and the Sigma bar against the four-plane epilogue's numerator ----------------
+@pytest.mark.parametrize("n,missing", [(403, 0.0), (403, 0.02), (125 * 4 - 3, 0.01), (5, 0.1)])
+def test_blas_planes_equal_the_oracle_bit_for_bit(n, missing):
+    rng = np.random.default_rng(n + int(missing * 100))
+    G = synth.make_genotypes(rng, [40, 23], n, missing_rate=missing)
+    bed = synth.pack_bed(G)
+    pos = np.array([0, 5, 5, 62, 17, 40, 3, 61, 22], np.int32)           # out of order, one row twice
+    assert np.array_equal(R.bed_genotypes(bed, n, pos), G[pos])
+    for chunk in (256 << 20, 4 * pos.size * 7):                            # one chunk; chunks of 7 samples
+        for got, want in zip(R.gram_planes(R.bed_genotypes(bed, n, pos), chunk_bytes=chunk), O.gram_int(bed, n, pos)):
+            assert got.dtype == np.int64 and np.array_equal(got, want)
+
+
+def decoder_r(S, ni, sq, n, tau):
+    """r_i as the decoder computes it in FP64 (decode.cu): sqrt(tau (n - 1) / (n n_i d)), d = n_i sum g^2 - S^2."""
+    d = ni.astype(np.float64) * sq.astype(np.float64) - S.astype(np.float64) ** 2
+    return np.sqrt(tau * (float(n) - 1.0) / (float(n) * ni.astype(np.float64) * d))
+
+
+def epilogue_sigma(Q, A, N, n, tau, numerator):
+    """The four-plane epilogue's Sigma, replayed on the host with exactly rounded fma, then (num r_i) r_j and 1 - tau added
+    on the diagonal.  The numerator is
+      "exact"  the exact integer, rounded once to FP64;
+      "chain"  num = (n_i n_j) Q; num = fma(-(n_i S_j), A_ij, num); num = fma(-(n_j S_i), A_ji, num);
+               num = fma(S_i S_j, N_ij, num) -- what gram.cu computed before, exact only while every term is below 2^53;
+      "split"  u = fma(-S_j, A_ij, n_j Q); w = fma(-S_j, N, n_j A_ji); p = n_i u; pe = fma(n_i, u, -p);
+               num = fma(-S_i, w, p) + pe -- what gram.cu computes."""
+    from fractions import Fraction
+
+    def fma(a, b, c):
+        return float(Fraction(a) * Fraction(b) + Fraction(c))
+    S, ni = np.diag(A).astype(np.int64), np.diag(N).astype(np.int64)
+    r = decoder_r(S, ni, np.diag(Q), n, tau)
+    m = Q.shape[0]
+    out = np.zeros((m, m))
+    for i in range(m):
+        for j in range(i + 1):
+            Ni, Nj, Si, Sj = (int(x) for x in (ni[i], ni[j], S[i], S[j]))
+            if numerator == "exact":
+                num = float(Ni * Nj * int(Q[i, j]) - Ni * Sj * int(A[i, j]) - Nj * Si * int(A[j, i]) + Si * Sj * int(N[i, j]))
+            elif numerator == "split":
+                u = fma(-float(Sj), float(A[i, j]), float(Nj) * float(Q[i, j]))
+                w = fma(-float(Sj), float(N[i, j]), float(Nj) * float(A[j, i]))
+                p = float(Ni) * u
+                num = fma(-float(Si), w, p) + fma(float(Ni), u, -p)
+            else:
+                num = (float(Ni) * float(Nj)) * float(Q[i, j])
+                num = fma(-(float(Ni) * float(Sj)), float(A[i, j]), num)
+                num = fma(-(float(Nj) * float(Si)), float(A[j, i]), num)
+                num = fma(float(Si) * float(Sj), float(N[i, j]), num)
+            v = num * r[i] * r[j]
+            out[i, j] = out[j, i] = v + (1.0 - tau) if i == j else v
+    return out
+
+
+def test_sigma_bar_detects_an_fp64_numerator_at_max_n_ref():
+    """At n = 409,344 with 1 % missing calls and half the SNPs counting the major allele, the terms of the four-plane
+    numerator reach 4 n^3 = 2.7e17 > 2^53: the FP64 chain rounds them and misses the 16-ulp Sigma bar; the exact numerator
+    and the split form meet it.  Below n = 2^17 every term is exact and the three agree bit for bit."""
+    for n, fails in ((409_344, True), (2_000, False)):
+        rng = np.random.default_rng(1)
+        G = synth.make_genotypes(rng, [24], n)
+        flip = rng.random(24) < 0.5
+        G[flip] = 2 - G[flip]
+        G = np.where(rng.random(G.shape) < 0.01, np.int8(-1), G)
+        Q, A, N = R.gram_planes(G)
+        sstar = R.sigma_from_planes(Q, A, N, n, TAU)
+        chain, exact, split = (epilogue_sigma(Q, A, N, n, TAU, k) for k in ("chain", "exact", "split"))
+        for S in (exact, split):
+            assert R.sigma_ratio(S, sstar) <= R.BARS["sigma"], (n, R.sigma_ratio(S, sstar))
+        assert (R.sigma_ratio(chain, sstar) > R.BARS["sigma"]) == fails, (n, R.sigma_ratio(chain, sstar))
+        if not fails:
+            assert np.array_equal(chain, exact) and np.array_equal(split, exact)
